@@ -198,31 +198,43 @@ static int segmax_scan(fslrc_ctx *ctx, Pipe *P, const int *seg, const int *val, 
     KL(prims::k_scan_segmax, tiles, prims::SC_THREADS, seg, val, out, n, (unsigned long long *)(P->prim + 256), (unsigned *)P->prim);
     return 0;
 }
-// stable LSD radix sort of (key, value) pairs on key bits [b0, b1); the inputs are left untouched
-static int sort_pairs(fslrc_ctx *ctx, Pipe *P, const unsigned *kin, unsigned *kout, const int *vin, int *vout, int n, int b0, int b1) {
+// stable LSD radix sort of (key, value) pairs on key bits [b0, b1); the inputs are left untouched.  The last pass hands
+// every pair to `last` with its output position; *last_start (optional) receives the start of every digit of that pass.
+template <typename Out>
+static int sort_pairs_to(fslrc_ctx *ctx, Pipe *P, const unsigned *kin, const int *vin, int n, int b0, int b1, Out last,
+                         const unsigned **last_start = nullptr) {
     cudaStream_t st = ctx->stream;
     if (n <= 0) return 0;
     const int npass = std::max(1, (b1 - b0 + 7) / 8);
     if (npass > 4) return fail(ctx, FSLRC_ERR_ARG, "radix sort: more than 32 key bits");
     unsigned *hist; DA(hist, 4 * 256);
     CK(cudaMemsetAsync(hist, 0, sizeof(unsigned) * 4 * 256, st));
-    unsigned *tk = nullptr; int *tv = nullptr;
-    if (npass > 1) { DA(tk, n); DA(tv, n); }
+    prims::PairOut tmp[2] = {};
+    for (int k = 0; k < std::min(npass - 1, 2); k++) { DA(tmp[k].kout, n); DA(tmp[k].vout, n); }
     KL(prims::k_rs_hist, std::min(nblk(n, 256 * 16), n_sms(ctx) * 8), 256, kin, n, b0, b1, npass, hist);
     KL(prims::k_rs_scan, npass, 256, hist);
     const int tiles = nblk(n, prims::RS_TILE);
     const unsigned *ks = kin; const int *vs = vin;
     for (int p = 0; p < npass; p++) {
-        unsigned *kd = ((npass - 1 - p) % 2 == 0) ? kout : tk;       // the last pass lands in (kout, vout)
-        int *vd = ((npass - 1 - p) % 2 == 0) ? vout : tv;
         int r = prim_scratch(ctx, P, sizeof(unsigned) * 256 * (size_t)tiles); if (r) return r;
         const int nbits = std::min(8, b1 - b0 - 8 * p);
+        const unsigned *gb = hist + 256 * p;
         ctx->launches++;
-        prims::k_rs_onesweep<<<tiles, prims::RS_THREADS, sizeof(prims::RsSmem), st>>>(ks, kd, vs, vd, n, b0 + 8 * p, (1 << nbits) - 1, hist + 256 * p,
-                                                                                      (unsigned *)(P->prim + 256), (unsigned *)P->prim);
-        ks = kd; vs = vd;
+        if (p == npass - 1) {
+            prims::k_rs_onesweep<<<tiles, prims::RS_THREADS, sizeof(prims::RsSmem), st>>>(ks, vs, last, n, b0 + 8 * p, (1 << nbits) - 1, gb,
+                                                                                          (unsigned *)(P->prim + 256), (unsigned *)P->prim);
+        } else {
+            const prims::PairOut o = tmp[p & 1];
+            prims::k_rs_onesweep<<<tiles, prims::RS_THREADS, sizeof(prims::RsSmem), st>>>(ks, vs, o, n, b0 + 8 * p, (1 << nbits) - 1, gb,
+                                                                                          (unsigned *)(P->prim + 256), (unsigned *)P->prim);
+            ks = o.kout; vs = o.vout;
+        }
     }
+    if (last_start) *last_start = hist + 256 * (npass - 1);
     return 0;
+}
+static int sort_pairs(fslrc_ctx *ctx, Pipe *P, const unsigned *kin, unsigned *kout, const int *vin, int *vout, int n, int b0, int b1) {
+    return sort_pairs_to(ctx, P, kin, vin, n, b0, b1, prims::PairOut{kout, vout});
 }
 // wait for the context's stream: spinning (lowest latency) or, for contexts driven from several host threads at once
 // (engine.HostPipeline), sleeping on a blocking-sync event so that a waiting thread leaves its core to the others
@@ -248,7 +260,8 @@ static int err_code(fslrc_ctx *ctx) {
 }
 static int bits_for(int64_t n) { int b = 1; while ((1ll << b) < n && b < 32) b++; return b; }
 
-static int pipe_bands(fslrc_ctx *ctx, Pipe *P, const int *s_dp, const int *rmidx, const int *it_q, const int4 *IT0, const int2 *IT1, const int4 *DREC);
+static int alloc_records(fslrc_ctx *ctx, Pipe *P, int **s_m, int **s_end);
+static int pipe_bands(fslrc_ctx *ctx, Pipe *P, const int *s_m, const int *s_end);
 
 // exclusive sum of int64 (k_reads_fast's packed (count << 32 | L) flags)
 static int xscan64(fslrc_ctx *ctx, Pipe *P, const long long *in, long long *out, int n, int64_t *total) {
@@ -301,8 +314,9 @@ static int pipe_ingest_fast(fslrc_ctx *ctx, Pipe *P, const long long *d_clen, co
     cudaStream_t st = ctx->stream;
     const int A = P->A, R = P->R, TB = 256;
     int *flagA, *posA, *qlen2;
-    DA(flagA, A); DA(posA, A); DA(qlen2, R); DA(P->q_of_rid, R);
-    if (R > 0) KL(k_fill<int>, nblk(R, TB), TB, P->q_of_rid, R, -1);
+    long long *QO;                                                          // per read: q << 32 | off, -1 = no interval
+    DA(flagA, A); DA(posA, A); DA(qlen2, R); DA(P->q_of_rid, R); DA(QO, R);
+    if (R > 0) KL(k_fill<long long>, nblk(R, TB), TB, QO, R, -1ll);
     if (A > 0) {
         KL(k_rows_fast, nblk(A, TB), TB, A, R, tb.read_id, tb.chrom, tb.rstart, tb.rend, tb.qstart, tb.qend, pr.n_chrom, d_clen, d_cmask,
            pr.mask_subtelomere, (long long)pr.subtel, flagA, qlen2, (unsigned long long *)(P->cnt + 0), P->err);
@@ -318,9 +332,9 @@ static int pipe_ingest_fast(fslrc_ctx *ctx, Pipe *P, const long long *d_clen, co
     P->F = (int)ctx->h_pin[0];
     const int D = P->D = (int)ctx->h_pin[1];
     { int r = mark(ctx, ST_KEEP); if (r) return r; }
-    int4 *REC, *IT0; unsigned *key, *key2; int *val, *dfill, *ITn; long long *flag64, *qo64, *QO;
-    DA(REC, 2 * (int64_t)D); DA(key, D); DA(key2, D); DA(val, D); DA(dfill, D); DA(IT0, D); DA(ITn, D);
-    DA(flag64, D); DA(qo64, D); DA(QO, R);
+    int4 *REC, *IT0, *IT1; unsigned *key, *key2; int *val, *dfill; long long *flag64, *qo64;
+    DA(REC, 2 * (int64_t)D); DA(key, D); DA(key2, D); DA(val, D); DA(dfill, D); DA(IT0, D); DA(IT1, D);
+    DA(flag64, D); DA(qo64, D);
     unsigned *tkey = nullptr, *tval = nullptr;
     int kbits = 32;
     if (D > 0) {
@@ -333,37 +347,46 @@ static int pipe_ingest_fast(fslrc_ctx *ctx, Pipe *P, const long long *d_clen, co
         for (int c = 0; c < pr.n_chrom; c++) { if (pr.chrom_len[c] <= 0) known = false; mx = std::max<long long>(mx, pr.chrom_len[c]); }
         kbits = (known && mx < 0x7fffffffLL) ? std::min(32, bits_for(mx + 2)) : 32;
         int r = sort_pairs(ctx, P, key, key2, val, dfill, D, 0, kbits); if (r) return r;
-        KL(k_items_fast, nblk(D, TB), TB, D, dfill, REC, IT0, ITn, flag64);
+        KL(k_items_fast, nblk(D, TB), TB, D, dfill, REC, IT0, IT1, flag64);
         DA(tkey, D); DA(tval, D);
-        KL(k_tie_delta, nblk(D, TB), TB, D, IT0, (const int *)dfill, tkey, tval, (unsigned long long *)(P->cnt + 41), P->err);
+        KL(k_tie_delta, nblk(D, TB), TB, D, IT0, tkey, tval, (unsigned long long *)(P->cnt + 41), P->err);
     }
     { int r = mark(ctx, ST_ORDER); if (r) return r; }
     // ---- query rank + read-major offsets from one scan over data order
     DA(P->RI, std::min(R, D));
     if (D > 0) {
         int r = xscan64(ctx, P, flag64, qo64, D, P->cnt + 2); if (r) return r;
-        KL(k_firsts_fast, nblk(D, TB), TB, D, flag64, qo64, IT0, ITn, qlen2, pr.qlen_c, pr.naln_c, QO, P->RI, P->err);
-        KL(k_assign_fast, nblk(D, TB), TB, D, REC, QO, P->q_of_rid);
+        KL(k_firsts_fast, nblk(D, TB), TB, D, flag64, qo64, IT0, IT1, qlen2, pr.qlen_c, pr.naln_c, QO, P->RI, P->err);
     }
-    { int r = read_counts(ctx, P); if (r) return r; r = err_code(ctx); if (r) return r; }
+    if (R > 0) KL(k_q_of_rid, nblk(R, TB), TB, R, QO, P->q_of_rid);
+    { int r = read_counts(ctx, P); if (r) return r; }
     if (kbits < 32 && ((unsigned long long)ctx->h_pin[48] >> kbits) != 0) {   // a start beyond its chromosome's length: the short sort key was
-        CK(cudaMemsetAsync(P->err, 0, sizeof(int), st));                      // wrong, the general path sorts on all 32 bits
-        CK(cudaMemsetAsync(P->cnt, 0, NCNT * sizeof(int64_t), st));
+        CK(cudaMemsetAsync(P->err, 0, sizeof(int), st));                      // wrong (and data order with it: k_tie_delta's EF_RANGE), the
+        CK(cudaMemsetAsync(P->cnt, 0, NCNT * sizeof(int64_t), st));           // general path sorts on all 32 bits
         return 1;
     }
+    { int r = err_code(ctx); if (r) return r; }
     if (D > 0 && (ctx->h_pin[2] & 0xffffffffLL) != D) return fail(ctx, FSLRC_ERR_CUDA, "internal: read-major offsets do not add up");
     P->Q = (int)(ctx->h_pin[2] >> 32);
     { int r = mark(ctx, ST_QRANK); if (r) return r; }
-    int *s_u; DA(s_u, D);
-    const bool tie_ok = tkey && ctx->h_pin[41] == 0;
-    { int r = pipe_chrom_order(ctx, P, IT0, tkey, tval, tie_ok, s_u); if (r) return r; }
-    if (D > 0 && !tie_ok) {                                                        // (the three-sort fallback yields data positions, not filling indices)
-        int *tmp; DA(tmp, D);
-        KL(k_gather_int, nblk(D, TB), TB, D, s_u, dfill, tmp);
-        s_u = tmp;
+    // ---- IntervalMap order and the records of sorted order
+    int *s_m, *s_end;
+    { int r = alloc_records(ctx, P, &s_m, &s_end); if (r) return r; }
+    const FastRec rec{IT0, IT1, QO, P->RI, pr.overlap, P->SR0, P->SR1, s_m, P->s_chrom, s_end};
+    if (D > 0 && ctx->h_pin[41] == 0) {                                      // partition by chromosome, moving the records
+        const int cbits = bits_for(pr.n_chrom);
+        const unsigned *cstart = nullptr;
+        int r = sort_pairs_to(ctx, P, tkey, (const int *)tval, D, 0, cbits, ChromRecOut{rec}, &cstart); if (r) return r;
+        if (cbits <= 8) KL(k_chrom_bounds_digits, 1, 256, pr.n_chrom, D, cstart, P->chrom_lo, P->chrom_hi);
+        else KL(k_chrom_bounds, nblk(D, TB), TB, D, P->s_chrom, P->chrom_lo, P->chrom_hi);
+    } else if (D > 0) {                                                      // long runs of equal (chrom, start): three full sorts
+        int *s_dp; DA(s_dp, D);
+        int r = pipe_chrom_order(ctx, P, IT0, tkey, tval, false, s_dp); if (r) return r;
+        KL(k_records_fast, nblk(D, TB), TB, D, s_dp, rec);
+        KL(k_chrom_bounds, nblk(D, TB), TB, D, P->s_chrom, P->chrom_lo, P->chrom_hi);
     }
     { int r = mark(ctx, ST_CHROM); if (r) return r; }
-    return pipe_bands(ctx, P, s_u, nullptr, nullptr, nullptr, nullptr, REC);
+    return pipe_bands(ctx, P, s_m, s_end);
 }
 
 // ---- stages 1-5: ingestion, orders, records (replicated on every rank)
@@ -434,7 +457,7 @@ static int pipe_prepare(fslrc_ctx *ctx, Pipe *P) {
     if (D > 0) KL(k_build_items, nblk(D, TB), TB, D, dfill, FR0, FR1, IT0, IT1, firstdp, P->err);
     if (D > 0 && D < (1 << 26)) {
         DA(tkey, D); DA(tkey2, D); DA(tval, D); DA(tval2, D);
-        KL(k_tie_delta, nblk(D, TB), TB, D, IT0, (const int *)nullptr, tkey, tval, (unsigned long long *)(P->cnt + 41), P->err);
+        KL(k_tie_delta, nblk(D, TB), TB, D, IT0, tkey, tval, (unsigned long long *)(P->cnt + 41), P->err);
     }
     { int r = mark(ctx, ST_ORDER); if (r) return r; }
     // ---- stage 3: query rank + per-read lists
@@ -463,28 +486,30 @@ static int pipe_prepare(fslrc_ctx *ctx, Pipe *P) {
     int *s_dp; DA(s_dp, D);
     { int r = pipe_chrom_order(ctx, P, IT0, tkey, tval, tkey && ctx->h_pin[41] == 0, s_dp); if (r) return r; }   // (flag read back with the stage-3 counters)
     { int r = mark(ctx, ST_CHROM); if (r) return r; }
-    return pipe_bands(ctx, P, s_dp, rmidx, it_q, IT0, IT1, nullptr);
+    int *s_m, *s_end;
+    { int r = alloc_records(ctx, P, &s_m, &s_end); if (r) return r; }
+    if (D >= (1 << 26)) return fail(ctx, FSLRC_ERR_RANGE, "more than 2^26 intervals");
+    if (D > 0) KL(k_records, nblk(D, TB), TB, D, s_dp, rmidx, it_q, IT0, IT1, P->RI, pr.overlap, P->SR0, P->SR1,
+                  s_m, P->s_chrom, s_end, P->chrom_lo, P->chrom_hi, P->err);
+    return pipe_bands(ctx, P, s_m, s_end);
 }
 
-// ---- stage 5: records, thresholds, bands; sizes of the pair stage's buffers
-static int pipe_bands(fslrc_ctx *ctx, Pipe *P, const int *s_dp, const int *rmidx, const int *it_q, const int4 *IT0, const int2 *IT1, const int4 *DREC) {
+// ---- records of sorted order (written by the ingest that computed the order): SR0, SR1, s_m, s_chrom, s_end, chrom bounds
+static int alloc_records(fslrc_ctx *ctx, Pipe *P, int **s_m, int **s_end) {
+    const int D = P->D, nc = P->pr.n_chrom;
+    cudaStream_t st = ctx->stream;
+    DA(P->SR0, D); DA(P->SR1, D); DA(P->s_chrom, D); DA(*s_end, D); DA(*s_m, D);
+    DA(P->chrom_lo, nc); DA(P->chrom_hi, nc);
+    if (nc > 0) { CK(cudaMemsetAsync(P->chrom_lo, 0, sizeof(int) * nc, st)); CK(cudaMemsetAsync(P->chrom_hi, 0, sizeof(int) * nc, st)); }
+    return 0;
+}
+// ---- stage 5: thresholds, bands; sizes of the pair stage's buffers
+static int pipe_bands(fslrc_ctx *ctx, Pipe *P, const int *s_m, const int *s_end) {
     const fslrc_params &pr = P->pr;
     cudaStream_t st = ctx->stream;
-    const int D = P->D, Q = P->Q, TB = 256;
-    int *s_end;
-    DA(P->SR0, D); DA(P->SR1, D); DA(P->RM, 2 * (int64_t)D); DA(P->s_chrom, D); DA(s_end, D);
-    DA(P->pmaxS, D); DA(P->chrom_lo, pr.n_chrom); DA(P->chrom_hi, pr.n_chrom);
-    if (pr.n_chrom > 0) { CK(cudaMemsetAsync(P->chrom_lo, 0, sizeof(int) * pr.n_chrom, st)); CK(cudaMemsetAsync(P->chrom_hi, 0, sizeof(int) * pr.n_chrom, st)); }
-    DA(P->rclass, Q);
+    const int D = P->D, Q = P->Q;
+    DA(P->RM, 2 * (int64_t)D); DA(P->pmaxS, D); DA(P->rclass, Q);
     if (D > 0) {
-        if (D >= (1 << 26)) return fail(ctx, FSLRC_ERR_RANGE, "more than 2^26 intervals");
-        int *s_m; DA(s_m, D);
-        if (DREC) {                                                                // fast ingest: s_dp holds filling indices, DREC the packed records
-            KL(k_records_fast, nblk(D, TB), TB, D, s_dp, DREC, P->RI, pr.overlap, P->SR0, P->SR1, s_m, P->s_chrom, s_end);
-            KL(k_chrom_bounds, nblk(D, TB), TB, D, P->s_chrom, P->chrom_lo, P->chrom_hi);
-        }
-        else KL(k_records, nblk(D, TB), TB, D, s_dp, rmidx, it_q, IT0, IT1, P->RI, pr.overlap, P->SR0, P->SR1,
-                                               s_m, P->s_chrom, s_end, P->chrom_lo, P->chrom_hi, P->err);
         int r = segmax_scan(ctx, P, P->s_chrom, s_end, P->pmaxS, D); if (r) return r;
         CK(cudaMemsetAsync(P->rclass, 0, sizeof(int) * (size_t)std::max(Q, 1), st));
         KL(k_bands, nblk(D, 256), 256, D, P->SR0, s_m, P->s_chrom, P->pmaxS, P->chrom_lo, P->chrom_hi, P->RM, P->rclass,
@@ -796,7 +821,8 @@ int fslrc_create(int device, fslrc_ctx **out) {
     if (cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking) != cudaSuccess) { ctx->copy_stream = nullptr; cudaGetLastError(); }
     cudaEventCreateWithFlags(&ctx->ev_c1, cudaEventDisableTiming);
     cudaEventCreateWithFlags(&ctx->ev_c2, cudaEventDisableTiming);
-    cudaFuncSetAttribute(prims::k_rs_onesweep, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(prims::RsSmem));
+    cudaFuncSetAttribute(prims::k_rs_onesweep<prims::PairOut>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(prims::RsSmem));
+    cudaFuncSetAttribute(prims::k_rs_onesweep<ChromRecOut>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(prims::RsSmem));
     cudaMemPool_t pool;                                   // keep freed scratch cached between calls
     if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
         uint64_t thr = UINT64_MAX;

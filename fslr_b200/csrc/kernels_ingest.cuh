@@ -191,8 +191,7 @@ __global__ void k_gather_key(int D, const int *__restrict__ dp_in, const int4 *_
 // as a block, so the item's final position is its partition position + (rank - idx).  val[d] = d | (rank - idx + 32) << 26.
 // Runs that do not fit the window raise `overflow` and the caller falls back to the two full radix sorts.
 #define TIE_WIN 48
-// vmap (optional): the value sent through the partition is vmap[d] instead of d (fast ingest: the filling index)
-__global__ void k_tie_delta(int D, const int4 *__restrict__ IT0, const int *__restrict__ vmap, unsigned *ckey, unsigned *val,
+__global__ void k_tie_delta(int D, const int4 *__restrict__ IT0, unsigned *ckey, unsigned *val,
                             unsigned long long *overflow, int *err) {
     int d = blockIdx.x * blockDim.x + threadIdx.x;
     if (d >= D) return;
@@ -217,7 +216,7 @@ __global__ void k_tie_delta(int D, const int4 *__restrict__ IT0, const int *__re
     if (idx > 31 || rank > 31) ovf = true;
     if (ovf) { atomicAdd(overflow, 1ull); rank = idx; }
     ckey[d] = (unsigned)me.y;
-    val[d] = (unsigned)(vmap ? vmap[d] : d) | ((unsigned)(rank - idx + 32) << 26);
+    val[d] = (unsigned)d | ((unsigned)(rank - idx + 32) << 26);
 }
 __global__ void k_apply_delta(int D, const unsigned *__restrict__ val, int *s_dp) {
     int p = blockIdx.x * blockDim.x + threadIdx.x;
@@ -359,7 +358,7 @@ __global__ void k_rows_fast(int A, int R, const int *__restrict__ rid_, const in
     if (threadIdx.x == 0 && cnt) atomicAdd(n_fillings, (unsigned long long)cnt);
 }
 // unmasked fillings in bed order, one 32-byte sector each: REC[2u] = {read_id, chrom, start, end},
-// REC[2u+1] = {aln_size, n_alignments, q | fi << 26, m} (.z/.w filled in by k_assign_fast); sort key = start
+// REC[2u+1] = {aln_size, n_alignments, fi, L}; sort key = start
 __global__ void k_compact_fast(int A, const int *__restrict__ flag, const int *__restrict__ pos, const int *__restrict__ rid,
                                const int *__restrict__ chrom, const int *__restrict__ rstart, const int *__restrict__ rend,
                                const int *__restrict__ aln, const int *__restrict__ naln, int4 *REC, unsigned *key, int *val,
@@ -390,7 +389,7 @@ __global__ void k_compact_fast(int A, const int *__restrict__ flag, const int *_
         }
         if (over) { atomicOr(err, EF_TOOMANY); L = LMAX; fi &= 63; }
         REC[2 * u] = make_int4(r, chrom[i], s, max(rs, re));
-        REC[2 * u + 1] = make_int4(a, na, fi, L);                                   // .zw = {fi, L} until k_assign_fast overwrites them
+        REC[2 * u + 1] = make_int4(a, na, fi, L);
         key[u] = (unsigned)s; val[u] = u;
     }
     __shared__ int s_max;                                                           // one atomic per block, and only when it can matter
@@ -401,22 +400,23 @@ __global__ void k_compact_fast(int A, const int *__restrict__ flag, const int *_
     __syncthreads();
     if (threadIdx.x == 0 && (unsigned long long)s_max > *(volatile unsigned long long *)max_start) atomicMax(max_start, (unsigned long long)s_max);
 }
-// per data position d (filling u = dfill[d]): the filling's record, gathered as one sector, written out coalesced;
+// per data position d (filling u = dfill[d]): the filling's record, gathered as one sector — the one random permutation of
+// the fast ingest — and written out coalesced in data order (IT0[d] = REC[2u], IT1[d] = REC[2u+1]);
 // flag64[d] = (1 << 32 | L) when the filling is its read's first item in data order (fi == 0), else 0
-__global__ void k_items_fast(int D, const int *__restrict__ dfill, const int4 *__restrict__ REC, int4 *IT0, int *ITn, long long *flag64) {
+__global__ void k_items_fast(int D, const int *__restrict__ dfill, const int4 *__restrict__ REC, int4 *IT0, int4 *IT1, long long *flag64) {
     const int d = blockIdx.x * blockDim.x + threadIdx.x;
     if (d >= D) return;
     const int u = dfill[d];
     const int4 r0 = REC[2 * u], r1 = REC[2 * u + 1];                                // (one sector) r1 = {aln_size, n_alignments, fi, L}
     IT0[d] = r0;
-    ITn[d] = r1.y;
+    IT1[d] = r1;
     flag64[d] = r1.z == 0 ? ((1ll << 32) | (long long)r1.w) : 0ll;
 }
 // the read's first item in data order knows the read's query rank q and read-major offset `off` (the scan at its position):
-// QO[read_id] = (q << 32 | off) — the only scattered write of the fast ingest, one per query read — and RI[q] (k_read_info;
-// consecutive first items write consecutive q)
+// QO[read_id] = (q << 32 | off) — the only scattered write of the fast ingest, one per query read — and RI[q]
+// (k_read_info; consecutive first items write consecutive q)
 __global__ void k_firsts_fast(int D, const long long *__restrict__ flag64, const long long *__restrict__ qo64, const int4 *__restrict__ IT0,
-                              const int *__restrict__ ITn, const int *__restrict__ qlen2, double qlen_c,
+                              const int4 *__restrict__ IT1, const int *__restrict__ qlen2, double qlen_c,
                               double naln_c, long long *QO, int4 *RI, int *err) {
     const int d = blockIdx.x * blockDim.x + threadIdx.x;
     if (d >= D) return;
@@ -425,41 +425,46 @@ __global__ void k_firsts_fast(int D, const long long *__restrict__ flag64, const
     const long long qo = qo64[d];
     const int q = (int)(qo >> 32), off = (int)(qo & 0xffffffffll), L = (int)(fl & 0xffffffffll), rid = IT0[d].x;
     QO[rid] = qo;
-    int ql = qlen2[rid], na = ITn[d];
+    int ql = qlen2[rid], na = IT1[d].y;
     if (ql <= 0 || na <= 0) { atomicOr(err, EF_ZERO); ql = ql <= 0 ? 1 : ql; na = na <= 0 ? 1 : na; }
     int Ln = thr_f64(na, naln_c);
     if (Ln > 65535) Ln = 65535;
     RI[q] = make_int4(ql, thr_f64(ql, qlen_c), (na & 0xffff) | (Ln << 16), (int)(((unsigned)off << 6) | (unsigned)((L - 1) & 63)));
 }
-// per filling in bed order (coalesced: the reads are contiguous and QO is indexed by the non-decreasing read id): its query
-// rank, its index fi in the read's list and its read-major index m = off + fi into REC[2u+1].zw; q_of_rid
-__global__ void k_assign_fast(int D, int4 *REC, const long long *__restrict__ QO, int *q_of_rid) {
-    const int u = blockIdx.x * blockDim.x + threadIdx.x;
-    if (u >= D) return;
-    const int rid = REC[2 * u].x;
-    int4 r1 = REC[2 * u + 1];
-    const int fi = r1.z;
-    const long long qo = QO[rid];
-    const int q = (int)(qo >> 32), off = (int)(qo & 0xffffffffll);
-    r1.z = (int)((unsigned)q | ((unsigned)(fi & 63) << 26)); r1.w = off + fi;
-    REC[2 * u + 1] = r1;
-    if (u == 0 || REC[2 * (u - 1)].x != rid) q_of_rid[rid] = q;
+// q_of_rid from QO (filled with -1 beforehand), coalesced: a second scattered 4-byte write in k_firsts_fast costs ~10x this
+__global__ void k_q_of_rid(int R, const long long *__restrict__ QO, int *q_of_rid) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r < R) q_of_rid[r] = (int)(QO[r] >> 32);
 }
-// sorted order: one sector gather per position
-__global__ void k_records_fast(int D, const int *__restrict__ s_u, const int4 *__restrict__ REC, const int4 *__restrict__ RI, double overlap,
-                               int4 *SR0, int4 *SR1, int *s_m, int *s_chrom, int *s_end) {
+// sorted position p of data position d: SR0[p] = {start, end, T, q | fi << 26}, SR1[p] = RI[q], s_m[p] = m = off + fi
+// (the read's query rank and read-major offset come from QO: 8 bytes per read, mostly L2 hits)
+struct FastRec {
+    const int4 *IT0, *IT1; const long long *QO; const int4 *RI; double overlap;
+    int4 *SR0, *SR1; int *s_m, *s_chrom, *s_end;
+    __device__ __forceinline__ void operator()(int p, int d) const {
+        const int4 r0 = __ldg(&IT0[d]), r1 = __ldg(&IT1[d]);                         // r1 = {aln_size, n_alignments, fi, L}
+        const long long qo = __ldg(&QO[r0.x]);
+        const int q = (int)(qo >> 32), off = (int)(qo & 0xffffffffll);
+        SR0[p] = make_int4(r0.z, r0.w, thr_f64(max(r1.x, 1), overlap), (int)((unsigned)q | ((unsigned)(r1.z & 63) << 26)));
+        SR1[p] = __ldg(&RI[q]);
+        s_m[p] = off + r1.z;
+        s_chrom[p] = r0.y; s_end[p] = r0.w;
+    }
+};
+// IntervalMap order in one move of the records: the last pass of the stable partition of data order by chromosome
+// (key = chrom, val = k_tie_delta's d | (shift + 32) << 26) writes the record of d straight to its final position, the
+// partition position moved by the tie shift.  The pass hands over global partition positions, so a run of equal
+// (chrom, start) that straddles tiles lands exactly where k_tie_delta's shift expects it.
+struct ChromRecOut {
+    FastRec rec;
+    __device__ __forceinline__ void operator()(unsigned g, unsigned, int val) const {
+        rec((int)g + (int)((unsigned)val >> 26) - 32, val & QMASK);
+    }
+};
+// the same records from a list of data positions (IntervalMap order by the three full sorts)
+__global__ void k_records_fast(int D, const int *__restrict__ s_dp, FastRec rec) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= D) return;
-    const int u = s_u[p];
-    const int4 r0 = REC[2 * u], r1 = REC[2 * u + 1];
-    SR0[p] = make_int4(r0.z, r0.w, thr_f64(max(r1.x, 1), overlap), r1.z);
-    SR1[p] = RI[r1.z & QMASK];
-    s_m[p] = r1.w;
-    s_chrom[p] = r0.y; s_end[p] = r0.w;
-}
-__global__ void k_gather_int(int n, const int *__restrict__ idx, const int *__restrict__ src, int *dst) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) dst[i] = src[idx[i]];
+    if (p < D) rec(p, s_dp[p]);
 }
 __global__ void k_chrom_bounds(int D, const int *__restrict__ s_chrom, int *chrom_lo, int *chrom_hi) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
@@ -467,5 +472,12 @@ __global__ void k_chrom_bounds(int D, const int *__restrict__ s_chrom, int *chro
     const int c = s_chrom[p];
     if (p == 0 || s_chrom[p - 1] != c) chrom_lo[c] = p;
     if (p == D - 1 || s_chrom[p + 1] != c) chrom_hi[c] = p + 1;
+}
+// the same bounds from the digit starts of a one-pass partition by chromosome (start[c]: first position of chromosome c)
+__global__ void k_chrom_bounds_digits(int n_chrom, int D, const unsigned *__restrict__ start, int *chrom_lo, int *chrom_hi) {
+    const int c = threadIdx.x;
+    if (c >= n_chrom) return;
+    const unsigned e = c + 1 < 256 ? start[c + 1] : (unsigned)D;
+    if (e > start[c]) { chrom_lo[c] = (int)start[c]; chrom_hi[c] = (int)e; }
 }
 

@@ -247,9 +247,15 @@ struct RsSmem {
     unsigned keys[RS_TILE];
     int vals[RS_TILE];
 };
-__global__ void __launch_bounds__(RS_THREADS, RS_MINB) k_rs_onesweep(const unsigned *__restrict__ kin, unsigned *__restrict__ kout,
-                                                            const int *__restrict__ vin, int *__restrict__ vout, int n, int shift,
-                                                            int mask, const unsigned *__restrict__ gbase, unsigned *status, unsigned *ticket) {
+// where a pass puts pair (key, val) of output position g: the next pass's key / value arrays, or (last pass) a caller's sink
+struct PairOut {
+    unsigned *kout; int *vout;
+    __device__ __forceinline__ void operator()(unsigned g, unsigned key, int val) const { kout[g] = key; vout[g] = val; }
+};
+template <typename Out>
+__global__ void __launch_bounds__(RS_THREADS, RS_MINB) k_rs_onesweep(const unsigned *__restrict__ kin, const int *__restrict__ vin, Out out,
+                                                            int n, int shift, int mask, const unsigned *__restrict__ gbase,
+                                                            unsigned *status, unsigned *ticket) {
     extern __shared__ __align__(16) unsigned char rs_raw[];
     RsSmem &sm = *reinterpret_cast<RsSmem *>(rs_raw);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -336,9 +342,7 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MINB) k_rs_onesweep(const unsig
         if (pos < valid) {
             const unsigned k = sm.keys[pos];
             const unsigned d = (k >> shift) & (unsigned)mask;
-            const unsigned g = sm.gofs[d] + (unsigned)pos;
-            kout[g] = k;
-            vout[g] = sm.vals[pos];
+            out(sm.gofs[d] + (unsigned)pos, k, sm.vals[pos]);
         }
     }
 }
