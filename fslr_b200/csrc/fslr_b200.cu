@@ -799,6 +799,35 @@ static int run_device(fslrc_ctx *ctx, Pipe *P, int32_t *oc, int32_t *on, fslrc_s
     return 0;
 }
 
+// choose_alignment (cluster.py:237-254) on device columns: per read the sum and count of alignment_score over its rows,
+// per cluster the read with the highest mean, the one whose first row comes first on ties.  is_rep[r] = 1 for those
+// reads; rep_read (nullable) receives each cluster's.  A read id >= R or a cluster id outside [0, C) sets EF_RANGE in *err.
+static int choose_alignment_dev(fslrc_ctx *ctx, int A, int R, int C, const int *rid, const int *score, const int *cluster,
+                                long long *sum, int *cnt, unsigned char *is_rep, int *rep_read, int *err) {
+    cudaStream_t st = ctx->stream;
+    const int TB = 256;
+    int *first, *minrow; unsigned long long *best;
+    DA(first, R); DA(minrow, C); DA(best, C);
+    if (R > 0) {
+        CK(cudaMemsetAsync(cnt, 0, sizeof(int) * R, st));
+        CK(cudaMemsetAsync(sum, 0, sizeof(long long) * R, st));
+        KL(k_fill<int>, nblk(R, TB), TB, first, R, 0x7fffffff);
+    }
+    if (C > 0) {
+        CK(cudaMemsetAsync(best, 0, sizeof(unsigned long long) * C, st));
+        KL(k_fill<int>, nblk(C, TB), TB, minrow, C, 0x7fffffff);
+        if (rep_read) KL(k_fill<int>, nblk(C, TB), TB, rep_read, C, -1);
+    }
+    CK(cudaMemsetAsync(err, 0, sizeof(int), st));
+    if (A > 0) KL(k_ca_rows, nblk(A, TB), TB, A, R, rid, score, sum, cnt, first, err);
+    if (R > 0) {
+        KL(k_ca_best, nblk(R, TB), TB, R, C, sum, cnt, cluster, best, err);
+        KL(k_ca_first, nblk(R, TB), TB, R, C, sum, cnt, first, cluster, best, minrow);
+        KL(k_ca_flag, nblk(R, TB), TB, R, C, cnt, first, cluster, minrow, is_rep, rep_read);
+    }
+    return 0;
+}
+
 extern "C" {
 
 int fslrc_version(void) { return FSLRC_VERSION; }
@@ -989,32 +1018,16 @@ int fslrc_choose_alignment_host(fslrc_ctx *ctx, int64_t n_rows, int64_t n_reads,
     CK(cudaSetDevice(ctx->device));
     ctx->stream = (cudaStream_t)stream;
     cudaStream_t st = ctx->stream;
-    const int A = (int)n_rows, R = (int)n_reads, C = (int)n_clusters, TB = 256;
-    int *d_rid, *d_sc, *d_cl, *cnt, *first, *minrow, *rep, *err; long long *sum; unsigned long long *best; unsigned char *flag;
-    DA(d_rid, A); DA(d_sc, A); DA(d_cl, R); DA(cnt, R); DA(first, R); DA(minrow, C); DA(rep, C); DA(err, 1); DA(sum, R); DA(best, C); DA(flag, R);
+    const int A = (int)n_rows, R = (int)n_reads, C = (int)n_clusters;
+    int *d_rid, *d_sc, *d_cl, *cnt, *rep, *err; long long *sum; unsigned char *flag;
+    DA(d_rid, A); DA(d_sc, A); DA(d_cl, R); DA(cnt, R); DA(rep, C); DA(err, 1); DA(sum, R); DA(flag, R);
     if (A > 0) {
         CK(cudaMemcpyAsync(d_rid, read_id, sizeof(int) * A, cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(d_sc, alignment_score, sizeof(int) * A, cudaMemcpyHostToDevice, st));
     }
-    if (R > 0) {
-        CK(cudaMemcpyAsync(d_cl, cluster, sizeof(int) * R, cudaMemcpyHostToDevice, st));
-        CK(cudaMemsetAsync(cnt, 0, sizeof(int) * R, st));
-        CK(cudaMemsetAsync(sum, 0, sizeof(long long) * R, st));
-        KL(k_fill<int>, nblk(R, TB), TB, first, R, 0x7fffffff);
-    }
-    if (C > 0) {
-        CK(cudaMemsetAsync(best, 0, sizeof(unsigned long long) * C, st));
-        KL(k_fill<int>, nblk(C, TB), TB, minrow, C, 0x7fffffff);
-        KL(k_fill<int>, nblk(C, TB), TB, rep, C, -1);
-    }
-    CK(cudaMemsetAsync(err, 0, sizeof(int), st));
-    if (A > 0) KL(k_ca_rows, nblk(A, TB), TB, A, R, d_rid, d_sc, sum, cnt, first, err);
-    if (R > 0) {
-        KL(k_ca_best, nblk(R, TB), TB, R, C, sum, cnt, d_cl, best, err);
-        KL(k_ca_first, nblk(R, TB), TB, R, C, sum, cnt, first, d_cl, best, minrow);
-        KL(k_ca_flag, nblk(R, TB), TB, R, C, cnt, first, d_cl, minrow, flag, rep);
-        CK(cudaMemcpyAsync(out_is_rep, flag, R, cudaMemcpyDeviceToHost, st));
-    }
+    if (R > 0) CK(cudaMemcpyAsync(d_cl, cluster, sizeof(int) * R, cudaMemcpyHostToDevice, st));
+    { int r = choose_alignment_dev(ctx, A, R, C, d_rid, d_sc, d_cl, sum, cnt, flag, rep, err); if (r) return r; }
+    if (R > 0) CK(cudaMemcpyAsync(out_is_rep, flag, R, cudaMemcpyDeviceToHost, st));
     if (C > 0 && out_rep_read) CK(cudaMemcpyAsync(out_rep_read, rep, sizeof(int) * C, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(ctx->h_pin + 60, err, sizeof(int), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
@@ -1222,6 +1235,53 @@ int fslrc_tsv_write_cluster_bed(fslrc_ctx *ctx, const int32_t *cluster_dev, cons
             unsigned char *d_out; DA(d_out, *n_out);
             KL(tsv::k_tsv_emit, nblk((int64_t)L * 32, TB), TB, L, T->text, T->line_start, T->read_id, cluster_dev, n_reads_dev, any_single, off, d_out);
             CK(cudaMemcpyAsync(out, d_out, *n_out, cudaMemcpyDeviceToHost, st));
+        }
+    }
+    free_all(ctx);
+    CK(cudaStreamSynchronize(st));
+    return rc;
+}
+int fslrc_tsv_write_representative_bed(fslrc_ctx *ctx, const int32_t *cluster_dev, const int32_t *n_reads_dev, char *out,
+                                       int64_t cap, int64_t *n_out, void *stream) {
+    if (!ctx || !ctx->tsv || !cluster_dev || !n_reads_dev || !n_out) return FSLRC_ERR_ARG;
+    TsvState *T = ctx->tsv;
+    if (!T->score) return fail(ctx, FSLRC_ERR_ARG, "tsv: the table has no alignment_score column");
+    CK(cudaSetDevice(ctx->device));
+    ctx->stream = (cudaStream_t)stream;
+    cudaStream_t st = ctx->stream;
+    Pipe Pp; memset((void *)&Pp, 0, sizeof(Pp)); Pipe *P = &Pp;
+    const int L = T->n_lines, R = T->n_reads, TB = 256;
+    long long *sum, *len, *off; int *cnt, *err, *any_single, *txt_len; unsigned char *is_rep; char *txt; int64_t *tot;
+    DA(sum, R); DA(cnt, R); DA(is_rep, R); DA(txt_len, R); DA(txt, (int64_t)R * fmtd::FMT_F64_MAX); DA(err, 1); DA(any_single, 1);
+    DA(len, L); DA(off, L); DA(tot, 1);
+    // cluster ids of the clustering are < n_reads, so n_reads bounds them without a read-back; ids from elsewhere are checked
+    { int r = choose_alignment_dev(ctx, T->n_rows, R, R, T->read_id, T->score, cluster_dev, sum, cnt, is_rep, nullptr, err); if (r) return r; }
+    CK(cudaMemsetAsync(any_single, 0, sizeof(int), st));
+    if (R > 0) {
+        KL(tsv::k_tsv_any_single, nblk(R, TB), TB, R, n_reads_dev, any_single);
+        KL(tsv::k_tsv_rep_mean, nblk(R, TB), TB, R, is_rep, sum, cnt, txt, txt_len);
+    }
+    KL(tsv::k_tsv_rep_outlen, nblk(L, TB), TB, L, T->line_start, T->read_id, cluster_dev, n_reads_dev, any_single, is_rep, txt_len, len);
+    {
+        const int tiles = nblk(L, prims::SC_TILE);
+        int r = prim_scratch(ctx, P, sizeof(unsigned long long) * tiles); if (r) return r;
+        KL(prims::k_scan_excl<long long>, tiles, prims::SC_THREADS, len, off, L, (unsigned long long *)(P->prim + 256), (unsigned *)P->prim, (long long *)tot);
+    }
+    CK(cudaMemcpyAsync(ctx->h_pin, tot, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(ctx->h_pin + 1, err, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    int rc = 0;
+    if ((int)(ctx->h_pin[1] & 0xffffffff)) rc = fail(ctx, FSLRC_ERR_RANGE, "tsv: a cluster id is negative or not below n_reads");
+    else {
+        *n_out = ctx->h_pin[0];
+        if (out) {
+            if (cap < *n_out) rc = fail(ctx, FSLRC_ERR_ARG, "tsv: output buffer too small");
+            else {
+                unsigned char *d_out; DA(d_out, *n_out);
+                KL(tsv::k_tsv_rep_emit, nblk((int64_t)L * 32, TB), TB, L, T->text, T->line_start, T->read_id, cluster_dev, n_reads_dev,
+                   any_single, is_rep, txt, txt_len, off, d_out);
+                CK(cudaMemcpyAsync(out, d_out, *n_out, cudaMemcpyDeviceToHost, st));
+            }
         }
     }
     free_all(ctx);

@@ -8,9 +8,13 @@
 //                               byte-for-byte verification against that row, dense ids in order of first appearance
 //                               (= pandas.factorize = the singleton numbering order of main.py:336-341)
 //   k_tsv_outlen / k_tsv_emit   every input line + "\t<cluster>.0\t<n_reads>.0" (the float columns of main.py:334-342)
+//   k_tsv_rep_mean / k_tsv_rep_outlen / k_tsv_rep_emit
+//                               `<base>.mappings.representative.bed` (main.py:351-352): the lines of every cluster's
+//                               representative read only, + the same two columns + repr(mean alignment_score)
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "fmt_double.cuh"
 
 namespace tsv {
 
@@ -166,6 +170,14 @@ __global__ void k_tsv_any_single(int n_reads, const int *__restrict__ nreads, in
     const bool s = r < n_reads && nreads[r] == 1;
     if (__syncthreads_or(s) && threadIdx.x == 0) *any_single = 1;
 }
+// the columns both files append to a data line: "\t<c>.0\t<n>.0" (floats) or "\t<c>\t<n>"
+__device__ __forceinline__ int cluster_cols_len(int c, int n, bool fl) { return 2 + dec_digits(c) + dec_digits(n) + (fl ? 4 : 0); }
+__device__ __forceinline__ unsigned char *put_cluster_cols(unsigned char *q, int c, int n, bool fl) {
+    *q++ = '\t'; q = put_dec(q, c); if (fl) { *q++ = '.'; *q++ = '0'; }
+    *q++ = '\t'; q = put_dec(q, n); if (fl) { *q++ = '.'; *q++ = '0'; }
+    return q;
+}
+__device__ __forceinline__ unsigned char *put_str(unsigned char *q, const char *h) { while (*h) *q++ = (unsigned char)*h++; return q; }
 // output length of every line: header + "\tcluster\tn_reads\n"; row: line + "\t<c>.0\t<n>.0\n" (floats) or "\t<c>\t<n>\n"
 __global__ void k_tsv_outlen(int n_lines, const long long *__restrict__ line_start, const int *__restrict__ rid,
                              const int *__restrict__ cluster, const int *__restrict__ nreads, const int *__restrict__ any_single,
@@ -173,9 +185,8 @@ __global__ void k_tsv_outlen(int n_lines, const long long *__restrict__ line_sta
     const int l = blockIdx.x * blockDim.x + threadIdx.x;
     if (l >= n_lines) return;
     const long long body = line_start[l + 1] - 1 - line_start[l];
-    const int frac = *any_single ? 2 : 0;
     if (l == 0) len[l] = body + 17;                                     // "\tcluster\tn_reads\n"
-    else { const int r = rid[l - 1]; len[l] = body + 1 + dec_digits(cluster[r]) + frac + 1 + dec_digits(nreads[r]) + frac + 1; }
+    else { const int r = rid[l - 1]; len[l] = body + cluster_cols_len(cluster[r], nreads[r], *any_single != 0) + 1; }
 }
 // one warp per line: coalesced byte copy, lane 0 appends the two columns
 __global__ void k_tsv_emit(int n_lines, const unsigned char *__restrict__ text, const long long *__restrict__ line_start,
@@ -190,13 +201,55 @@ __global__ void k_tsv_emit(int n_lines, const unsigned char *__restrict__ text, 
     for (long long i = lane; i < body; i += 32) o[i] = text[s + i];
     if (lane == 0) {
         unsigned char *q = o + body;
-        if (l == 0) { const char *h = "\tcluster\tn_reads\n"; for (int i = 0; i < 17; i++) q[i] = (unsigned char)h[i]; }
+        if (l == 0) put_str(q, "\tcluster\tn_reads\n");
+        else { const int r = rid[l - 1]; q = put_cluster_cols(q, cluster[r], nreads[r], *any_single != 0); *q = '\n'; }
+    }
+}
+// ---- mappings.representative.bed (cluster.py:237-254): is_rep / sum / cnt per read come from the k_ca_* kernels
+constexpr int REP_HEADER_LEN = 37;                                      // "\tcluster\tn_reads\tavg_alignment_score\n"
+// the mean of every representative read, formatted once per read into a fixed slot: repr(sum / cnt) (pandas' to_csv of
+// the float64 column; the same IEEE division k_ca_best ranks the reads by)
+__global__ void k_tsv_rep_mean(int n_reads, const unsigned char *__restrict__ is_rep, const long long *__restrict__ sum,
+                               const int *__restrict__ cnt, char *txt, int *txt_len) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n_reads || !is_rep[r]) return;
+    txt_len[r] = fmtd::fmt_repr_f64(__ddiv_rn((double)sum[r], (double)cnt[r]), txt + (long long)r * fmtd::FMT_F64_MAX);
+}
+// output length of every line: 0 for the lines of a read that is not its cluster's representative
+__global__ void k_tsv_rep_outlen(int n_lines, const long long *__restrict__ line_start, const int *__restrict__ rid,
+                                 const int *__restrict__ cluster, const int *__restrict__ nreads, const int *__restrict__ any_single,
+                                 const unsigned char *__restrict__ is_rep, const int *__restrict__ txt_len, long long *len) {
+    const int l = blockIdx.x * blockDim.x + threadIdx.x;
+    if (l >= n_lines) return;
+    const long long body = line_start[l + 1] - 1 - line_start[l];
+    if (l == 0) { len[l] = body + REP_HEADER_LEN; return; }
+    const int r = rid[l - 1];
+    len[l] = is_rep[r] ? body + cluster_cols_len(cluster[r], nreads[r], *any_single != 0) + 1 + txt_len[r] + 1 : 0;
+}
+// one warp per kept line: coalesced byte copy, lane 0 appends the cluster columns and the formatted mean
+__global__ void k_tsv_rep_emit(int n_lines, const unsigned char *__restrict__ text, const long long *__restrict__ line_start,
+                               const int *__restrict__ rid, const int *__restrict__ cluster, const int *__restrict__ nreads,
+                               const int *__restrict__ any_single, const unsigned char *__restrict__ is_rep,
+                               const char *__restrict__ txt, const int *__restrict__ txt_len, const long long *__restrict__ out_off,
+                               unsigned char *out) {
+    const long long wg = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (wg >= n_lines) return;
+    const int l = (int)wg;
+    const int r = l > 0 ? rid[l - 1] : -1;
+    if (l > 0 && !is_rep[r]) return;
+    const long long s = line_start[l], body = line_start[l + 1] - 1 - s;
+    unsigned char *o = out + out_off[l];
+    for (long long i = lane; i < body; i += 32) o[i] = text[s + i];
+    if (lane == 0) {
+        unsigned char *q = o + body;
+        if (l == 0) put_str(q, "\tcluster\tn_reads\tavg_alignment_score\n");
         else {
-            const int r = rid[l - 1];
-            const bool fl = *any_single != 0;
-            *q++ = '\t'; q = put_dec(q, cluster[r]); if (fl) { *q++ = '.'; *q++ = '0'; }
-            *q++ = '\t'; q = put_dec(q, nreads[r]); if (fl) { *q++ = '.'; *q++ = '0'; }
-            *q++ = '\n';
+            q = put_cluster_cols(q, cluster[r], nreads[r], *any_single != 0);
+            *q++ = '\t';
+            const char *m = txt + (long long)r * fmtd::FMT_F64_MAX;
+            for (int i = 0; i < txt_len[r]; i++) *q++ = (unsigned char)m[i];
+            *q = '\n';
         }
     }
 }

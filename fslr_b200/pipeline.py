@@ -16,7 +16,8 @@ from .table import ColumnarTable
 def cluster_step_fast(bed_path, chr_lengths, out_base, cluster_mask="subtelomere", jaccard_cutoffs="1,1,0.66,0.66,0.66,0.5",
                       overlap=0.8, n_alignment_diff=0.25, qlen_diff=0.04, representative=True, device=0):
     """The same block with the table never leaving the GPU between the file bytes and the output bytes (fslr_b200.tsv):
-    GPU TSV parse -> clustering on the device-resident columns -> GPU rendering of `<out_base>.mappings.cluster.bed`.
+    GPU TSV parse -> clustering on the device-resident columns -> GPU rendering of `<out_base>.mappings.cluster.bed` and
+    (representative=True) `<out_base>.mappings.representative.bed`.
     Tie order of equal starts is the GPU's stable one (ids equal the reference's whenever its unstable sort keeps ties in
     table order, the partition always).  Returns the ClusterResult, or None for main.py:247-249's early return."""
     from . import tsv
@@ -28,12 +29,9 @@ def cluster_step_fast(bed_path, chr_lengths, out_base, cluster_mask="subtelomere
         if res.no_clusters:
             print("No clusters were found.", file=sys.stderr)                    # main.py:247-249
             return None
-        out = pb.cluster_bed_bytes()
-        out.tofile(f"{out_base}.mappings.cluster.bed")                           # main.py:349
+        pb.write_cluster_bed(f"{out_base}.mappings.cluster.bed")                 # main.py:349
         if representative:                                                       # main.py:351-352
-            import io
-            rep = gcluster.choose_alignment(pd.read_csv(io.BytesIO(out.tobytes()), sep="\t"), device=device)
-            rep.to_csv(f"{out_base}.mappings.representative.bed", index=False, sep="\t")
+            pb.write_representative_bed(f"{out_base}.mappings.representative.bed")
         return res
     finally:
         pb.close()

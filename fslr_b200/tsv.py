@@ -4,7 +4,8 @@
 host side of fslr_b200.table.ColumnarTable.from_dataframe): the raw bytes go to the device once, the columnar table is
 built there (fslrc_tsv_open) and stays there, so the clustering step runs on it without any further host<->device
 traffic.  `ParsedBed.write_cluster_bed` renders the reference's output file (main.py:334-349): every input line plus the
-float `cluster` / `n_reads` columns.  There is no CPU path: these functions raise without the CUDA library or a device.
+float `cluster` / `n_reads` columns; `ParsedBed.write_representative_bed` the second one (main.py:351-352): the lines of
+each cluster's representative read plus those columns and `avg_alignment_score`.  There is no CPU path: these functions raise without the CUDA library or a device.
 """
 import ctypes as C
 
@@ -79,23 +80,35 @@ class ParsedBed:
         n = self.n_reads
         return ClusterResult(self.out_cluster[:n].cpu().numpy(), self.out_n_reads[:n].cpu().numpy(), bool(stats["no_clusters"]), stats)
 
+    def _render(self, entry):
+        self._live()
+        fn, ctx = getattr(self.engine.lib, entry), self.engine.ctx
+        stream = C.c_void_p(torch.cuda.current_stream(self.engine.device).cuda_stream)
+        n = C.c_int64()
+        self.engine._check(fn(ctx, self.out_cluster.data_ptr(), self.out_n_reads.data_ptr(), None, 0, C.byref(n), stream))
+        out = self.engine.pinned_bytes(n.value)       # reused staging buffer: the result is valid until the next rendering call
+        self.engine._check(fn(ctx, self.out_cluster.data_ptr(), self.out_n_reads.data_ptr(), out.data_ptr(), n.value, C.byref(n), stream))
+        return out[:n.value].numpy()
+
     def cluster_bed_bytes(self):
         """`<base>.mappings.cluster.bed` (main.py:349) as bytes, rendered on the device from out_cluster / out_n_reads.  The
         returned array is a VIEW of the engine's reused pinned staging buffer: valid until the next rendering call of any
         table on this engine (copy it, or write it out, before that)."""
-        self._live()
-        lib, ctx = self.engine.lib, self.engine.ctx
-        stream = C.c_void_p(torch.cuda.current_stream(self.engine.device).cuda_stream)
-        n = C.c_int64()
-        self.engine._check(lib.fslrc_tsv_write_cluster_bed(ctx, self.out_cluster.data_ptr(), self.out_n_reads.data_ptr(), None, 0,
-                                                          C.byref(n), stream))
-        out = self.engine.pinned_bytes(n.value)       # reused staging buffer: the result is valid until the next rendering call
-        self.engine._check(lib.fslrc_tsv_write_cluster_bed(ctx, self.out_cluster.data_ptr(), self.out_n_reads.data_ptr(), out.data_ptr(),
-                                                          n.value, C.byref(n), stream))
-        return out[:n.value].numpy()
+        return self._render("fslrc_tsv_write_cluster_bed")
 
     def write_cluster_bed(self, path):
         self.cluster_bed_bytes().tofile(path)
+
+    def representative_bed_bytes(self):
+        """`<base>.mappings.representative.bed` (main.py:351-352, cluster.py:237-254) as bytes, rendered on the device from
+        the parsed alignment_score column and out_cluster / out_n_reads: the lines of each cluster's representative read
+        (highest mean alignment_score, first in the table on ties) plus `cluster`, `n_reads` and `avg_alignment_score`
+        (repr of the mean, as pandas writes a float64).  Raises FslrError without an alignment_score column or for a
+        cluster id outside [0, n_reads).  Like cluster_bed_bytes, a VIEW of the engine's reused pinned staging buffer."""
+        return self._render("fslrc_tsv_write_representative_bed")
+
+    def write_representative_bed(self, path):
+        self.representative_bed_bytes().tofile(path)
 
     def close(self):
         if self.engine is not None:

@@ -176,6 +176,14 @@ int fslrc_tsv_chrom_name(fslrc_ctx *ctx, int32_t chrom_id, char *buf, int32_t ca
 int fslrc_tsv_read_names(fslrc_ctx *ctx, int64_t *offsets, int32_t *lengths);           /* [n_reads]: where each qname sits in `text` */
 int fslrc_tsv_write_cluster_bed(fslrc_ctx *ctx, const int32_t *cluster_dev, const int32_t *n_reads_dev, char *out, int64_t cap,
                                 int64_t *n_out, void *stream);
+/* fslrc_tsv_write_representative_bed renders `<base>.mappings.representative.bed` (main.py:351-352, cluster.py:237-254) the
+ * same way: the header + "\tcluster\tn_reads\tavg_alignment_score", then, in table order, every line of each cluster's
+ * representative read (highest mean alignment_score, the read whose first row comes first on ties) with the two columns
+ * above and the read's mean score as Python's repr of the double sum / count.  cluster_dev / n_reads_dev: [n_reads] device
+ * arrays, as fslrc_cluster_device leaves them.  FSLRC_ERR_ARG when the table has no alignment_score column;
+ * FSLRC_ERR_RANGE when a cluster id is negative or >= n_reads. */
+int fslrc_tsv_write_representative_bed(fslrc_ctx *ctx, const int32_t *cluster_dev, const int32_t *n_reads_dev, char *out,
+                                       int64_t cap, int64_t *n_out, void *stream);
 void fslrc_tsv_close(fslrc_ctx *ctx);
 
 /* ---- The producer of `<base>.mappings.bed` (SURVEY §8f row 4): replaces collect_mapping_info.mapping_info
