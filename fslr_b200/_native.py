@@ -12,7 +12,7 @@ N_STAGES = 14
 SYMBOLS = ["fslrc_create", "fslrc_destroy", "fslrc_last_error", "fslrc_stage_name", "fslrc_version",
            "fslrc_cluster_device", "fslrc_cluster_host", "fslrc_mg_prepare", "fslrc_mg_pair", "fslrc_mg_partners", "fslrc_mg_replay",
            "fslrc_mg_finish", "fslrc_int_peak", "fslrc_launch_count", "fslrc_set_blocking_sync", "fslrc_choose_alignment_host",
-           "fslrc_tsv_open", "fslrc_tsv_chrom_name", "fslrc_tsv_read_names", "fslrc_tsv_write_cluster_bed", "fslrc_tsv_write_representative_bed",
+           "fslrc_tsv_open", "fslrc_tsv_delete_false", "fslrc_tsv_chrom_name", "fslrc_tsv_read_names", "fslrc_tsv_write_cluster_bed", "fslrc_tsv_write_representative_bed",
            "fslrc_tsv_close",
            "fslrc_bam_open", "fslrc_bam_open_bgzf", "fslrc_bam_read_stream", "fslrc_bam_write_mappings_bed", "fslrc_bam_read_names", "fslrc_bam_close"]
 
@@ -53,7 +53,7 @@ class Stats(C.Structure):
 class TsvInfo(C.Structure):
     _fields_ = [("n_rows", C.c_int64), ("n_reads", C.c_int64), ("n_chrom", C.c_int32), ("has_score", C.c_int32)] + \
                [(n, C.c_void_p) for n in ("read_id", "chrom", "rstart", "rend", "aln_size", "qstart", "qend", "n_alignments",
-                                          "alignment_score")] + [("parse_ms", C.c_float), ("reserved", C.c_int32)]
+                                          "alignment_score")] + [("parse_ms", C.c_float), ("filter_ms", C.c_float)]
 
 
 BAM_COLUMNS = ("read_id", "chrom", "rstart", "rend", "n_alignments", "aln_size", "qstart", "qend", "strand", "mapq", "qlen",
@@ -103,6 +103,7 @@ def load():
     lib.fslrc_int_peak.argtypes = [vp, C.POINTER(C.c_double)]
     lib.fslrc_choose_alignment_host.argtypes = [vp, C.c_int64, C.c_int64, C.c_int64, vp, vp, vp, vp, vp, vp]
     lib.fslrc_tsv_open.argtypes = [vp, vp, C.c_int64, C.c_uint64, C.POINTER(TsvInfo), vp]
+    lib.fslrc_tsv_delete_false.argtypes = [vp, C.POINTER(TsvInfo), vp]
     lib.fslrc_tsv_chrom_name.argtypes = [vp, C.c_int32, C.c_char_p, C.c_int32]
     lib.fslrc_tsv_read_names.argtypes = [vp, vp, vp]
     lib.fslrc_tsv_write_cluster_bed.argtypes = [vp, vp, vp, vp, C.c_int64, i64p, vp]

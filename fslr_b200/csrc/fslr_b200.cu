@@ -1045,6 +1045,7 @@ struct TsvState {
     int n_lines, n_rows, n_reads, n_chrom;
     int *read_id, *chrom, *rstart, *rend, *aln, *qstart, *qend, *naln, *score, *first_row;
     long long *q_off; int *q_len;
+    long long *line_end;     // nullptr: line l ends at line_start[l + 1] - 1; set once fslrc_tsv_delete_false removed rows
     std::vector<std::string> chrom_names;
 };
 template <typename T>
@@ -1171,6 +1172,60 @@ static int tsv_open_impl(fslrc_ctx *ctx, const char *text, int64_t n_bytes, uint
     if (cudaEventElapsedTime(&ms, ctx->ev[0 + 1], ctx->ev[2]) == cudaSuccess) info->parse_ms = ms; else cudaGetLastError();
     return 0;
 }
+static void pfree(fslrc_ctx *ctx, void *p) {                            // one persistent array, before fslrc_tsv_close
+    std::vector<void *> &a = ctx->tsv->allocs;
+    std::vector<void *>::iterator it = std::find(a.begin(), a.end(), p);
+    if (it != a.end()) { a.erase(it); cudaFreeAsync(p, ctx->stream); }
+}
+// --filter-false on the parsed table: flag the reads (one thread per read), two exclusive scans give the new read ids and
+// the new row positions, one read-back of both totals, and, if any row goes, one compaction into fresh arrays
+static int tsv_delete_false_impl(fslrc_ctx *ctx, fslrc_tsv_info *info, void *stream) {
+    CK(cudaSetDevice(ctx->device));
+    ctx->stream = (cudaStream_t)stream;
+    cudaStream_t st = ctx->stream;
+    TsvState *T = ctx->tsv;
+    const int n = T->n_rows, R = T->n_reads, TB = 256;
+    CK(cudaEventRecord(ctx->ev[1], st));
+    if (R > 0) {
+        Pipe Pp; memset((void *)&Pp, 0, sizeof(Pp)); Pipe *P = &Pp;
+        int *keep_read, *new_id, *keep_row, *new_pos; int64_t *tot;
+        DA(keep_read, R); DA(new_id, R); DA(keep_row, n); DA(new_pos, n); DA(tot, 2);
+        KL(tsv::k_tsv_false, nblk(R, TB), TB, R, T->text, T->first_row, T->q_off, T->q_len, keep_read);
+        int r = xscan(ctx, P, keep_read, new_id, R, tot); if (r) return r;
+        KL(tsv::k_tsv_row_keep, nblk(n, TB), TB, n, T->read_id, keep_read, keep_row);
+        r = xscan(ctx, P, keep_row, new_pos, n, tot + 1); if (r) return r;
+        CK(cudaMemcpyAsync(ctx->h_pin, tot, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        const int R2 = (int)ctx->h_pin[0], n2 = (int)ctx->h_pin[1];
+        if (n2 < n) {
+            const tsv::Cols s = {T->read_id, T->chrom, T->rstart, T->rend, T->aln, T->qstart, T->qend, T->naln, T->score,
+                                 T->q_off, T->q_len, T->line_start, T->line_end};
+            tsv::Cols d; memset((void *)&d, 0, sizeof(d));
+            int *first_row;
+            PA(d.read_id, n2); PA(d.chrom, n2); PA(d.rstart, n2); PA(d.rend, n2); PA(d.aln, n2); PA(d.qstart, n2); PA(d.qend, n2);
+            PA(d.naln, n2); PA(d.q_off, n2); PA(d.q_len, n2); PA(d.line_start, (int64_t)n2 + 1); PA(d.line_end, (int64_t)n2 + 1);
+            PA(first_row, R2);
+            if (T->score) PA(d.score, n2);
+            KL(tsv::k_tsv_compact, nblk(n, TB), TB, n, keep_row, new_pos, new_id, T->first_row, s, d, first_row);
+            void *old[] = {s.read_id, s.chrom, s.rstart, s.rend, s.aln, s.qstart, s.qend, s.naln, s.score, s.q_off, s.q_len,
+                           s.line_start, s.line_end, T->first_row};
+            for (void *p : old) if (p) pfree(ctx, p);                  // (stream-ordered: after the compaction has read them)
+            T->read_id = d.read_id; T->chrom = d.chrom; T->rstart = d.rstart; T->rend = d.rend; T->aln = d.aln;
+            T->qstart = d.qstart; T->qend = d.qend; T->naln = d.naln; T->score = d.score; T->q_off = d.q_off; T->q_len = d.q_len;
+            T->line_start = d.line_start; T->line_end = d.line_end; T->first_row = first_row;
+            T->n_rows = n2; T->n_reads = R2; T->n_lines = n2 + 1;
+        }
+    }
+    CK(cudaEventRecord(ctx->ev[2], st));
+    free_all(ctx);
+    CK(cudaStreamSynchronize(st));
+    info->n_rows = T->n_rows; info->n_reads = T->n_reads;
+    info->read_id = T->read_id; info->chrom = T->chrom; info->rstart = T->rstart; info->rend = T->rend; info->aln_size = T->aln;
+    info->qstart = T->qstart; info->qend = T->qend; info->n_alignments = T->naln; info->alignment_score = T->score;
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, ctx->ev[1], ctx->ev[2]) == cudaSuccess) info->filter_ms = ms; else cudaGetLastError();
+    return 0;
+}
 extern "C" {
 
 int fslrc_tsv_open(fslrc_ctx *ctx, const char *text, int64_t n_bytes, uint64_t hash_seed, fslrc_tsv_info *info, void *stream) {
@@ -1179,6 +1234,16 @@ int fslrc_tsv_open(fslrc_ctx *ctx, const char *text, int64_t n_bytes, uint64_t h
     const int r = tsv_open_impl(ctx, text, n_bytes, hash_seed, info, stream);
     if (r) {                                                           // every error path: scratch and the half-built table go
         free_all(ctx); tsv_free(ctx);
+        cudaStreamSynchronize(ctx->stream);
+    }
+    return r;
+}
+int fslrc_tsv_delete_false(fslrc_ctx *ctx, fslrc_tsv_info *info, void *stream) {
+    if (!ctx) return FSLRC_ERR_ARG;
+    if (!ctx->tsv || !info) return fail(ctx, FSLRC_ERR_ARG, "tsv: no parsed table (fslrc_tsv_open first) or null info");
+    const int r = tsv_delete_false_impl(ctx, info, stream);
+    if (r) {                                                           // the table keeps its old arrays until the compaction ran
+        free_all(ctx);
         cudaStreamSynchronize(ctx->stream);
     }
     return r;
@@ -1219,7 +1284,7 @@ int fslrc_tsv_write_cluster_bed(fslrc_ctx *ctx, const int32_t *cluster_dev, cons
     DA(len, L); DA(off, L); DA(tot, 1); DA(any_single, 1);
     CK(cudaMemsetAsync(any_single, 0, sizeof(int), st));
     if (T->n_reads > 0) KL(tsv::k_tsv_any_single, nblk(T->n_reads, TB), TB, T->n_reads, n_reads_dev, any_single);
-    KL(tsv::k_tsv_outlen, nblk(L, TB), TB, L, T->line_start, T->read_id, cluster_dev, n_reads_dev, any_single, len);
+    KL(tsv::k_tsv_outlen, nblk(L, TB), TB, L, T->line_start, T->line_end, T->read_id, cluster_dev, n_reads_dev, any_single, len);
     {
         const int tiles = nblk(L, prims::SC_TILE);
         int r = prim_scratch(ctx, P, sizeof(unsigned long long) * tiles); if (r) return r;
@@ -1233,7 +1298,7 @@ int fslrc_tsv_write_cluster_bed(fslrc_ctx *ctx, const int32_t *cluster_dev, cons
         if (cap < *n_out) rc = fail(ctx, FSLRC_ERR_ARG, "tsv: output buffer too small");
         else {
             unsigned char *d_out; DA(d_out, *n_out);
-            KL(tsv::k_tsv_emit, nblk((int64_t)L * 32, TB), TB, L, T->text, T->line_start, T->read_id, cluster_dev, n_reads_dev, any_single, off, d_out);
+            KL(tsv::k_tsv_emit, nblk((int64_t)L * 32, TB), TB, L, T->text, T->line_start, T->line_end, T->read_id, cluster_dev, n_reads_dev, any_single, off, d_out);
             CK(cudaMemcpyAsync(out, d_out, *n_out, cudaMemcpyDeviceToHost, st));
         }
     }
@@ -1261,7 +1326,7 @@ int fslrc_tsv_write_representative_bed(fslrc_ctx *ctx, const int32_t *cluster_de
         KL(tsv::k_tsv_any_single, nblk(R, TB), TB, R, n_reads_dev, any_single);
         KL(tsv::k_tsv_rep_mean, nblk(R, TB), TB, R, is_rep, sum, cnt, txt, txt_len);
     }
-    KL(tsv::k_tsv_rep_outlen, nblk(L, TB), TB, L, T->line_start, T->read_id, cluster_dev, n_reads_dev, any_single, is_rep, txt_len, len);
+    KL(tsv::k_tsv_rep_outlen, nblk(L, TB), TB, L, T->line_start, T->line_end, T->read_id, cluster_dev, n_reads_dev, any_single, is_rep, txt_len, len);
     {
         const int tiles = nblk(L, prims::SC_TILE);
         int r = prim_scratch(ctx, P, sizeof(unsigned long long) * tiles); if (r) return r;
@@ -1278,7 +1343,7 @@ int fslrc_tsv_write_representative_bed(fslrc_ctx *ctx, const int32_t *cluster_de
             if (cap < *n_out) rc = fail(ctx, FSLRC_ERR_ARG, "tsv: output buffer too small");
             else {
                 unsigned char *d_out; DA(d_out, *n_out);
-                KL(tsv::k_tsv_rep_emit, nblk((int64_t)L * 32, TB), TB, L, T->text, T->line_start, T->read_id, cluster_dev, n_reads_dev,
+                KL(tsv::k_tsv_rep_emit, nblk((int64_t)L * 32, TB), TB, L, T->text, T->line_start, T->line_end, T->read_id, cluster_dev, n_reads_dev,
                    any_single, is_rep, txt, txt_len, off, d_out);
                 CK(cudaMemcpyAsync(out, d_out, *n_out, cudaMemcpyDeviceToHost, st));
             }

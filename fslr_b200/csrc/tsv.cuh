@@ -7,6 +7,9 @@
 //   k_tsv_intern_*              open-addressing hash table keyed by the 64-bit hash: first row of every distinct string,
 //                               byte-for-byte verification against that row, dense ids in order of first appearance
 //                               (= pandas.factorize = the singleton numbering order of main.py:336-341)
+//   k_tsv_false / k_tsv_row_keep / k_tsv_compact
+//                               --filter-false (main.py:229-230, cluster.py:80-86): the reads whose qname contains "False"
+//                               leave the table; the kept rows move down in table order and the reads are renumbered densely
 //   k_tsv_outlen / k_tsv_emit   every input line + "\t<cluster>.0\t<n_reads>.0" (the float columns of main.py:334-342)
 //   k_tsv_rep_mean / k_tsv_rep_outlen / k_tsv_rep_emit
 //                               `<base>.mappings.representative.bed` (main.py:351-352): the lines of every cluster's
@@ -149,7 +152,54 @@ __global__ void k_tsv_intern_ids(int n_rows, const int *__restrict__ slot_of_row
     id[r] = i;
     if (f == r && first_row_of_id) first_row_of_id[i] = r;
 }
+// ---- --filter-false: bed_file[~bed_file["qname"].str.contains("False")] on the parsed table
+// every row of a read carries the same name bytes (k_tsv_intern_verify), so the read's first row decides for all of them;
+// "False" has no regex metacharacter, so str.contains is a case-sensitive substring search
+__global__ void k_tsv_false(int n_reads, const unsigned char *__restrict__ text, const int *__restrict__ first_row,
+                            const long long *__restrict__ q_off, const int *__restrict__ q_len, int *keep) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n_reads) return;
+    const int f = first_row[r];
+    const unsigned char *p = text + q_off[f];
+    const int l = q_len[f];
+    bool hit = false;
+    for (int i = 0; i + 5 <= l && !hit; i++)
+        hit = p[i] == 'F' && p[i + 1] == 'a' && p[i + 2] == 'l' && p[i + 3] == 's' && p[i + 4] == 'e';
+    keep[r] = !hit;
+}
+__global__ void k_tsv_row_keep(int n_rows, const int *__restrict__ rid, const int *__restrict__ keep_read, int *keep_row) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r < n_rows) keep_row[r] = keep_read[rid[r]];
+}
+// the per-row columns of the parsed table; line_start / line_end describe lines (line 0 is the header, row r is line r + 1)
+struct Cols {
+    int *read_id, *chrom, *rstart, *rend, *aln, *qstart, *qend, *naln, *score;   // score: nullable
+    long long *q_off; int *q_len;
+    long long *line_start, *line_end;                                           // line_end: nullable (= line_start[l + 1] - 1)
+};
+// kept row r goes to new_pos[r]; read ids become new_id[read_id] (the kept reads in order of first appearance, which is
+// pandas.factorize of the filtered frame).  Chromosome ids keep the numbering of the unfiltered table (main.py:227 numbers
+// the chromosomes before :229-230 filters).  The kept lines are no longer contiguous in the text, so every line gets its end.
+__global__ void k_tsv_compact(int n_rows, const int *__restrict__ keep_row, const int *__restrict__ new_pos,
+                              const int *__restrict__ new_id, const int *__restrict__ first_row, Cols s, Cols d, int *first_row_out) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n_rows) return;
+    if (r == 0) { d.line_start[0] = s.line_start[0]; d.line_end[0] = s.line_end ? s.line_end[0] : s.line_start[1] - 1; }
+    if (!keep_row[r]) return;
+    const int p = new_pos[r], q = s.read_id[r], id = new_id[q];
+    d.read_id[p] = id; d.chrom[p] = s.chrom[r]; d.rstart[p] = s.rstart[r]; d.rend[p] = s.rend[r]; d.aln[p] = s.aln[r];
+    d.qstart[p] = s.qstart[r]; d.qend[p] = s.qend[r]; d.naln[p] = s.naln[r];
+    if (s.score) d.score[p] = s.score[r];
+    d.q_off[p] = s.q_off[r]; d.q_len[p] = s.q_len[r];
+    d.line_start[p + 1] = s.line_start[r + 1];
+    d.line_end[p + 1] = s.line_end ? s.line_end[r + 1] : s.line_start[r + 2] - 1;
+    if (first_row[q] == r) first_row_out[id] = p;
+}
 // ---- egress
+// line l without its '\n' is [line_start[l], line_end(l)); line_end == nullptr: the lines are contiguous in the text
+__device__ __forceinline__ long long line_end_of(const long long *__restrict__ line_start, const long long *__restrict__ line_end, int l) {
+    return line_end ? line_end[l] : line_start[l + 1] - 1;
+}
 __device__ __forceinline__ int dec_digits(int v) {
     int d = 1;
     unsigned u = v < 0 ? (unsigned)(-(long long)v) : (unsigned)v;
@@ -179,24 +229,25 @@ __device__ __forceinline__ unsigned char *put_cluster_cols(unsigned char *q, int
 }
 __device__ __forceinline__ unsigned char *put_str(unsigned char *q, const char *h) { while (*h) *q++ = (unsigned char)*h++; return q; }
 // output length of every line: header + "\tcluster\tn_reads\n"; row: line + "\t<c>.0\t<n>.0\n" (floats) or "\t<c>\t<n>\n"
-__global__ void k_tsv_outlen(int n_lines, const long long *__restrict__ line_start, const int *__restrict__ rid,
-                             const int *__restrict__ cluster, const int *__restrict__ nreads, const int *__restrict__ any_single,
-                             long long *len) {
+__global__ void k_tsv_outlen(int n_lines, const long long *__restrict__ line_start, const long long *__restrict__ line_end,
+                             const int *__restrict__ rid, const int *__restrict__ cluster, const int *__restrict__ nreads,
+                             const int *__restrict__ any_single, long long *len) {
     const int l = blockIdx.x * blockDim.x + threadIdx.x;
     if (l >= n_lines) return;
-    const long long body = line_start[l + 1] - 1 - line_start[l];
+    const long long body = line_end_of(line_start, line_end, l) - line_start[l];
     if (l == 0) len[l] = body + 17;                                     // "\tcluster\tn_reads\n"
     else { const int r = rid[l - 1]; len[l] = body + cluster_cols_len(cluster[r], nreads[r], *any_single != 0) + 1; }
 }
 // one warp per line: coalesced byte copy, lane 0 appends the two columns
 __global__ void k_tsv_emit(int n_lines, const unsigned char *__restrict__ text, const long long *__restrict__ line_start,
-                           const int *__restrict__ rid, const int *__restrict__ cluster, const int *__restrict__ nreads,
-                           const int *__restrict__ any_single, const long long *__restrict__ out_off, unsigned char *out) {
+                           const long long *__restrict__ line_end, const int *__restrict__ rid, const int *__restrict__ cluster,
+                           const int *__restrict__ nreads, const int *__restrict__ any_single, const long long *__restrict__ out_off,
+                           unsigned char *out) {
     const long long wg = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (wg >= n_lines) return;
     const int l = (int)wg;
-    const long long s = line_start[l], body = line_start[l + 1] - 1 - s;
+    const long long s = line_start[l], body = line_end_of(line_start, line_end, l) - s;
     unsigned char *o = out + out_off[l];
     for (long long i = lane; i < body; i += 32) o[i] = text[s + i];
     if (lane == 0) {
@@ -216,19 +267,21 @@ __global__ void k_tsv_rep_mean(int n_reads, const unsigned char *__restrict__ is
     txt_len[r] = fmtd::fmt_repr_f64(__ddiv_rn((double)sum[r], (double)cnt[r]), txt + (long long)r * fmtd::FMT_F64_MAX);
 }
 // output length of every line: 0 for the lines of a read that is not its cluster's representative
-__global__ void k_tsv_rep_outlen(int n_lines, const long long *__restrict__ line_start, const int *__restrict__ rid,
-                                 const int *__restrict__ cluster, const int *__restrict__ nreads, const int *__restrict__ any_single,
-                                 const unsigned char *__restrict__ is_rep, const int *__restrict__ txt_len, long long *len) {
+__global__ void k_tsv_rep_outlen(int n_lines, const long long *__restrict__ line_start, const long long *__restrict__ line_end,
+                                 const int *__restrict__ rid, const int *__restrict__ cluster, const int *__restrict__ nreads,
+                                 const int *__restrict__ any_single, const unsigned char *__restrict__ is_rep,
+                                 const int *__restrict__ txt_len, long long *len) {
     const int l = blockIdx.x * blockDim.x + threadIdx.x;
     if (l >= n_lines) return;
-    const long long body = line_start[l + 1] - 1 - line_start[l];
+    const long long body = line_end_of(line_start, line_end, l) - line_start[l];
     if (l == 0) { len[l] = body + REP_HEADER_LEN; return; }
     const int r = rid[l - 1];
     len[l] = is_rep[r] ? body + cluster_cols_len(cluster[r], nreads[r], *any_single != 0) + 1 + txt_len[r] + 1 : 0;
 }
 // one warp per kept line: coalesced byte copy, lane 0 appends the cluster columns and the formatted mean
 __global__ void k_tsv_rep_emit(int n_lines, const unsigned char *__restrict__ text, const long long *__restrict__ line_start,
-                               const int *__restrict__ rid, const int *__restrict__ cluster, const int *__restrict__ nreads,
+                               const long long *__restrict__ line_end, const int *__restrict__ rid,
+                               const int *__restrict__ cluster, const int *__restrict__ nreads,
                                const int *__restrict__ any_single, const unsigned char *__restrict__ is_rep,
                                const char *__restrict__ txt, const int *__restrict__ txt_len, const long long *__restrict__ out_off,
                                unsigned char *out) {
@@ -238,7 +291,7 @@ __global__ void k_tsv_rep_emit(int n_lines, const unsigned char *__restrict__ te
     const int l = (int)wg;
     const int r = l > 0 ? rid[l - 1] : -1;
     if (l > 0 && !is_rep[r]) return;
-    const long long s = line_start[l], body = line_start[l + 1] - 1 - s;
+    const long long s = line_start[l], body = line_end_of(line_start, line_end, l) - s;
     unsigned char *o = out + out_off[l];
     for (long long i = lane; i < body; i += 32) o[i] = text[s + i];
     if (lane == 0) {

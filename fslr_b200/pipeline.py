@@ -14,15 +14,16 @@ from .table import ColumnarTable
 
 
 def cluster_step_fast(bed_path, chr_lengths, out_base, cluster_mask="subtelomere", jaccard_cutoffs="1,1,0.66,0.66,0.66,0.5",
-                      overlap=0.8, n_alignment_diff=0.25, qlen_diff=0.04, representative=True, device=0):
+                      overlap=0.8, n_alignment_diff=0.25, qlen_diff=0.04, representative=True, filter_false=False, device=0):
     """The same block with the table never leaving the GPU between the file bytes and the output bytes (fslr_b200.tsv):
     GPU TSV parse -> clustering on the device-resident columns -> GPU rendering of `<out_base>.mappings.cluster.bed` and
     (representative=True) `<out_base>.mappings.representative.bed`.
+    filter_false drops the reads whose qname contains "False" (main.py:229-230) on the device, after the parse.
     Tie order of equal starts is the GPU's stable one (ids equal the reference's whenever its unstable sort keeps ties in
     table order, the partition always).  Returns the ClusterResult, or None for main.py:247-249's early return."""
     from . import tsv
     print("Making clusters", file=sys.stderr)                                    # main.py:207
-    pb = tsv.read_mappings_bed(bed_path, chr_lengths, device=device)
+    pb = tsv.read_mappings_bed(bed_path, chr_lengths, device=device, filter_false=filter_false)   # main.py:209, 229-230
     try:
         res = pb.cluster(cluster_mask=cluster_mask, jaccard_cutoffs=jaccard_cutoffs, overlap=overlap,
                          n_alignment_diff=n_alignment_diff, qlen_diff=qlen_diff)
@@ -41,7 +42,8 @@ def bam_to_clusters(bam_path, primers, out_base, regions_path=None, fslr_version
     """main.py:181-183 + main.py:190-352 without the table ever being parsed on the host: `<base>.bwa_dodi.bam` ->
     `<out_base>.mappings.bed` (fslr_b200.mapping_info, the GPU stand-in for collect_mapping_info.mapping_info) ->
     `<out_base>.mappings.cluster.bed` (+ representative).  The chromosome lengths come from the same BAM header
-    (cluster.py:173-175).  primers: {name: sequence} as main.py:69 builds it from primers.csv."""
+    (cluster.py:173-175).  primers: {name: sequence} as main.py:69 builds it from primers.csv.  cluster_options go to
+    cluster_step_fast; with filter_false=True the written mappings.bed still holds every read, as in main.py."""
     from . import mapping_info as mi
     t = mi.read_bam_table(bam_path, regions_path, primers, device=device)
     try:
@@ -105,14 +107,14 @@ def main(argv=None):
         primers = {k: v for k, v in zip(d["primer_name"], d["primer_seq"]) if k in want}       # main.py:69
         bam_to_clusters(a.bam, primers, a.out_base, a.regions, cluster_mask=a.cluster_mask, jaccard_cutoffs=a.jaccard_cutoffs,
                         overlap=a.overlap, n_alignment_diff=a.n_alignment_diff, qlen_diff=a.qlen_diff,
-                        representative=not a.no_representative)
+                        representative=not a.no_representative, filter_false=a.filter_false)
         return
     if not a.bed or not a.chr_lengths:
         ap.error("--bed and --chr-lengths are required without --bam")
     lengths = gcluster.get_chromosome_lengths(a.chr_lengths) if a.chr_lengths.endswith(".bam") else json.load(open(a.chr_lengths))
-    if a.fast_io and not a.filter_false:
+    if a.fast_io:
         cluster_step_fast(a.bed, lengths, a.out_base, a.cluster_mask, a.jaccard_cutoffs, a.overlap,
-                          a.n_alignment_diff, a.qlen_diff, not a.no_representative)
+                          a.n_alignment_diff, a.qlen_diff, not a.no_representative, filter_false=a.filter_false)
         return
     cluster_step(a.bed, lengths, a.cluster_mask, a.jaccard_cutoffs, a.overlap, a.n_alignment_diff,
                  a.qlen_diff, a.filter_false, a.out_base)

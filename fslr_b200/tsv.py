@@ -29,6 +29,7 @@ class ParsedBed:
         self.chrom_names = chrom_names
         self.chrom_len = np.array([int((chr_lengths or {}).get(c, 0) or 0) for c in chrom_names], dtype=np.int64)
         self.parse_ms = float(info.parse_ms)
+        self.filter_ms = float(info.filter_ms)
         dev = engine.device
         view = lambda p: (torch.as_tensor(_DevView(p, (self.n_rows,)), device=dev) if self.n_rows > 0 and p
                           else torch.zeros(0, dtype=torch.int32, device=dev))
@@ -117,8 +118,12 @@ class ParsedBed:
             self.engine = None
 
 
-def read_mappings_bed(path_or_bytes, chr_lengths=None, device=0, hash_seed=0):
-    """Parse `<base>.mappings.bed` on the GPU.  chr_lengths: {chrom name: length} (the BAM-header lookup of main.py:225)."""
+def read_mappings_bed(path_or_bytes, chr_lengths=None, device=0, hash_seed=0, filter_false=False):
+    """Parse `<base>.mappings.bed` on the GPU.  chr_lengths: {chrom name: length} (the BAM-header lookup of main.py:225).
+    filter_false: --filter-false (main.py:229-230), on the device: the reads whose qname contains "False" leave the table
+    (fslrc_tsv_delete_false), so n_rows, n_reads, the columns, qnames() and both rendered files describe the kept rows.
+    Chromosome ids and names stay those of the whole file, as main.py numbers them before it filters; malformed rows of
+    dropped reads still raise, as pandas reads every row before delete_false runs."""
     eng = get_engine(device)
     if isinstance(path_or_bytes, (bytes, bytearray)):
         data = np.frombuffer(path_or_bytes, dtype=np.uint8)
@@ -131,6 +136,8 @@ def read_mappings_bed(path_or_bytes, chr_lengths=None, device=0, hash_seed=0):
         if rc != _native.ERR_HASH_COLLISION:
             break
     eng._check(rc)
+    if filter_false:
+        eng._check(eng.lib.fslrc_tsv_delete_false(eng.ctx, C.byref(info), stream))
     names = []
     buf = C.create_string_buffer(4096)
     for c in range(info.n_chrom):

@@ -169,9 +169,17 @@ typedef struct {
     int32_t n_chrom, has_score;
     const int32_t *read_id, *chrom, *rstart, *rend, *aln_size, *qstart, *qend, *n_alignments, *alignment_score;  /* device */
     float parse_ms;                /* device time of the parse (after the upload) */
-    int32_t reserved;
+    float filter_ms;               /* device time of fslrc_tsv_delete_false (0 until it runs) */
 } fslrc_tsv_info;
 int fslrc_tsv_open(fslrc_ctx *ctx, const char *text, int64_t n_bytes, uint64_t hash_seed, fslrc_tsv_info *info, void *stream);
+/* fslrc_tsv_delete_false applies --filter-false (main.py:229-230, cluster.py:80-86: bed_file[~qname.str.contains("False")])
+ * to the table fslrc_tsv_open left in the context: every row of every read whose qname contains the bytes "False" (case
+ * sensitive) leaves the table.  The kept rows keep their order; read ids are renumbered densely in order of first appearance
+ * (pandas.factorize of the filtered frame); chromosome ids and names stay those of the unfiltered table (main.py:227 numbers
+ * them before the filter).  Rewrites info->n_rows, n_reads, the device column pointers and filter_ms; the pointers an
+ * earlier info held are invalid afterwards when rows were removed.  fslrc_tsv_read_names and both renderers then describe
+ * the kept rows.  A second call removes nothing.  FSLRC_ERR_ARG without an open table. */
+int fslrc_tsv_delete_false(fslrc_ctx *ctx, fslrc_tsv_info *info, void *stream);
 int fslrc_tsv_chrom_name(fslrc_ctx *ctx, int32_t chrom_id, char *buf, int32_t cap);     /* returns the length */
 int fslrc_tsv_read_names(fslrc_ctx *ctx, int64_t *offsets, int32_t *lengths);           /* [n_reads]: where each qname sits in `text` */
 int fslrc_tsv_write_cluster_bed(fslrc_ctx *ctx, const int32_t *cluster_dev, const int32_t *n_reads_dev, char *out, int64_t cap,
