@@ -10,7 +10,7 @@ MAX_FILLINGS = 64
 N_STAGES = 14
 
 SYMBOLS = ["fslrc_create", "fslrc_destroy", "fslrc_last_error", "fslrc_stage_name", "fslrc_version",
-           "fslrc_cluster_device", "fslrc_cluster_host", "fslrc_mg_prepare", "fslrc_mg_pair", "fslrc_mg_partners", "fslrc_mg_replay",
+           "fslrc_cluster_device", "fslrc_cluster_host", "fslrc_filling_starts", "fslrc_mg_prepare", "fslrc_mg_pair", "fslrc_mg_partners", "fslrc_mg_replay",
            "fslrc_mg_finish", "fslrc_int_peak", "fslrc_launch_count", "fslrc_set_blocking_sync", "fslrc_choose_alignment_host",
            "fslrc_tsv_open", "fslrc_tsv_delete_false", "fslrc_tsv_chrom_name", "fslrc_tsv_read_names", "fslrc_tsv_write_cluster_bed", "fslrc_tsv_write_representative_bed",
            "fslrc_tsv_close",
@@ -95,6 +95,7 @@ def load():
     lib.fslrc_version.restype = C.c_int
     for f in (lib.fslrc_cluster_device, lib.fslrc_cluster_host):
         f.argtypes = [vp, C.POINTER(Table), C.POINTER(Params), vp, vp, C.POINTER(Stats), vp]
+    lib.fslrc_filling_starts.argtypes = [vp, C.POINTER(Table), vp, C.c_int64, i64p, vp]
     lib.fslrc_mg_prepare.argtypes = [vp, C.POINTER(Table), C.POINTER(Params), vp]
     lib.fslrc_mg_pair.argtypes = [vp, C.c_int, C.c_int, C.POINTER(vp), i64p]
     lib.fslrc_mg_partners.argtypes = [vp, C.c_int, C.c_int, C.POINTER(vp), i64p]

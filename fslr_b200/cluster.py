@@ -92,10 +92,17 @@ def get_chromosome_lengths(bam_path):
     return out
 
 
+def reference_order_of_starts(start):
+    """The permutation `sort_values('start')` (cluster.py:114) applies to a fillings frame whose `start` column is `start`
+    (in bed order).  pandas hands an int64 column to numpy's default quicksort, which is unstable and whose tie order
+    depends on the CPU numpy dispatches to; calling the same routine on the same int64 column reproduces the reference's
+    tie order on this host exactly.  The one definition of "reference tie order" for every route."""
+    start = np.asarray(start).astype(np.int64)              # the dtype read_csv gives the reference: ties are sorted as int64
+    return pd.DataFrame({"start": start}).sort_values("start").index.to_numpy().astype(np.int32)
+
+
 def reference_tie_order(table: ColumnarTable):
-    """The permutation `sort_values('start')` (cluster.py:114) applies to the fillings frame: pandas hands an int64
-    column to numpy's default quicksort, which is unstable; calling the same routine on the same column reproduces
-    the reference's tie order on this host exactly."""
+    """reference_order_of_starts of the fillings frame keep_fillings (cluster.py:14-31) makes of a host table."""
     rid = table.read_id
     A = rid.shape[0]
     idx = np.arange(A)
@@ -104,8 +111,7 @@ def reference_tie_order(table: ColumnarTable):
     np.minimum.at(first, rid, idx)
     np.maximum.at(last, rid, idx)
     keep = (idx != first[rid]) & (idx != last[rid])
-    start = np.minimum(table.rstart[keep], table.rend[keep]).astype(np.int64)
-    return pd.DataFrame({"start": start}).sort_values("start").index.to_numpy().astype(np.int32)
+    return reference_order_of_starts(np.minimum(table.rstart[keep], table.rend[keep]))
 
 
 # ---------------------------------------------------------------- opaque handles

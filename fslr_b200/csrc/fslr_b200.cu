@@ -389,6 +389,32 @@ static int pipe_ingest_fast(fslrc_ctx *ctx, Pipe *P, const long long *d_clen, co
     return pipe_bands(ctx, P, s_m, s_end);
 }
 
+// ---- stage 1 of the general ingest, keep_fillings (cluster.py:14-31): flagA[i] = 1 for every row that is neither the first
+// nor the last row of its read by occurrence (the rows of a read need not be contiguous), posA[i] = its filling index in bed
+// order, P->cnt[0] = the number of fillings.  qmin / qmax: per read the smallest qstart / largest qend over its kept rows, or
+// NULL (the flags only).  A read id outside [0, R) sets EF_RANGE.
+static int keep_rows(fslrc_ctx *ctx, Pipe *P, const int *rid, const int *qstart, const int *qend, int *flagA, int *posA,
+                     int *qmin, int *qmax) {
+    cudaStream_t st = ctx->stream;
+    const int A = P->A, R = P->R, TB = 256;
+    int *first, *last;
+    DA(first, R); DA(last, R);
+    if (R > 0) {
+        KL(k_fill<int>, nblk(R, TB), TB, first, R, 0x7fffffff);
+        KL(k_fill<int>, nblk(R, TB), TB, last, R, -1);
+        if (qmin) {
+            KL(k_fill<int>, nblk(R, TB), TB, qmin, R, 0x7fffffff);
+            KL(k_fill<int>, nblk(R, TB), TB, qmax, R, (int)0x80000000);
+        }
+    }
+    if (A > 0) {
+        KL(k_first_last, nblk(A, TB), TB, A, R, rid, first, last, P->err);
+        KL(k_keep, nblk(A, TB), TB, A, R, rid, first, last, qstart, qend, flagA, qmin, qmax);
+        return xscan(ctx, P, flagA, posA, A, P->cnt + 0);
+    }
+    return 0;
+}
+
 // ---- stages 1-5: ingestion, orders, records (replicated on every rank)
 static int pipe_prepare(fslrc_ctx *ctx, Pipe *P) {
     const fslrc_table &tb = P->tb; const fslrc_params &pr = P->pr;
@@ -408,21 +434,11 @@ static int pipe_prepare(fslrc_ctx *ctx, Pipe *P) {
         if (r <= 0) return r;
     }
     // ---- stage 1: keep_fillings
-    int *first, *last, *qmin, *qmax, *flagA, *posA;
-    DA(first, R); DA(last, R); DA(qmin, R); DA(qmax, R); DA(flagA, A); DA(posA, A);
+    int *qmin, *qmax, *flagA, *posA;
+    DA(qmin, R); DA(qmax, R); DA(flagA, A); DA(posA, A);
     DA(P->q_of_rid, R);
-    if (R > 0) {
-        KL(k_fill<int>, nblk(R, TB), TB, first, R, 0x7fffffff);
-        KL(k_fill<int>, nblk(R, TB), TB, last, R, -1);
-        KL(k_fill<int>, nblk(R, TB), TB, qmin, R, 0x7fffffff);
-        KL(k_fill<int>, nblk(R, TB), TB, qmax, R, (int)0x80000000);
-        KL(k_fill<int>, nblk(R, TB), TB, P->q_of_rid, R, -1);
-    }
-    if (A > 0) {
-        KL(k_first_last, nblk(A, TB), TB, A, R, tb.read_id, first, last, P->err);
-        KL(k_keep, nblk(A, TB), TB, A, R, tb.read_id, first, last, tb.qstart, tb.qend, flagA, qmin, qmax);
-        int r = xscan(ctx, P, flagA, posA, A, P->cnt + 0); if (r) return r;
-    }
+    if (R > 0) KL(k_fill<int>, nblk(R, TB), TB, P->q_of_rid, R, -1);
+    { int r = keep_rows(ctx, P, tb.read_id, tb.qstart, tb.qend, flagA, posA, qmin, qmax); if (r) return r; }
     { int r = read_counts(ctx, P); if (r) return r; r = err_code(ctx); if (r) return r; }
     const int F = P->F = (int)ctx->h_pin[0];
     if (tb.order && tb.n_order != F) return fail(ctx, FSLRC_ERR_ARG, "order has the wrong length (must equal the number of fillings)");
@@ -919,6 +935,40 @@ int fslrc_cluster_host(fslrc_ctx *ctx, const fslrc_table *table, const fslrc_par
     if (!r) r = mark(ctx, ST_D2H);
     if (!r) { r = read_counts(ctx, &P); if (!r) r = err_code(ctx); }
     if (!r) fill_stats(ctx, &P, stats);
+    free_all(ctx);
+    ctx_sync(ctx);
+    return r;
+}
+
+// The column cluster.py:114 sorts, for a host sort with the reference's own call (its tie order is numpy's, not ours): stage 1
+// of the general ingest, then one scatter of min(rstart, rend) of the kept rows.  Only the count is read back.
+int fslrc_filling_starts(fslrc_ctx *ctx, const fslrc_table *table, int32_t *out_start, int64_t cap, int64_t *n_fillings,
+                         void *stream) {
+    if (!ctx) return FSLRC_ERR_ARG;
+    if (!table || !out_start || !n_fillings) return fail(ctx, FSLRC_ERR_ARG, "null argument");
+    const int64_t A = table->n_rows, R = table->n_reads;
+    if (A < 0 || R < 0 || A > 0x7ffffff0LL || R > 0x7ffffff0LL) return fail(ctx, FSLRC_ERR_ARG, "table size out of range");
+    if (cap < A) return fail(ctx, FSLRC_ERR_ARG, "out_start is smaller than the table (cap < n_rows)");
+    if (A > 0 && (!table->read_id || !table->rstart || !table->rend))
+        return fail(ctx, FSLRC_ERR_ARG, "the wide device columns read_id, rstart and rend are needed (wire-format-only table)");
+    CK(cudaSetDevice(ctx->device));
+    ctx->stream = (cudaStream_t)stream;
+    cudaStream_t st = ctx->stream;
+    Pipe P; memset((void *)&P, 0, sizeof(P));
+    P.A = (int)A; P.R = (int)R;
+    auto run = [&]() -> int {
+        int *flagA, *posA;
+        DA(P.err, 1); DA(P.cnt, NCNT); DA(flagA, A); DA(posA, A);
+        CK(cudaMemsetAsync(P.err, 0, sizeof(int), st));
+        CK(cudaMemsetAsync(P.cnt, 0, NCNT * sizeof(int64_t), st));
+        int q = keep_rows(ctx, &P, table->read_id, nullptr, nullptr, flagA, posA, nullptr, nullptr); if (q) return q;
+        if (A > 0) KL(k_filling_starts, nblk(A, 256), 256, (int)A, flagA, posA, table->rstart, table->rend, out_start);
+        q = read_counts(ctx, &P); if (q) return q;
+        q = err_code(ctx); if (q) return q;
+        *n_fillings = ctx->h_pin[0];
+        return 0;
+    };
+    const int r = run();
     free_all(ctx);
     ctx_sync(ctx);
     return r;

@@ -70,9 +70,15 @@ __global__ void k_keep(int A, int R, const int *__restrict__ rid, const int *__r
     int keep = 0;
     if ((unsigned)r < (unsigned)R) {
         keep = (i != first[r] && i != last[r]);
-        if (keep) { atomicMax(&qmax[r], qend[i]); atomicMin(&qmin[r], qstart[i]); }
+        if (keep && qmin) { atomicMax(&qmax[r], qend[i]); atomicMin(&qmin[r], qstart[i]); }   // (qmin == NULL: flags only)
     }
     flag[i] = keep;
+}
+// the `start` column of the fillings frame (cluster.py:111), in bed order: min(rstart, rend) of every kept row at its filling index
+__global__ void k_filling_starts(int A, const int *__restrict__ flag, const int *__restrict__ pos, const int *__restrict__ rstart,
+                                 const int *__restrict__ rend, int *start) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < A && flag[i]) start[pos[i]] = min(rstart[i], rend[i]);
 }
 // fillings in bed order as packed records: FR0[k] = {read_id, chrom, start, end}, FR1[k] = {aln_size, n_alignments}
 // (start/end = min/max of rstart, rend: cluster.py:111-112).  One coalesced pass over the kept rows.

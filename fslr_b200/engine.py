@@ -53,6 +53,9 @@ class DeviceTable:
         self.out_n_reads = torch.empty(max(self.n_reads, 1), dtype=torch.int32, device=device)
 
 
+_TABLE_ORDER = object()          # run_resident / _table default: the `order` the table object carries
+
+
 NARROW_OF = {"chrom": ("chrom_u8", np.uint8), "n_alignments": ("n_alignments_u16", np.uint16), "rend": ("rspan_i16", np.int16),
              "qstart": ("qstart_u16", np.uint16), "qend": ("qend_u16", np.uint16)}
 
@@ -209,7 +212,7 @@ class Engine:
         return p
 
     @staticmethod
-    def _table(buf):
+    def _table(buf, order=_TABLE_ORDER):
         t = _native.Table()
         t.n_rows, t.n_reads = buf.n_rows, buf.n_reads
         for k in _COLS:
@@ -220,8 +223,10 @@ class Engine:
         t.aln_size_is_qspan = int(bool(getattr(buf, "aln_is_qspan", False)))
         rpr = getattr(buf, "rows_per_read", None)
         t.rows_per_read_u8 = rpr.data_ptr() if rpr is not None else None
-        if buf.order is not None:
-            t.order, t.n_order = buf.order.data_ptr(), int(buf.order.numel())
+        if order is _TABLE_ORDER:
+            order = buf.order
+        if order is not None:
+            t.order, t.n_order = order.data_ptr(), int(order.numel())
         else:
             t.order, t.n_order = None, 0
         return t
@@ -231,15 +236,49 @@ class Engine:
             raise _native.FslrError(rc, self.lib.fslrc_last_error(self.ctx).decode())
 
     # ---- compute entry points
-    def run_resident(self, dtab: DeviceTable, chrom_table, params: ClusterParams):
-        """Inputs already in HBM; outputs stay in HBM (dtab.out_cluster / out_n_reads).  Returns stats dict."""
+    def run_resident(self, dtab: DeviceTable, chrom_table, params: ClusterParams, order=_TABLE_ORDER):
+        """Inputs already in HBM; outputs stay in HBM (dtab.out_cluster / out_n_reads).  Returns stats dict.
+        order: the tie permutation of this call only (device int32 [n_fillings]; None = the GPU's stable sort); by default
+        dtab.order."""
         p = self._params(chrom_table, params)
-        t = self._table(dtab)
+        t = self._table(dtab, order)
         st = _native.Stats()
         stream = torch.cuda.current_stream(self.device).cuda_stream
         self._check(self.lib.fslrc_cluster_device(self.ctx, C.byref(t), C.byref(p), dtab.out_cluster.data_ptr(),
                                                   dtab.out_n_reads.data_ptr(), C.byref(st), C.c_void_p(stream)))
         return st.as_dict(self.lib)
+
+    def filling_starts(self, dtab):
+        """The `start` column cluster.py:114 sorts (fslrc_filling_starts), computed on the device from dtab's device
+        columns: a device int32 tensor [n_fillings]."""
+        out = torch.empty(max(dtab.n_rows, 1), dtype=torch.int32, device=self.device)
+        n = C.c_int64()
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        self._check(self.lib.fslrc_filling_starts(self.ctx, C.byref(self._table(dtab, None)), out.data_ptr(), out.numel(),
+                                                  C.byref(n), C.c_void_p(stream)))
+        return out[:n.value]
+
+    def reference_order(self, dtab):
+        """The reference's tie permutation (cluster.py:114) for a device-resident table (ParsedBed, BamTable): the start
+        column from the device, sorted on the host by cluster.reference_order_of_starts (numpy's unstable sort, whose tie
+        order is this host's), uploaded as the device int32 `order` fslrc_cluster_device takes."""
+        from .cluster import reference_order_of_starts
+        start = self.filling_starts(dtab).cpu().numpy()
+        return torch.from_numpy(reference_order_of_starts(start)).to(self.device)
+
+    def tie_order(self, dtab, tie_order):
+        """The `order` run_resident gets for ParsedBed / BamTable.cluster(tie_order=...): None = dtab.order as set by the
+        caller (else stable), "stable" = the GPU's stable sort, "reference" = reference_order(dtab), computed once and kept
+        on the table (dtab._reference_order; the table does not change after it is built)."""
+        if tie_order is None:
+            return dtab.order
+        if tie_order == "stable":
+            return None
+        if tie_order == "reference":
+            if getattr(dtab, "_reference_order", None) is None:
+                dtab._reference_order = self.reference_order(dtab)
+            return dtab._reference_order
+        raise ValueError("tie_order must be None, 'stable' or 'reference', not %r" % (tie_order,))
 
     def run_host(self, ptab: PinnedTable, chrom_table, params: ClusterParams):
         """Host buffers in, host buffers out (H2D + D2H inside the call).  Returns stats dict."""

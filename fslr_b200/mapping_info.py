@@ -237,11 +237,13 @@ class BamTable:
     def write_mappings_bed(self, path, fslr_version=None):
         self.mappings_bed_bytes(fslr_version).tofile(path)
 
-    def cluster(self, cluster_mask="subtelomere", **options):
-        """The clustering step (main.py:209-257,334-342) on the device-resident table, GPU stable tie order."""
+    def cluster(self, cluster_mask="subtelomere", tie_order=None, **options):
+        """The clustering step (main.py:209-257,334-342) on the device-resident table.  tie_order as ParsedBed.cluster:
+        None (`self.order` if set, else the GPU's stable sort), "stable", or "reference" (fslr's own tie order on this
+        host, computed once per table)."""
         params = ClusterParams.from_options(self, cluster_mask=cluster_mask, **options)
         self._live()
-        stats = self.engine.run_resident(self, self, params)
+        stats = self.engine.run_resident(self, self, params, order=self.engine.tie_order(self, tie_order))
         n = self.n_reads
         return ClusterResult(self.out_cluster[:n].cpu().numpy(), self.out_n_reads[:n].cpu().numpy(), bool(stats["no_clusters"]), stats)
 

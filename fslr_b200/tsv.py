@@ -72,12 +72,17 @@ class ParsedBed:
             self._names = np.array([buf[o:o + l].decode() for o, l in zip(off[:self.n_reads], ln[:self.n_reads])], dtype=object)
         return self._names
 
-    def cluster(self, cluster_mask="subtelomere", **options):
-        """The clustering step on the device-resident table (GPU stable tie order).  Returns ClusterResult; the per-read
-        result also stays on the device (out_cluster / out_n_reads) for write_cluster_bed."""
+    def cluster(self, cluster_mask="subtelomere", tie_order=None, **options):
+        """The clustering step on the device-resident table.  Returns ClusterResult; the per-read result also stays on the
+        device (out_cluster / out_n_reads) for write_cluster_bed.
+        tie_order: how fillings with equal starts are ordered (cluster.py:114), which decides the cluster numbering.
+        None: `self.order` when the caller set one, else the GPU's stable sort (ties keep bed order).  "stable": the GPU's
+        stable sort.  "reference": the permutation fslr's own `sort_values('start')` gives on this host, so the ids equal
+        fslr's: the start column is built on the device (fslrc_filling_starts), sorted on the host with the reference's
+        pandas call and sent back, once per table (kept for later calls); it applies to that call only."""
         self._live()
         params = ClusterParams.from_options(self, cluster_mask=cluster_mask, **options)
-        stats = self.engine.run_resident(self, self, params)
+        stats = self.engine.run_resident(self, self, params, order=self.engine.tie_order(self, tie_order))
         n = self.n_reads
         return ClusterResult(self.out_cluster[:n].cpu().numpy(), self.out_n_reads[:n].cpu().numpy(), bool(stats["no_clusters"]), stats)
 

@@ -127,6 +127,17 @@ int fslrc_cluster_device(fslrc_ctx *ctx, const fslrc_table *table, const fslrc_p
 int fslrc_cluster_host(fslrc_ctx *ctx, const fslrc_table *table, const fslrc_params *params,
                        int32_t *out_cluster, int32_t *out_n_reads, fslrc_stats *stats, void *stream);
 
+/* The `start` column of the frame keep_fillings returns (cluster.py:14-31,111): min(rstart, rend) of every row that is
+ * neither the first nor the last row of its read in table order, in table order.  This is the column cluster.py:114 sorts:
+ * sorting it on the host with the reference's own call gives the `order` fslrc_cluster_device takes (the reference's tie
+ * order, which depends on the host's numpy and CPU, so it is not reproduced on the device).  The rows of a read need not be
+ * contiguous; a read with 1 or 2 rows contributes nothing.
+ * `table`: wide DEVICE columns (read_id, rstart, rend; n_rows, n_reads), as fslrc_tsv_open / fslrc_bam_open leave them.
+ * out_start: device int32 [cap], cap >= n_rows.  *n_fillings: host.  FSLRC_ERR_ARG: null pointers, cap too small,
+ * wire-format-only table.  FSLRC_ERR_RANGE: a read_id outside [0, n_reads). */
+int fslrc_filling_starts(fslrc_ctx *ctx, const fslrc_table *table, int32_t *out_start, int64_t cap, int64_t *n_fillings,
+                         void *stream);
+
 /* ---- multi-GPU staging (SURVEY §8e): the interval table is replicated, the pair space is sharded ----
  * fslrc_mg_prepare     : ingestion + sort/band on this device (identical on every rank)
  * fslrc_mg_pair        : candidate generation + pair tests for the query reads of shard `rank` of `world`; leaves one
