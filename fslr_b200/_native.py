@@ -13,7 +13,7 @@ SYMBOLS = ["fslrc_create", "fslrc_destroy", "fslrc_last_error", "fslrc_stage_nam
            "fslrc_cluster_device", "fslrc_cluster_host", "fslrc_filling_starts", "fslrc_mg_prepare", "fslrc_mg_pair", "fslrc_mg_partners", "fslrc_mg_replay",
            "fslrc_mg_finish", "fslrc_int_peak", "fslrc_launch_count", "fslrc_set_blocking_sync", "fslrc_choose_alignment_host",
            "fslrc_tsv_open", "fslrc_tsv_delete_false", "fslrc_tsv_chrom_name", "fslrc_tsv_read_names", "fslrc_tsv_write_cluster_bed", "fslrc_tsv_write_representative_bed",
-           "fslrc_tsv_close",
+           "fslrc_tsv_write_edges", "fslrc_tsv_close", "fslrc_set_edge_capture", "fslrc_edges",
            "fslrc_bam_open", "fslrc_bam_open_bgzf", "fslrc_bam_read_stream", "fslrc_bam_write_mappings_bed", "fslrc_bam_read_names", "fslrc_bam_close"]
 
 ERRORS = {-1: "FSLRC_ERR_CUDA", -2: "FSLRC_ERR_ARG", -3: "FSLRC_ERR_ZERO_DIVISOR", -4: "FSLRC_ERR_TOO_MANY_FILLINGS",
@@ -109,6 +109,9 @@ def load():
     lib.fslrc_tsv_read_names.argtypes = [vp, vp, vp]
     lib.fslrc_tsv_write_cluster_bed.argtypes = [vp, vp, vp, vp, C.c_int64, i64p, vp]
     lib.fslrc_tsv_write_representative_bed.argtypes = [vp, vp, vp, vp, C.c_int64, i64p, vp]
+    lib.fslrc_tsv_write_edges.argtypes = [vp, vp, C.c_int64, i64p, vp]
+    lib.fslrc_set_edge_capture.argtypes = [vp, C.c_int]
+    lib.fslrc_edges.argtypes = [vp, vp, vp, vp, C.c_int64, i64p, vp]
     lib.fslrc_tsv_close.argtypes = [vp]
     lib.fslrc_tsv_close.restype = None
     lib.fslrc_bam_open.argtypes = [vp, vp, C.c_int64, C.c_int64, C.c_int32, C.c_char_p, vp, C.c_int32, vp, vp, vp, C.c_int32, C.c_uint64,

@@ -154,6 +154,15 @@ class ClusterGraph:
     def number_of_edges(self):
         return int(self.result.stats["edges"])
 
+    def edges(self):
+        """The graph's edges as (query1, query2) qname pairs, in match_df's row order.  Needs the graph to have been
+        captured: query_interval_trees(..., with_matches=True)."""
+        e = self.result.edges
+        if e is None:
+            raise RuntimeError("the similarity graph was not captured: call query_interval_trees(..., with_matches=True)")
+        q = self.table.qnames
+        return [(q[a], q[b]) for a, b in zip(e.read1.tolist(), e.read2.tolist())]
+
 
 def keep_fillings(bed_file):
     return Fillings(bed_file)
@@ -169,19 +178,30 @@ def build_interval_trees(data):
     return IntervalIndex(data)
 
 
-def _run(table, params, tie_order, device):
+def _run(table, params, tie_order, device, edges=False):
     order = reference_tie_order(table) if tie_order == "reference" else None
     try:
-        return get_engine(device).cluster(table, params, order=order)
+        return get_engine(device).cluster(table, params, order=order, edges=edges)
     except FslrError as e:
         if e.code == -3:
             raise ZeroDivisionError(str(e))      # what cluster.py:135,179,181 raise
         raise
 
 
+def match_frame(qnames, edges):
+    """cluster.py:226's match_df from an EdgeList: query1, query2 (qnames), jaccard_similarity (float64)."""
+    if edges is None:
+        return pd.DataFrame(columns=["query1", "query2", "jaccard_similarity"])
+    q = np.asarray(qnames, dtype=object)
+    return pd.DataFrame({"query1": q[edges.read1], "query2": q[edges.read2], "jaccard_similarity": edges.jaccard})
+
+
 def query_interval_trees(interval_trees, data, overlap_cutoff, jaccard_threshold, edge_threshold, qlen_diff, diff,
-                         tie_order=None, device=0):
-    """cluster.py:187-227.  Returns (match_df, G): match_df is unused by main.py:242 and comes back empty."""
+                         tie_order=None, device=0, with_matches=False):
+    """cluster.py:187-227.  Returns (match_df, G).  main.py:242 ignores match_df, so by default it comes back empty;
+    with_matches=True fills it with one row per edge of the similarity graph (query1 = the read whose query tested the
+    pair, query2, jaccard_similarity), sorted by the order in which cluster.py:197 visits query1 and query2, and lets
+    G.edges() list the same pairs."""
     d = data if isinstance(data, PreparedData) else interval_trees.data
     table = ColumnarTable.from_dataframe(d.bed_file, {k: v for k, v in d.chromosome_lengths.items() if k is not None})
     masked = np.zeros(table.n_chrom, dtype=np.uint8)
@@ -194,9 +214,8 @@ def query_interval_trees(interval_trees, data, overlap_cutoff, jaccard_threshold
     params = ClusterParams(jaccard_cutoffs=[float(x) for x in jaccard_threshold], overlap=float(overlap_cutoff),
                            n_alignment_diff=float(diff), qlen_diff=float(qlen_diff), chrom_masked=masked,
                            mask_subtelomere=sub, subtel=int(d.threshold), edge_threshold=int(edge_threshold))
-    res = _run(table, params, tie_order or TIE_ORDER, device)
-    match_df = pd.DataFrame(columns=["query1", "query2", "jaccard_similarity"])
-    return match_df, ClusterGraph(table, res)
+    res = _run(table, params, tie_order or TIE_ORDER, device, edges=with_matches)
+    return match_frame(table.qnames, res.edges), ClusterGraph(table, res)
 
 
 def get_subgraphs(G):
@@ -213,16 +232,17 @@ def get_subgraphs(G):
 # ---------------------------------------------------------------- fused entry
 def cluster_table(table, chr_lengths=None, cluster_mask="subtelomere", jaccard_cutoffs="1,1,0.66,0.66,0.66,0.5",
                   overlap=0.8, n_alignment_diff=0.25, qlen_diff=0.04, edge_threshold=10, subtel=SUBTEL_DEFAULT,
-                  order=None, tie_order=None, device=0) -> ClusterResult:
+                  order=None, tie_order=None, device=0, edges=False) -> ClusterResult:
     """table: ColumnarTable or a DataFrame as read at main.py:209 (then chr_lengths is the BAM-header dict).
-    Returns per-read-id `cluster` / `n_reads` (read id = order of first appearance of qname)."""
+    Returns per-read-id `cluster` / `n_reads` (read id = order of first appearance of qname); edges=True adds the
+    similarity graph (ClusterResult.edges)."""
     if not isinstance(table, ColumnarTable):
         table = ColumnarTable.from_dataframe(table, chr_lengths or {})
     params = ClusterParams.from_options(table, cluster_mask, jaccard_cutoffs, overlap, n_alignment_diff, qlen_diff,
                                         edge_threshold, subtel)
     if order is not None:
-        return get_engine(device).cluster(table, params, order=order)
-    return _run(table, params, tie_order or TIE_ORDER, device)
+        return get_engine(device).cluster(table, params, order=order, edges=edges)
+    return _run(table, params, tie_order or TIE_ORDER, device, edges=edges)
 
 
 def choose_alignment(bed_file, device=0):

@@ -60,10 +60,28 @@ struct fslrc_ctx {
     cudaStream_t copy_stream;
     cudaEvent_t ev_c1, ev_c2;
     bool late_pending;
+    int edge_capture;        // fslrc_set_edge_capture
+    struct EdgeList *edges;  // edge list of the last clustering call (capture on), kept until the next one
+    long long tsv_gen;       // bumped by fslrc_tsv_open / fslrc_tsv_delete_false: which parsed table a captured list names
 };
+// the similarity graph of one clustering call, sorted by (query rank of read1, query rank of read2); device arrays
+struct EdgeList {
+    int32_t *read1, *read2;
+    double *jac;
+    int64_t n;
+    const int32_t *read_id_col;  // the table's read_id column and ...
+    long long tsv_gen;           // ... ctx->tsv_gen at the call: the renderer checks both against the parsed table
+};
+static void edges_free(fslrc_ctx *ctx) {
+    if (!ctx->edges) return;
+    void *p[] = {ctx->edges->read1, ctx->edges->read2, ctx->edges->jac};
+    for (void *q : p) if (q) cudaFreeAsync(q, ctx->stream);
+    delete ctx->edges; ctx->edges = nullptr;
+}
 
 static void tsv_free(fslrc_ctx *ctx);
 static void bam_free(fslrc_ctx *ctx);
+static const int32_t *tsv_read_id(const fslrc_ctx *ctx);
 
 enum { ST_H2D = 0, ST_KEEP, ST_ORDER, ST_QRANK, ST_CHROM, ST_BANDS, ST_CAND, ST_PAIR, ST_HEAVY, ST_SAT, ST_REPLAY, ST_UNION, ST_NUMBER, ST_D2H };
 static const char *STAGE_NAMES[FSLRC_N_STAGES] = {
@@ -694,6 +712,46 @@ static int pipe_number(fslrc_ctx *ctx, Pipe *P, int *out_cluster, int *out_n) {
     return mark(ctx, ST_NUMBER);
 }
 
+// ---- edge capture (after union-find, before the scratch goes): the directed edges of the relation entries and of the replay,
+// which k_union_entries / k_union_edges handed to union-find, with their Jaccard similarity, in query-rank order
+static int export_edges(fslrc_ctx *ctx, Pipe *P, const int32_t *read_id_col) {
+    cudaStream_t st = ctx->stream;
+    const int Q = P->Q, R = P->R, TB = 256;
+    { int r = read_counts(ctx, P); if (r) return r; r = err_code(ctx); if (r) return r; }
+    const long long E = ctx->h_pin[8];
+    if (E > 0x7ffffff0LL) return fail(ctx, FSLRC_ERR_OVERFLOW, "edge capture: more than 2^31 edges");
+    const unsigned long long nent = std::min<unsigned long long>((unsigned long long)ctx->h_pin[5], P->cap_entries);
+    const unsigned long long nped = std::min<unsigned long long>((unsigned long long)ctx->h_pin[7], P->cap_pedges);
+    const int n = (int)E;
+    EdgeList *L = new EdgeList();
+    memset(L, 0, sizeof(*L));
+    L->n = n; L->read_id_col = read_id_col;
+    L->tsv_gen = (read_id_col && read_id_col == tsv_read_id(ctx)) ? ctx->tsv_gen : -1;
+    ctx->edges = L;
+    CK(cudaMallocAsync((void **)&L->read1, sizeof(int32_t) * (size_t)std::max(n, 1), st));
+    CK(cudaMallocAsync((void **)&L->read2, sizeof(int32_t) * (size_t)std::max(n, 1), st));
+    CK(cudaMallocAsync((void **)&L->jac, sizeof(double) * (size_t)std::max(n, 1), st));
+    int2 *dir; unsigned long long *cnt; int *rid_of_q, *iota, *perm1, *perm; unsigned *key, *key2;
+    DA(dir, n); DA(cnt, 1); DA(rid_of_q, Q); DA(iota, n); DA(perm1, n); DA(perm, n); DA(key, n); DA(key2, n);
+    CK(cudaMemsetAsync(cnt, 0, sizeof(unsigned long long), st));
+    if (nent > 0) KL(k_edges_of_entries, nblk((int64_t)nent, TB), TB, nent, P->entries, P->isP, P->tab, P->stop, dir, (unsigned long long)n, cnt);
+    if (nped > 0) KL(k_edges_of_pedges, nblk((int64_t)nped, TB), TB, nped, P->pedges, dir, (unsigned long long)n, cnt);
+    CK(cudaMemcpyAsync(ctx->h_pin + 60, cnt, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CK(ctx_sync(ctx));
+    if (ctx->h_pin[60] != E) return fail(ctx, FSLRC_ERR_OVERFLOW, "internal: the edge export disagrees with the union-find edge count");
+    if (R > 0) KL(k_rid_of_q, nblk(R, TB), TB, R, P->q_of_rid, rid_of_q);
+    if (n > 0) {
+        const int qb = bits_for(Q);
+        KL(k_edges_key2, nblk(n, TB), TB, n, dir, key, iota);
+        int r = sort_pairs(ctx, P, key, key2, iota, perm1, n, 0, qb); if (r) return r;
+        KL(k_edges_key1, nblk(n, TB), TB, n, dir, perm1, key);
+        r = sort_pairs(ctx, P, key, key2, perm1, perm, n, 0, qb); if (r) return r;
+        if (!(P->pr.overlap > 0.0)) KL(k_edges_final<true>, nblk(n, TB), TB, n, P->tab, dir, perm, rid_of_q, L->read1, L->read2, L->jac);
+        else KL(k_edges_final<false>, nblk(n, TB), TB, n, P->tab, dir, perm, rid_of_q, L->read1, L->read2, L->jac);
+    }
+    return 0;
+}
+
 static void fill_stats(fslrc_ctx *ctx, Pipe *P, fslrc_stats *s) {
     if (!s) return;
     const int64_t *h = ctx->h_pin;
@@ -863,6 +921,7 @@ int fslrc_create(int device, fslrc_ctx **out) {
     cudaEventCreateWithFlags(&ctx->ev_block, cudaEventBlockingSync | cudaEventDisableTiming);
     ctx->blocking = 0;
     ctx->copy_stream = nullptr; ctx->late_pending = false;
+    ctx->edge_capture = 0; ctx->edges = nullptr; ctx->tsv_gen = 0;
     if (cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking) != cudaSuccess) { ctx->copy_stream = nullptr; cudaGetLastError(); }
     cudaEventCreateWithFlags(&ctx->ev_c1, cudaEventDisableTiming);
     cudaEventCreateWithFlags(&ctx->ev_c2, cudaEventDisableTiming);
@@ -880,6 +939,7 @@ int fslrc_create(int device, fslrc_ctx **out) {
 void fslrc_destroy(fslrc_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
+    edges_free(ctx);
     free_all(ctx);
     tsv_free(ctx);
     bam_free(ctx);
@@ -893,8 +953,17 @@ void fslrc_destroy(fslrc_ctx *ctx) {
     delete ctx;
 }
 
+// a clustering call drops the edge list of the previous one first (also when it fails)
+static void begin_clustering(fslrc_ctx *ctx, void *stream) {
+    if (!ctx || !ctx->edges) return;
+    cudaSetDevice(ctx->device);
+    ctx->stream = (cudaStream_t)stream;
+    edges_free(ctx);
+}
+
 int fslrc_cluster_device(fslrc_ctx *ctx, const fslrc_table *table, const fslrc_params *params, int32_t *out_cluster,
                          int32_t *out_n_reads, fslrc_stats *stats, void *stream) {
+    begin_clustering(ctx, stream);
     int r = check_args(ctx, table, params, out_cluster, out_n_reads); if (r) return r;
     CK(cudaSetDevice(ctx->device));
     ctx->stream = (cudaStream_t)stream;
@@ -905,15 +974,18 @@ int fslrc_cluster_device(fslrc_ctx *ctx, const fslrc_table *table, const fslrc_p
     if (!r) CK(cudaEventRecord(ctx->ev[1], ctx->stream));                  // closes stage 0 (widening of narrow columns, if any)
     if (!r) r = run_device(ctx, &P, out_cluster, out_n_reads, stats);
     if (!r) { r = mark(ctx, ST_D2H); }
+    if (!r && ctx->edge_capture) r = export_edges(ctx, &P, table->read_id);
     if (!r) { r = read_counts(ctx, &P); if (!r) r = err_code(ctx); }
     if (!r) fill_stats(ctx, &P, stats);
     free_all(ctx);
+    if (r) edges_free(ctx);
     ctx_sync(ctx);
     return r;
 }
 
 int fslrc_cluster_host(fslrc_ctx *ctx, const fslrc_table *table, const fslrc_params *params, int32_t *out_cluster,
                        int32_t *out_n_reads, fslrc_stats *stats, void *stream) {
+    begin_clustering(ctx, stream);
     int r = check_args(ctx, table, params, out_cluster, out_n_reads); if (r) return r;
     CK(cudaSetDevice(ctx->device));
     ctx->stream = (cudaStream_t)stream;
@@ -933,9 +1005,11 @@ int fslrc_cluster_host(fslrc_ctx *ctx, const fslrc_table *table, const fslrc_par
         CK(cudaMemcpyAsync(out_n_reads, d_on, sizeof(int32_t) * R, cudaMemcpyDeviceToHost, st));
     }
     if (!r) r = mark(ctx, ST_D2H);
+    if (!r && ctx->edge_capture) r = export_edges(ctx, &P, nullptr);
     if (!r) { r = read_counts(ctx, &P); if (!r) r = err_code(ctx); }
     if (!r) fill_stats(ctx, &P, stats);
     free_all(ctx);
+    if (r) edges_free(ctx);
     ctx_sync(ctx);
     return r;
 }
@@ -976,6 +1050,7 @@ int fslrc_filling_starts(fslrc_ctx *ctx, const fslrc_table *table, int32_t *out_
 
 // ---------------------------------------------------------------- multi-GPU staging
 int fslrc_mg_prepare(fslrc_ctx *ctx, const fslrc_table *table, const fslrc_params *params, void *stream) {
+    begin_clustering(ctx, stream);                                      // (the multi-GPU sequence captures no edges)
     int dummy = 0;
     int r = check_args(ctx, table, params, &dummy, &dummy); if (r) return r;
     CK(cudaSetDevice(ctx->device));
@@ -1107,6 +1182,7 @@ static int palloc(fslrc_ctx *ctx, T **p, int64_t n) {                  // persis
     return 0;
 }
 #define PA(ptr, n) do { int r__ = palloc(ctx, &(ptr), (int64_t)(n)); if (r__) return r__; } while (0)
+static const int32_t *tsv_read_id(const fslrc_ctx *ctx) { return ctx->tsv ? ctx->tsv->read_id : nullptr; }
 static void tsv_free(fslrc_ctx *ctx) {
     if (!ctx->tsv) return;
     for (void *p : ctx->tsv->allocs) cudaFreeAsync(p, ctx->stream);
@@ -1150,6 +1226,7 @@ static int tsv_open_impl(fslrc_ctx *ctx, const char *text, int64_t n_bytes, uint
         for (int k = 0; k < tsv::W_SCORE; k++) if (w.col[k] < 0) return fail(ctx, FSLRC_ERR_ARG, "tsv: header lacks column %s", names[k]);
     }
     TsvState *T = ctx->tsv = new TsvState();
+    ctx->tsv_gen++;
     Pipe Pp; memset((void *)&Pp, 0, sizeof(Pp)); Pipe *P = &Pp;       // (scratch of the scan primitive)
     const bool pad = text[n_bytes - 1] != '\n';
     T->n = n_bytes + (pad ? 1 : 0);
@@ -1235,6 +1312,7 @@ static int tsv_delete_false_impl(fslrc_ctx *ctx, fslrc_tsv_info *info, void *str
     cudaStream_t st = ctx->stream;
     TsvState *T = ctx->tsv;
     const int n = T->n_rows, R = T->n_reads, TB = 256;
+    ctx->tsv_gen++;
     CK(cudaEventRecord(ctx->ev[1], st));
     if (R > 0) {
         Pipe Pp; memset((void *)&Pp, 0, sizeof(Pp)); Pipe *P = &Pp;
@@ -1403,6 +1481,43 @@ int fslrc_tsv_write_representative_bed(fslrc_ctx *ctx, const int32_t *cluster_de
     CK(cudaStreamSynchronize(st));
     return rc;
 }
+int fslrc_tsv_write_edges(fslrc_ctx *ctx, char *out, int64_t cap, int64_t *n_out, void *stream) {
+    if (!ctx) return FSLRC_ERR_ARG;
+    if (!n_out) return fail(ctx, FSLRC_ERR_ARG, "tsv: null n_out");
+    TsvState *T = ctx->tsv;
+    const EdgeList *E = ctx->edges;
+    if (!T || !E || E->tsv_gen != ctx->tsv_gen || E->read_id_col != T->read_id)
+        return fail(ctx, FSLRC_ERR_ARG, "tsv: no captured edge list of a clustering of the table that is open now "
+                                        "(fslrc_set_edge_capture, then fslrc_cluster_device on this table's columns)");
+    CK(cudaSetDevice(ctx->device));
+    ctx->stream = (cudaStream_t)stream;
+    cudaStream_t st = ctx->stream;
+    Pipe Pp; memset((void *)&Pp, 0, sizeof(Pp)); Pipe *P = &Pp;
+    const int n = (int)E->n, L = n + 1, TB = 256;
+    long long *len, *off; int64_t *tot;
+    DA(len, L); DA(off, L); DA(tot, 1);
+    KL(tsv::k_tsv_edge_outlen, nblk(L, TB), TB, n, E->read1, E->read2, E->jac, T->first_row, T->q_len, len);
+    {
+        const int tiles = nblk(L, prims::SC_TILE);
+        int r = prim_scratch(ctx, P, sizeof(unsigned long long) * tiles); if (r) return r;
+        KL(prims::k_scan_excl<long long>, tiles, prims::SC_THREADS, len, off, L, (unsigned long long *)(P->prim + 256), (unsigned *)P->prim, (long long *)tot);
+    }
+    CK(cudaMemcpyAsync(ctx->h_pin, tot, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    *n_out = ctx->h_pin[0];
+    int rc = 0;
+    if (out) {
+        if (cap < *n_out) rc = fail(ctx, FSLRC_ERR_ARG, "tsv: output buffer too small");
+        else {
+            unsigned char *d_out; DA(d_out, *n_out);
+            KL(tsv::k_tsv_edge_emit, nblk((int64_t)L * 32, TB), TB, n, T->text, E->read1, E->read2, E->jac, T->first_row, T->q_off, T->q_len, off, d_out);
+            CK(cudaMemcpyAsync(out, d_out, *n_out, cudaMemcpyDeviceToHost, st));
+        }
+    }
+    free_all(ctx);
+    CK(cudaStreamSynchronize(st));
+    return rc;
+}
 void fslrc_tsv_close(fslrc_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
@@ -1414,6 +1529,36 @@ void fslrc_tsv_close(fslrc_ctx *ctx) {
 int fslrc_set_blocking_sync(fslrc_ctx *ctx, int on) {
     if (!ctx) return FSLRC_ERR_ARG;
     ctx->blocking = on != 0;
+    return 0;
+}
+
+int fslrc_set_edge_capture(fslrc_ctx *ctx, int on) {
+    if (!ctx) return FSLRC_ERR_ARG;
+    ctx->edge_capture = on != 0;
+    if (!on && ctx->edges) {
+        CK(cudaSetDevice(ctx->device));
+        edges_free(ctx);
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    return 0;
+}
+
+int fslrc_edges(fslrc_ctx *ctx, int32_t *read1, int32_t *read2, double *jaccard, int64_t cap, int64_t *n_edges, void *stream) {
+    if (!ctx) return FSLRC_ERR_ARG;
+    if (!n_edges) return fail(ctx, FSLRC_ERR_ARG, "edges: null n_edges");
+    const EdgeList *E = ctx->edges;
+    if (!E) return fail(ctx, FSLRC_ERR_ARG, "edges: the last clustering call captured no edge list (capture off, the call failed, "
+                                            "or it was a fslrc_mg_* sequence)");
+    *n_edges = E->n;
+    if (!read1 && !read2 && !jaccard) return 0;                          // size query
+    if (cap < E->n) return fail(ctx, FSLRC_ERR_ARG, "edges: output buffers too small (cap < n_edges)");
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (E->n > 0) {
+        if (read1) CK(cudaMemcpyAsync(read1, E->read1, sizeof(int32_t) * E->n, cudaMemcpyDeviceToDevice, st));
+        if (read2) CK(cudaMemcpyAsync(read2, E->read2, sizeof(int32_t) * E->n, cudaMemcpyDeviceToDevice, st));
+        if (jaccard) CK(cudaMemcpyAsync(jaccard, E->jac, sizeof(double) * E->n, cudaMemcpyDeviceToDevice, st));
+    }
     return 0;
 }
 

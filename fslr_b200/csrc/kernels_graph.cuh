@@ -23,7 +23,30 @@ __device__ __forceinline__ void uf_union(int *parent, int a, int b) {
 }
 // entries (a, b) recorded by k_eval / k_pair (a -> b evaluated; only the passing ones matter here): a not saturating;
 // b > a -> a tested it (edge); b < a -> edge only if b is saturating and its scan stopped before reaching a (then a's
-// query tested the pair, direction a -> b)
+// query tested the pair, direction a -> b).  The rules live in the three functions below, which k_union_entries and the
+// edge export (k_edges_of_entries) share.
+// the directed pairs a slot stands for that pass the Jaccard cutoff: (a, b), and in symmetric mode (b, a)
+__device__ __forceinline__ bool slot_fwd(const int2 ab) { return ab.x >= 0 && !((unsigned)ab.y & EB_NOPASS); }
+__device__ __forceinline__ bool slot_rev(const int2 ab) {
+    return ab.x >= 0 && ((unsigned)ab.y & EB_SYM) && !((unsigned)ab.y & EB_NOPASS2);
+}
+// a -> b passes and a is not saturating: is it an edge of the reference's graph, i.e. did a's query test the pair?
+__device__ __forceinline__ bool directed_is_edge(const Tab &t, const int *isP, const int *stop, int a, int b) {
+    if (b > a) return true;
+    if (!isP[b]) return false;
+    const int wa = t.RI[a].w, wb = t.RI[b].w;
+    const int offa = (int)((unsigned)wa >> 6), La = (wa & 63) + 1, offb = (int)((unsigned)wb >> 6), Lb = (wb & 63) + 1;
+    for (int f = 0; f < Lb; f++) {                                                  // some scan of b got down to a: b's query saw it
+        const int4 bf = rm0(t, offb + f);
+        const int ubf = rm1(t, offb + f).y, sf = stop[offb + f];
+        for (int g = 0; g < La; g++) {
+            const int4 ag = rm0(t, offa + g);
+            const int pg = rm1(t, offa + g).x;
+            if (ag.x == bf.x && sf <= pg && pg <= ubf && ag.z >= bf.y) return false;
+        }
+    }
+    return true;
+}
 #define UE_PER 4
 #define UE_THREADS 256
 // Only about a third of the list's slots are edges (the rest: padding, pairs of saturating reads, pairs that do not pass), and
@@ -47,8 +70,8 @@ __global__ void __launch_bounds__(UE_THREADS) k_union_entries(unsigned long long
 #pragma unroll
     for (int u = 0; u < UE_PER; u++) {                                              // 1: nothing to do for that direction
         const unsigned y = (unsigned)ab[u].y;
-        pa[u] = (ab[u].x >= 0 && !(y & EB_NOPASS)) ? __ldg(&isP[ab[u].x]) : 1;
-        pb[u] = (ab[u].x >= 0 && (y & EB_SYM) && !(y & EB_NOPASS2)) ? __ldg(&isP[y & QMASK]) : 1;
+        pa[u] = slot_fwd(ab[u]) ? __ldg(&isP[ab[u].x]) : 1;
+        pb[u] = slot_rev(ab[u]) ? __ldg(&isP[y & QMASK]) : 1;
     }
     int mine = 0;
 #pragma unroll
@@ -71,25 +94,7 @@ __global__ void __launch_bounds__(UE_THREADS) k_union_entries(unsigned long long
     int ne = 0;
     for (int idx = tid; idx < total; idx += UE_THREADS) {
         const int a = sE[idx].x, b = sE[idx].y;
-        bool e = true;
-        if (b < a) {
-            e = false;
-            if (isP[b]) {
-                const int wa = t.RI[a].w, wb = t.RI[b].w;
-                const int offa = (int)((unsigned)wa >> 6), La = (wa & 63) + 1, offb = (int)((unsigned)wb >> 6), Lb = (wb & 63) + 1;
-                e = true;
-                for (int f = 0; f < Lb && e; f++) {
-                    const int4 bf = rm0(t, offb + f);
-                    const int ubf = rm1(t, offb + f).y, sf = stop[offb + f];
-                    for (int g = 0; g < La; g++) {
-                        const int4 ag = rm0(t, offa + g);
-                        const int pg = rm1(t, offa + g).x;
-                        if (ag.x == bf.x && sf <= pg && pg <= ubf && ag.z >= bf.y) { e = false; break; }
-                    }
-                }
-            }
-        }
-        if (e) { ing[a] = 1; ing[b] = 1; uf_union(parent, a, b); ne++; }
+        if (directed_is_edge(t, isP, stop, a, b)) { ing[a] = 1; ing[b] = 1; uf_union(parent, a, b); ne++; }
     }
     for (int o = 16; o; o >>= 1) ne += __shfl_down_sync(0xffffffffu, ne, o);
     if (lane == 0 && ne) atomicAdd(&s_ne, ne);
@@ -109,6 +114,82 @@ __global__ void k_union_edges(unsigned long long n, const int2 *__restrict__ edg
     }
     const int cnt = __syncthreads_count(e);
     if (threadIdx.x == 0 && cnt && n_edges) atomicAdd(n_edges, (unsigned long long)cnt);
+}
+// ---------------------------------------------------------------- edge export (fslrc_set_edge_capture)
+// Every edge union-find was handed, as the directed pair (query read, other read): the first read is the one whose query
+// tested the pair (cluster.py:197-220's query_key).  Appended in any order; k_edges_final puts them in a fixed one.
+__device__ __forceinline__ unsigned long long warp_reserve(int c, unsigned long long *n_out) {   // warp-aggregated append
+    const int lane = threadIdx.x & 31;
+    int incl = c;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += y; }
+    unsigned long long base = 0;
+    if (lane == 31 && incl) base = atomicAdd(n_out, (unsigned long long)incl);
+    return __shfl_sync(0xffffffffu, base, 31) + (unsigned long long)(incl - c);
+}
+__global__ void k_edges_of_entries(unsigned long long n, const int2 *__restrict__ entries, const int *__restrict__ isP, Tab t,
+                                   const int *stop, int2 *out, unsigned long long cap, unsigned long long *n_out) {
+    const unsigned long long k = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x;
+    const int2 ab = k < n ? entries[k] : make_int2(-1, -1);
+    const int a = ab.x, b = ab.y & QMASK;
+    const bool e1 = slot_fwd(ab) && !isP[a] && directed_is_edge(t, isP, stop, a, b);
+    const bool e2 = slot_rev(ab) && !isP[b] && directed_is_edge(t, isP, stop, b, a);
+    unsigned long long at = warp_reserve((int)e1 + (int)e2, n_out);
+    if (e1) { if (at < cap) out[at] = make_int2(a, b); at++; }
+    if (e2 && at < cap) out[at] = make_int2(b, a);
+}
+__global__ void k_edges_of_pedges(unsigned long long n, const int2 *__restrict__ pedges, int2 *out, unsigned long long cap,
+                                  unsigned long long *n_out) {
+    const unsigned long long k = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x;
+    const int2 ab = k < n ? pedges[k] : make_int2(-1, -1);
+    const bool e = ab.x >= 0;                                                       // skip chunk padding
+    const unsigned long long at = warp_reserve((int)e, n_out);
+    if (e && at < cap) out[at] = ab;
+}
+// radix keys of the two stable passes: first by the second read's query rank, then (gathered) by the first read's
+__global__ void k_edges_key2(int n, const int2 *__restrict__ dir, unsigned *key, int *iota) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    key[i] = (unsigned)dir[i].y; iota[i] = i;
+}
+__global__ void k_edges_key1(int n, const int2 *__restrict__ dir, const int *__restrict__ perm, unsigned *key) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    key[i] = (unsigned)dir[perm[i]].x;
+}
+__global__ void k_rid_of_q(int R, const int *__restrict__ q_of_rid, int *rid_of_q) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= R) return;
+    const int q = q_of_rid[r];
+    if (q >= 0) rid_of_q[q] = r;
+}
+// cluster.py:140-170 in the edge's direction: list1 = the query read's fillings in data order, list2 = the other's; each
+// filling of list1 takes the first free matching filling of list2 (k_eval's predicate, ALLMATCH for --overlap <= 0)
+template <bool ALLMATCH>
+__device__ int greedy_count(const Tab &t, int q1, int q2, int *L1, int *L2) {
+    const int w1 = __ldg(&t.RI[q1]).w, w2 = __ldg(&t.RI[q2]).w;
+    const int off1 = (int)((unsigned)w1 >> 6), La = (w1 & 63) + 1, off2 = (int)((unsigned)w2 >> 6), Lb = (w2 & 63) + 1;
+    unsigned long long used = 0;
+    int n = 0;
+    for (int fa = 0; fa < La; fa++) {
+        const int4 a = rm0(t, off1 + fa);
+        for (int fb = 0; fb < Lb; fb++)
+            if (!((used >> fb) & 1ull) && matchT<ALLMATCH>(a, rm0(t, off2 + fb))) { used |= 1ull << fb; n++; break; }
+    }
+    *L1 = La; *L2 = Lb;
+    return n;
+}
+// the sorted list: read ids and the Jaccard similarity n / (L1 + L2 - n), the IEEE division CPython does
+template <bool ALLMATCH>
+__global__ void k_edges_final(int n, Tab t, const int2 *__restrict__ dir, const int *__restrict__ perm, const int *__restrict__ rid_of_q,
+                              int *read1, int *read2, double *jac) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int2 e = dir[perm[i]];
+    int L1, L2;
+    const int c = greedy_count<ALLMATCH>(t, e.x, e.y, &L1, &L2);
+    read1[i] = rid_of_q[e.x]; read2[i] = rid_of_q[e.y];
+    jac[i] = __ddiv_rn((double)c, (double)(L1 + L2 - c));
 }
 __global__ void k_flatten(int Q, int *parent, const int *__restrict__ ing, int *isroot, int *csize) {
     int q = blockIdx.x * blockDim.x + threadIdx.x;

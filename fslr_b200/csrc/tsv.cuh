@@ -307,4 +307,43 @@ __global__ void k_tsv_rep_emit(int n_lines, const unsigned char *__restrict__ te
     }
 }
 
+// ---- the similarity graph's edges (fslrc_tsv_write_edges): match_df.to_csv(sep="\t", index=False) of cluster.py:226's frame
+constexpr int EDGE_HEADER_LEN = 33;                                     // "query1\tquery2\tjaccard_similarity\n"
+// line 0: the header; line l > 0: edge l - 1 = "<qname of read1>\t<qname of read2>\t<repr(jaccard)>\n"
+__global__ void k_tsv_edge_outlen(int n_edges, const int *__restrict__ read1, const int *__restrict__ read2, const double *__restrict__ jac,
+                                  const int *__restrict__ first_row, const int *__restrict__ q_len, long long *len) {
+    const int l = blockIdx.x * blockDim.x + threadIdx.x;
+    if (l > n_edges) return;
+    if (l == 0) { len[0] = EDGE_HEADER_LEN; return; }
+    char buf[fmtd::FMT_F64_MAX];
+    const int e = l - 1;
+    len[l] = (long long)q_len[first_row[read1[e]]] + q_len[first_row[read2[e]]] + fmtd::fmt_repr_f64(jac[e], buf) + 3;
+}
+// one warp per line: coalesced copies of both names, lane 0 writes the separators and the formatted value
+__global__ void k_tsv_edge_emit(int n_edges, const unsigned char *__restrict__ text, const int *__restrict__ read1,
+                                const int *__restrict__ read2, const double *__restrict__ jac, const int *__restrict__ first_row,
+                                const long long *__restrict__ q_off, const int *__restrict__ q_len, const long long *__restrict__ out_off,
+                                unsigned char *out) {
+    const long long wg = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (wg > n_edges) return;
+    const int l = (int)wg;
+    unsigned char *o = out + out_off[l];
+    if (l == 0) { if (lane == 0) put_str(o, "query1\tquery2\tjaccard_similarity\n"); return; }
+    const int e = l - 1, f1 = first_row[read1[e]], f2 = first_row[read2[e]];
+    const long long s1 = q_off[f1], s2 = q_off[f2];
+    const int n1 = q_len[f1], n2 = q_len[f2];
+    for (int i = lane; i < n1; i += 32) o[i] = text[s1 + i];
+    for (int i = lane; i < n2; i += 32) o[n1 + 1 + i] = text[s2 + i];
+    if (lane == 0) {
+        char buf[fmtd::FMT_F64_MAX];
+        const int nj = fmtd::fmt_repr_f64(jac[e], buf);
+        o[n1] = '\t';
+        unsigned char *q = o + n1 + 1 + n2;
+        *q++ = '\t';
+        for (int i = 0; i < nj; i++) *q++ = (unsigned char)buf[i];
+        *q = '\n';
+    }
+}
+
 }  // namespace tsv

@@ -33,11 +33,22 @@ def umax_table(cutoffs, n_max=_native.MAX_FILLINGS):
 
 
 @dataclass
+class EdgeList:
+    """The similarity graph of one clustering call (cluster.py:187-227's match_df / G), one row per edge handed to
+    union-find: read1 is the read whose query tested the pair (match_df's query1), jaccard its Jaccard similarity in that
+    direction.  Rows sorted by (query rank of read1, query rank of read2)."""
+    read1: np.ndarray          # int32 read id
+    read2: np.ndarray          # int32 read id
+    jaccard: np.ndarray        # float64
+
+
+@dataclass
 class ClusterResult:
     cluster: np.ndarray        # int32 per read id: the `cluster` value main.py:334-342 writes for that read's rows
     n_reads: np.ndarray        # int32 per read id
     no_clusters: bool          # main.py:247-249 early return ("No clusters were found.")
     stats: dict
+    edges: EdgeList = None     # the similarity graph, when the call asked for it (edges=True)
 
 
 class DeviceTable:
@@ -171,6 +182,7 @@ class Engine:
         rc = self.lib.fslrc_create(device, C.byref(self.ctx))
         if rc != 0:
             raise _native.FslrError(rc, "fslrc_create failed")
+        self._capture = False
 
     def pinned_bytes(self, n):
         """A pinned uint8 staging buffer of at least n bytes, kept and reused (pinning hundreds of MB costs more than the
@@ -235,17 +247,43 @@ class Engine:
         if rc != 0:
             raise _native.FslrError(rc, self.lib.fslrc_last_error(self.ctx).decode())
 
+    # ---- edge capture (fslrc_set_edge_capture)
+    def _set_capture(self, on):
+        """A call with edges=True switches capture on and leaves it on, so that the list stays in the context for the
+        renderer (ParsedBed.edges_bytes); the next call without edges switches it off first (which frees the list)."""
+        if bool(on) != self._capture:
+            self._check(self.lib.fslrc_set_edge_capture(self.ctx, int(bool(on))))
+            self._capture = bool(on)
+
+    def edge_list(self):
+        """The edge list the last clustering call captured (fslrc_edges), as host arrays."""
+        n = C.c_int64()
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        self._check(self.lib.fslrc_edges(self.ctx, None, None, None, 0, C.byref(n), C.c_void_p(stream)))
+        m = max(n.value, 1)
+        r1 = torch.empty(m, dtype=torch.int32, device=self.device)
+        r2 = torch.empty(m, dtype=torch.int32, device=self.device)
+        jac = torch.empty(m, dtype=torch.float64, device=self.device)
+        self._check(self.lib.fslrc_edges(self.ctx, r1.data_ptr(), r2.data_ptr(), jac.data_ptr(), m, C.byref(n), C.c_void_p(stream)))
+        k = n.value
+        return EdgeList(r1[:k].cpu().numpy(), r2[:k].cpu().numpy(), jac[:k].cpu().numpy())
+
     # ---- compute entry points
-    def run_resident(self, dtab: DeviceTable, chrom_table, params: ClusterParams, order=_TABLE_ORDER):
-        """Inputs already in HBM; outputs stay in HBM (dtab.out_cluster / out_n_reads).  Returns stats dict.
+    def run_resident(self, dtab: DeviceTable, chrom_table, params: ClusterParams, order=_TABLE_ORDER, edges=False):
+        """Inputs already in HBM; outputs stay in HBM (dtab.out_cluster / out_n_reads).  Returns stats dict, or
+        (stats, EdgeList) with edges=True (the similarity graph of this call, which also stays in the context until the
+        next clustering call).
         order: the tie permutation of this call only (device int32 [n_fillings]; None = the GPU's stable sort); by default
         dtab.order."""
         p = self._params(chrom_table, params)
         t = self._table(dtab, order)
         st = _native.Stats()
         stream = torch.cuda.current_stream(self.device).cuda_stream
+        self._set_capture(edges)
         self._check(self.lib.fslrc_cluster_device(self.ctx, C.byref(t), C.byref(p), dtab.out_cluster.data_ptr(),
                                                   dtab.out_n_reads.data_ptr(), C.byref(st), C.c_void_p(stream)))
+        if edges:
+            return st.as_dict(self.lib), self.edge_list()
         return st.as_dict(self.lib)
 
     def filling_starts(self, dtab):
@@ -280,22 +318,25 @@ class Engine:
             return dtab._reference_order
         raise ValueError("tie_order must be None, 'stable' or 'reference', not %r" % (tie_order,))
 
-    def run_host(self, ptab: PinnedTable, chrom_table, params: ClusterParams):
-        """Host buffers in, host buffers out (H2D + D2H inside the call).  Returns stats dict."""
+    def run_host(self, ptab: PinnedTable, chrom_table, params: ClusterParams, edges=False):
+        """Host buffers in, host buffers out (H2D + D2H inside the call).  Returns stats dict.  edges: capture the
+        similarity graph (read it with edge_list())."""
         p = self._params(chrom_table, params)
         t = self._table(ptab)
         st = _native.Stats()
         stream = torch.cuda.current_stream(self.device).cuda_stream
+        self._set_capture(edges)
         self._check(self.lib.fslrc_cluster_host(self.ctx, C.byref(t), C.byref(p), ptab.out_cluster.data_ptr(),
                                                 ptab.out_n_reads.data_ptr(), C.byref(st), C.c_void_p(stream)))
         return st.as_dict(self.lib)
 
-    def cluster(self, table: ColumnarTable, params: ClusterParams, order=None) -> ClusterResult:
+    def cluster(self, table: ColumnarTable, params: ClusterParams, order=None, edges=False) -> ClusterResult:
+        """edges=True: ClusterResult.edges holds the similarity graph of this call."""
         ptab = PinnedTable(table, order)
-        stats = self.run_host(ptab, table, params)
+        stats = self.run_host(ptab, table, params, edges=edges)
         n = table.n_reads
         return ClusterResult(ptab.out_cluster[:n].numpy().copy(), ptab.out_n_reads[:n].numpy().copy(),
-                             bool(stats["no_clusters"]), stats)
+                             bool(stats["no_clusters"]), stats, self.edge_list() if edges else None)
 
     # ---- multi-GPU: pair space sharded over ranks, three exchange steps (SURVEY §8e)
     def run_sharded(self, dtab: DeviceTable, chrom_table, params: ClusterParams, rank, world, group=None):

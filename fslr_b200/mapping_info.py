@@ -237,15 +237,16 @@ class BamTable:
     def write_mappings_bed(self, path, fslr_version=None):
         self.mappings_bed_bytes(fslr_version).tofile(path)
 
-    def cluster(self, cluster_mask="subtelomere", tie_order=None, **options):
+    def cluster(self, cluster_mask="subtelomere", tie_order=None, edges=False, **options):
         """The clustering step (main.py:209-257,334-342) on the device-resident table.  tie_order as ParsedBed.cluster:
         None (`self.order` if set, else the GPU's stable sort), "stable", or "reference" (fslr's own tie order on this
-        host, computed once per table)."""
+        host, computed once per table).  edges=True: ClusterResult.edges holds the similarity graph."""
         params = ClusterParams.from_options(self, cluster_mask=cluster_mask, **options)
         self._live()
-        stats = self.engine.run_resident(self, self, params, order=self.engine.tie_order(self, tie_order))
+        out = self.engine.run_resident(self, self, params, order=self.engine.tie_order(self, tie_order), edges=edges)
+        stats, el = out if edges else (out, None)
         n = self.n_reads
-        return ClusterResult(self.out_cluster[:n].cpu().numpy(), self.out_n_reads[:n].cpu().numpy(), bool(stats["no_clusters"]), stats)
+        return ClusterResult(self.out_cluster[:n].cpu().numpy(), self.out_n_reads[:n].cpu().numpy(), bool(stats["no_clusters"]), stats, el)
 
     def close(self):
         if self.engine is not None:

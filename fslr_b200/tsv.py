@@ -72,19 +72,22 @@ class ParsedBed:
             self._names = np.array([buf[o:o + l].decode() for o, l in zip(off[:self.n_reads], ln[:self.n_reads])], dtype=object)
         return self._names
 
-    def cluster(self, cluster_mask="subtelomere", tie_order=None, **options):
+    def cluster(self, cluster_mask="subtelomere", tie_order=None, edges=False, **options):
         """The clustering step on the device-resident table.  Returns ClusterResult; the per-read result also stays on the
         device (out_cluster / out_n_reads) for write_cluster_bed.
         tie_order: how fillings with equal starts are ordered (cluster.py:114), which decides the cluster numbering.
         None: `self.order` when the caller set one, else the GPU's stable sort (ties keep bed order).  "stable": the GPU's
         stable sort.  "reference": the permutation fslr's own `sort_values('start')` gives on this host, so the ids equal
         fslr's: the start column is built on the device (fslrc_filling_starts), sorted on the host with the reference's
-        pandas call and sent back, once per table (kept for later calls); it applies to that call only."""
+        pandas call and sent back, once per table (kept for later calls); it applies to that call only.
+        edges=True: ClusterResult.edges holds the similarity graph (cluster.py:187-227's match_df rows, as read ids), and
+        edges_bytes() / write_edges() can render it until the next clustering call on this engine."""
         self._live()
         params = ClusterParams.from_options(self, cluster_mask=cluster_mask, **options)
-        stats = self.engine.run_resident(self, self, params, order=self.engine.tie_order(self, tie_order))
+        out = self.engine.run_resident(self, self, params, order=self.engine.tie_order(self, tie_order), edges=edges)
+        stats, el = out if edges else (out, None)
         n = self.n_reads
-        return ClusterResult(self.out_cluster[:n].cpu().numpy(), self.out_n_reads[:n].cpu().numpy(), bool(stats["no_clusters"]), stats)
+        return ClusterResult(self.out_cluster[:n].cpu().numpy(), self.out_n_reads[:n].cpu().numpy(), bool(stats["no_clusters"]), stats, el)
 
     def _render(self, entry):
         self._live()
@@ -115,6 +118,23 @@ class ParsedBed:
 
     def write_representative_bed(self, path):
         self.representative_bed_bytes().tofile(path)
+
+    def edges_bytes(self):
+        """The edge list of the last cluster(edges=True) call as match_df.to_csv(sep="\\t", index=False) writes it (header
+        `query1\\tquery2\\tjaccard_similarity`, one line per edge: both qnames and repr of the Jaccard similarity), rendered on
+        the device (fslrc_tsv_write_edges).  Raises FslrError when the last clustering call on this engine was not a
+        cluster(edges=True) of this table.  Like cluster_bed_bytes, a VIEW of the engine's reused pinned staging buffer."""
+        self._live()
+        fn, ctx = self.engine.lib.fslrc_tsv_write_edges, self.engine.ctx
+        stream = C.c_void_p(torch.cuda.current_stream(self.engine.device).cuda_stream)
+        n = C.c_int64()
+        self.engine._check(fn(ctx, None, 0, C.byref(n), stream))
+        out = self.engine.pinned_bytes(n.value)
+        self.engine._check(fn(ctx, out.data_ptr(), n.value, C.byref(n), stream))
+        return out[:n.value].numpy()
+
+    def write_edges(self, path):
+        self.edges_bytes().tofile(path)
 
     def close(self):
         if self.engine is not None:

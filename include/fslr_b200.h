@@ -250,6 +250,26 @@ void fslrc_bam_close(fslrc_ctx *ctx);
  * instead of spinning — for contexts driven concurrently from several host threads (one context per thread). */
 int fslrc_set_blocking_sync(fslrc_ctx *ctx, int on);
 
+/* ---- The similarity graph (cluster.py:187-227 returns it as match_df and the nx.Graph G) ----
+ * on != 0: every later fslrc_cluster_device / fslrc_cluster_host call also builds the list of the edges it handed to
+ * union-find (stats.edges of them) and keeps it in the context until the next clustering call, fslrc_destroy, or
+ * fslrc_set_edge_capture(ctx, 0), which frees it.  Off (the default), the clustering launches no extra kernel and allocates
+ * nothing.  The fslrc_mg_* sequence captures nothing (multi-GPU export is not implemented).
+ * Each edge is the directed pair (read1, read2) of read ids: read1 is the read whose query tested the pair (cluster.py:197's
+ * query_key, match_df's query1).  jaccard is cluster.py:140-170's intersection / union in that direction (list1 = read1's
+ * fillings), as the same IEEE double division.  The list is sorted by (query rank of read1, query rank of read2), query rank
+ * = the order in which cluster.py:197 visits the query reads, and does not depend on scheduling. */
+int fslrc_set_edge_capture(fslrc_ctx *ctx, int on);
+/* Copies the captured list into DEVICE buffers of at least `cap` elements (any of the three may be NULL; all NULL: only
+ * *n_edges is set).  FSLRC_ERR_ARG when the last clustering call ran without capture, failed, or was a fslrc_mg_* sequence,
+ * and when cap < *n_edges. */
+int fslrc_edges(fslrc_ctx *ctx, int32_t *read1, int32_t *read2, double *jaccard, int64_t cap, int64_t *n_edges, void *stream);
+/* Renders the captured list as match_df.to_csv(sep="\t", index=False) writes it: the header "query1\tquery2\tjaccard_similarity"
+ * and one line per edge, "<qname>\t<qname>\t<repr(jaccard)>", into a HOST buffer (out == NULL: size query), with the qnames of
+ * the parsed table.  FSLRC_ERR_ARG unless the list was captured by a clustering of the columns of the table that is open
+ * now (not before a later fslrc_tsv_open or fslrc_tsv_delete_false). */
+int fslrc_tsv_write_edges(fslrc_ctx *ctx, char *out, int64_t cap, int64_t *n_out, void *stream);
+
 /* Integer-issue microbenchmark used as the pair-kernel roofline denominator (SURVEY §8d): returns the measured
  * dependent-free IADD3/LOP3/VIMNMX lane-ops per second on this device. */
 int fslrc_int_peak(fslrc_ctx *ctx, double *lane_ops_per_s);
