@@ -14,6 +14,8 @@ The intermediate objects are opaque handles (the reference only ever passes them
 fused GPU call when `query_interval_trees` is reached.  `cluster_table` is the fused entry (SURVEY.md §8b).
 There is no CPU path: without the CUDA library or a device these functions raise.
 """
+import os
+
 import numpy as np
 import pandas as pd
 
@@ -51,45 +53,20 @@ def delete_false(bed_file):
 
 
 def get_chromosome_lengths(bam_path):
-    """cluster.py:173-175 without pysam (SURVEY §8f row 3): {reference name: length} from the BAM header.  A BAM file is a
-    series of BGZF blocks (gzip members with a `BC` extra field giving the block size); the header is `BAM\1`, l_text,
-    text, n_ref, then per reference l_name, name (NUL terminated), l_ref — all little-endian int32."""
-    import struct
-    import zlib
-    buf = bytearray()
-    need = 12
-
-    def fill(f, n):
-        """inflate BGZF blocks until `buf` holds n bytes"""
-        while len(buf) < n:
-            head = f.read(18)
-            if len(head) < 18:
-                raise ValueError("%s: truncated BAM header" % bam_path)
-            if head[:4] != b"\x1f\x8b\x08\x04" or head[12:14] != b"BC":
-                raise ValueError("%s: not a BGZF/BAM file" % bam_path)
-            xlen = struct.unpack("<H", head[10:12])[0]
-            bsize = struct.unpack("<H", head[16:18])[0]
-            f.read(xlen - 6)
-            data = f.read(bsize - xlen - 19)
-            f.read(8)                                                         # CRC32, ISIZE
-            buf.extend(zlib.decompress(data, -15))
-
+    """cluster.py:173-175 without pysam (SURVEY §8f row 3): {reference name: length} from the BAM header.  The file is
+    mapped, not read, and the BGZF reader of mapping_info inflates only the blocks the header spans, each checked against
+    its CRC32 and ISIZE as htslib checks it (ValueError on a mismatch, naming the block)."""
+    import mmap
+    from .mapping_info import bgzf_header_prefix
     with open(bam_path, "rb") as f:
-        fill(f, need)
-        if bytes(buf[:4]) != b"BAM\x01":
-            raise ValueError("%s: bad BAM magic" % bam_path)
-        l_text = struct.unpack_from("<i", buf, 4)[0]
-        fill(f, 12 + l_text)
-        n_ref = struct.unpack_from("<i", buf, 8 + l_text)[0]
-        pos, out = 12 + l_text, {}
-        for _ in range(n_ref):
-            fill(f, pos + 4)
-            l_name = struct.unpack_from("<i", buf, pos)[0]
-            fill(f, pos + 4 + l_name + 4)
-            name = bytes(buf[pos + 4: pos + 4 + l_name - 1]).decode()
-            out[name] = struct.unpack_from("<i", buf, pos + 4 + l_name)[0]
-            pos += 8 + l_name
-    return out
+        if os.fstat(f.fileno()).st_size == 0:
+            raise ValueError("%s: empty file, not a BAM file" % bam_path)
+        raw = mmap.mmap(f.fileno(), 0, access=mmap.ACCESS_READ)           # (closed when the last view of it goes)
+    try:
+        refs, _ = bgzf_header_prefix(raw)
+    except ValueError as e:
+        raise ValueError("%s: %s" % (bam_path, e)) from None
+    return dict(refs)
 
 
 def reference_order_of_starts(start):

@@ -138,6 +138,7 @@ static inline int nblk(int64_t n, int t) { return (int)((n + t - 1) / t); }
 #include "kernels_graph.cuh"
 #include "bam.cuh"
 #include "bam_chain.cuh"
+#include "crc32.cuh"
 
 // ================================================================ host pipeline
 struct Pipe {

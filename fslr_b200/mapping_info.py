@@ -26,12 +26,10 @@ OUT_COLUMNS = ["chrom", "rstart", "rend", "qname", "n_alignments", "aln_size", "
                "alignment_score", "short_anchor<50bp", "fslr_version", "inferred_by_primer", "seq"]   # collect_mapping_info.py:176-177
 
 
-def inflate_bgzf(path_or_bytes, threads=8):
-    """The uncompressed stream of a BGZF file as a uint8 array.  Block sizes come from the `BC` extra field and the ISIZE
-    trailer, so every block inflates independently into its final place."""
-    raw = path_or_bytes if isinstance(path_or_bytes, (bytes, bytearray, memoryview, np.ndarray)) else open(path_or_bytes, "rb").read()
-    mv = memoryview(raw)
-    blocks, p, total = [], 0, 0
+def _bgzf_blocks(mv):
+    """The blocks of the BGZF bytes `mv`, in file order, as (index, file offset, payload start, payload end, CRC32, ISIZE).
+    A block is a gzip member whose `BC` extra subfield gives its size; the trailer holds CRC32 and ISIZE."""
+    p, k = 0, 0
     while p < len(mv):
         if len(mv) - p < 18 or bytes(mv[p:p + 4]) != b"\x1f\x8b\x08\x04":
             raise ValueError("not a BGZF/BAM file (block header at byte %d)" % p)
@@ -42,22 +40,43 @@ def inflate_bgzf(path_or_bytes, threads=8):
             if si1 == 66 and si2 == 67 and slen == 2:
                 bsize = struct.unpack_from("<H", mv, q + 4)[0] + 1
             q += 4 + slen
-        if bsize is None or p + bsize > len(mv):
+        if bsize is None or bsize < 12 + xlen + 8 or p + bsize > len(mv):
             raise ValueError("truncated BGZF block at byte %d" % p)
-        isize = struct.unpack_from("<I", mv, p + bsize - 4)[0]
-        blocks.append((p + 12 + xlen, p + bsize - 8, total, isize))
-        total += isize
+        crc, isize = struct.unpack_from("<II", mv, p + bsize - 8)
+        yield k, p, p + 12 + xlen, p + bsize - 8, crc, isize
         p += bsize
-    out = np.empty(total, dtype=np.uint8)
+        k += 1
+
+
+def _inflate_block(mv, block):
+    """One block of _bgzf_blocks inflated and checked against its trailer, as htslib checks it: the length against ISIZE,
+    then the CRC-32 against CRC32.  A mismatch raises ValueError naming the block and its offset in the file."""
+    k, p, s, e, crc, isize = block
+    data = zlib.decompress(mv[s:e], -15)
+    if len(data) != isize:
+        raise ValueError("ISIZE mismatch in BGZF block %d (file offset %d): %d bytes inflated, ISIZE %d" % (k, p, len(data), isize))
+    if zlib.crc32(data) != crc:
+        raise ValueError("CRC32 mismatch in BGZF block %d (file offset %d)" % (k, p))
+    return data
+
+
+def inflate_bgzf(path_or_bytes, threads=8):
+    """The uncompressed stream of a BGZF file as a uint8 array.  Block sizes come from the `BC` extra field and the ISIZE
+    trailer, so every block inflates independently into its final place.  Every block is checked against its CRC32 and
+    ISIZE; a mismatch raises ValueError naming the first bad block."""
+    raw = path_or_bytes if isinstance(path_or_bytes, (bytes, bytearray, memoryview, np.ndarray)) else open(path_or_bytes, "rb").read()
+    mv = memoryview(raw)
+    blocks = list(_bgzf_blocks(mv))
+    start = np.cumsum([0] + [b[5] for b in blocks])
+    out = np.empty(int(start[-1]), dtype=np.uint8)
 
     def work(b):
-        s, e, o, n = b
-        if n:
-            out[o:o + n] = np.frombuffer(zlib.decompress(mv[s:e], -15), dtype=np.uint8)
+        o = int(start[b[0]])
+        out[o:o + b[5]] = np.frombuffer(_inflate_block(mv, b), dtype=np.uint8)
 
     if threads > 1 and len(blocks) > 4:
         with ThreadPoolExecutor(threads) as ex:
-            list(ex.map(work, blocks, chunksize=64))
+            list(ex.map(work, blocks, chunksize=64))                      # (results in block order: the first bad block raises)
     else:
         for b in blocks:
             work(b)
@@ -66,30 +85,18 @@ def inflate_bgzf(path_or_bytes, threads=8):
 
 def bgzf_header_prefix(raw, want=None):
     """Inflate BGZF blocks from the start of `raw` (file bytes) until the BAM header — magic, text, reference list — is
-    complete.  Returns (references, offset of the first alignment record in the inflated stream)."""
+    complete.  Returns (references, offset of the first alignment record in the inflated stream).  The blocks read are
+    checked against their CRC32 and ISIZE (ValueError on a mismatch)."""
     mv = memoryview(raw)
     buf = bytearray()
-    p = 0
-
-    def more():
-        nonlocal p
-        if len(mv) - p < 18 or bytes(mv[p:p + 4]) != b"\x1f\x8b\x08\x04":
-            raise ValueError("not a BGZF/BAM file (block header at byte %d)" % p)
-        xlen = struct.unpack_from("<H", mv, p + 10)[0]
-        q, bsize = p + 12, None
-        while q < p + 12 + xlen:
-            slen = struct.unpack_from("<H", mv, q + 2)[0]
-            if mv[q] == 66 and mv[q + 1] == 67 and slen == 2:
-                bsize = struct.unpack_from("<H", mv, q + 4)[0] + 1
-            q += 4 + slen
-        if bsize is None or p + bsize > len(mv):
-            raise ValueError("truncated BGZF block at byte %d" % p)
-        buf.extend(zlib.decompress(mv[p + 12 + xlen:p + bsize - 8], -15))
-        p += bsize
+    blocks = _bgzf_blocks(mv)
 
     def need(n):
         while len(buf) < n:
-            more()
+            b = next(blocks, None)
+            if b is None:
+                raise ValueError("truncated BAM header")
+            buf.extend(_inflate_block(mv, b))
 
     need(12)
     if bytes(buf[:4]) != b"BAM\x01":

@@ -233,7 +233,10 @@ int fslrc_bam_open(fslrc_ctx *ctx, const uint8_t *bam, int64_t n_bytes, int64_t 
 /* The same from the COMPRESSED file bytes: BGZF blocks are inflated on the device (one warp per block) and the record
  * boundaries are found there as well, so only the compressed bytes cross PCIe.  first_record / n_ref come from the caller's
  * parse of the BAM header (the first blocks).  info->reserved is 1 when the device's record-boundary guess failed its chain
- * check and the host walk ran instead (same result).  CRC32 trailers are not verified; ISIZE is. */
+ * check and the host walk ran instead (same result).  Every block is checked as htslib checks it: its inflated length
+ * against ISIZE (a mismatch is reported as corrupt DEFLATE data), then the CRC-32 of its inflated bytes against the CRC32
+ * field of its trailer (on the device, one warp per block).  A CRC mismatch returns FSLRC_ERR_ARG with a message naming the
+ * first bad block and its offset in the file; a DEFLATE error is reported before it.  The context stays usable. */
 int fslrc_bam_open_bgzf(fslrc_ctx *ctx, const uint8_t *file, int64_t n_bytes, int64_t first_record, int32_t n_ref,
                         const char *primer_names, const int32_t *primer_seq_len, int32_t n_primers,
                         const int32_t *region_chrom, const int32_t *region_start, const int32_t *region_end, int32_t n_regions,
