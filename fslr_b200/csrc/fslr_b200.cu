@@ -63,6 +63,7 @@ struct fslrc_ctx {
     int edge_capture;        // fslrc_set_edge_capture
     struct EdgeList *edges;  // edge list of the last clustering call (capture on), kept until the next one
     long long tsv_gen;       // bumped by fslrc_tsv_open / fslrc_tsv_delete_false: which parsed table a captured list names
+    unsigned char *prim; size_t prim_bytes;   // scratch of the device-wide primitives: one of `allocs`, so free_all drops it
 };
 // the similarity graph of one clustering call, sorted by (query rank of read1, query rank of read2); device arrays
 struct EdgeList {
@@ -115,12 +116,51 @@ static void free_all(fslrc_ctx *ctx) {
     if (ctx->late_pending) { cudaStreamWaitEvent(ctx->stream, ctx->ev_c2, 0); ctx->late_pending = false; }   // (an error path got here first)
     for (void *p : ctx->allocs) cudaFreeAsync(p, ctx->stream);
     ctx->allocs.clear();
+    ctx->prim = nullptr; ctx->prim_bytes = 0;
 }
 #define DA(ptr, n)                                  \
     do {                                            \
         int r__ = dalloc(ctx, &(ptr), (int64_t)(n)); \
         if (r__) return r__;                        \
     } while (0)
+
+// the device arrays of a table kept on the device between calls (TsvState, BamState)
+struct Resident {
+    std::vector<void *> allocs;
+};
+template <typename T>
+static int res_alloc(fslrc_ctx *ctx, Resident &m, T **p, int64_t n) {
+    void *q = nullptr;
+    CK(cudaMallocAsync(&q, (size_t)(n > 0 ? n : 1) * sizeof(T), ctx->stream));
+    m.allocs.push_back(q);
+    *p = (T *)q;
+    return 0;
+}
+#define RA(m, ptr, n) do { int r__ = res_alloc(ctx, (m), &(ptr), (int64_t)(n)); if (r__) return r__; } while (0)
+static void res_free(fslrc_ctx *ctx, Resident &m, void *p) {           // one array, stream-ordered
+    std::vector<void *>::iterator it = std::find(m.allocs.begin(), m.allocs.end(), p);
+    if (it != m.allocs.end()) { m.allocs.erase(it); cudaFreeAsync(p, ctx->stream); }
+}
+// the context's table *s (ctx->tsv, ctx->bam) and all its arrays
+template <typename S>
+static void drop_table(fslrc_ctx *ctx, S *&s) {
+    if (!s) return;
+    for (void *p : s->mem.allocs) cudaFreeAsync(p, ctx->stream);
+    cudaStreamSynchronize(ctx->stream);
+    delete s; s = nullptr;
+}
+// The cleanup of the calls on a resident table: a failing call frees its scratch and, when it is an open (drop: tsv_free,
+// bam_free), the table it was building, so that the context never holds a half-built one.
+template <typename F>
+static int table_call(fslrc_ctx *ctx, void (*drop)(fslrc_ctx *), F &&body) {
+    const int r = body();
+    if (r) {
+        free_all(ctx);
+        if (drop) drop(ctx);
+        cudaStreamSynchronize(ctx->stream);
+    }
+    return r;
+}
 
 // every launch of one of OUR kernels goes through KL so that the count can be reported (bench.py "gpu_launches")
 #define KL(kernel, grid, block, ...)                         \
@@ -165,8 +205,7 @@ struct Pipe {
     unsigned long long cap_entries, cap_pedges, cap_pl;
     int *parent, *ing;
     unsigned *ticket;
-    unsigned char *prim; size_t prim_bytes;   // scratch of the device-wide primitives
-    int stage;               // next event index
+    int stage;              // next event index
     Tab tab;
     UmaxTab um;
 };
@@ -188,39 +227,48 @@ static int n_sms(fslrc_ctx *ctx) {
     return n;
 }
 // ---- device-wide primitives (prims.cuh): look-back status words + ticket live in one reusable scratch region
-static int prim_scratch(fslrc_ctx *ctx, Pipe *P, size_t status_bytes) {
+static int prim_scratch(fslrc_ctx *ctx, size_t status_bytes) {
     const size_t need = status_bytes + 256;
-    if (need > P->prim_bytes) {
+    if (need > ctx->prim_bytes) {
         void *q; const size_t nb = need + (need >> 1);
         CK(cudaMallocAsync(&q, nb, ctx->stream));
         ctx->allocs.push_back(q);
-        P->prim = (unsigned char *)q; P->prim_bytes = nb;
+        ctx->prim = (unsigned char *)q; ctx->prim_bytes = nb;
     }
-    CK(cudaMemsetAsync(P->prim, 0, need, ctx->stream));          // ticket (first 256 bytes) + status words
+    CK(cudaMemsetAsync(ctx->prim, 0, need, ctx->stream));        // ticket (first 256 bytes) + status words
     return 0;
 }
 // exclusive sum of int32; *total (device, optional) receives the grand total
-static int xscan(fslrc_ctx *ctx, Pipe *P, const int *in, int *out, int n, int64_t *total = nullptr) {
+static int xscan(fslrc_ctx *ctx, const int *in, int *out, int n, int64_t *total = nullptr) {
     cudaStream_t st = ctx->stream;
     if (n <= 0) { if (total) CK(cudaMemsetAsync(total, 0, sizeof(int64_t), st)); return 0; }
     const int tiles = nblk(n, prims::SC_TILE);
-    int r = prim_scratch(ctx, P, sizeof(unsigned long long) * tiles); if (r) return r;
-    KL(prims::k_scan_excl<int>, tiles, prims::SC_THREADS, in, out, n, (unsigned long long *)(P->prim + 256), (unsigned *)P->prim, (long long *)total);
+    int r = prim_scratch(ctx, sizeof(unsigned long long) * tiles); if (r) return r;
+    KL(prims::k_scan_excl<int>, tiles, prims::SC_THREADS, in, out, n, (unsigned long long *)(ctx->prim + 256), (unsigned *)ctx->prim, (long long *)total);
+    return 0;
+}
+// exclusive sum of int64 (k_reads_fast's packed (count << 32 | L) flags, the line lengths of a text render)
+static int xscan64(fslrc_ctx *ctx, const long long *in, long long *out, int n, int64_t *total) {
+    cudaStream_t st = ctx->stream;
+    if (n <= 0) { if (total) CK(cudaMemsetAsync(total, 0, sizeof(int64_t), st)); return 0; }
+    const int tiles = nblk(n, prims::SC_TILE);
+    int r = prim_scratch(ctx, sizeof(unsigned long long) * tiles); if (r) return r;
+    KL(prims::k_scan_excl<long long>, tiles, prims::SC_THREADS, in, out, n, (unsigned long long *)(ctx->prim + 256), (unsigned *)ctx->prim, (long long *)total);
     return 0;
 }
 // per-segment inclusive prefix max (seg non-decreasing)
-static int segmax_scan(fslrc_ctx *ctx, Pipe *P, const int *seg, const int *val, int *out, int n) {
+static int segmax_scan(fslrc_ctx *ctx, const int *seg, const int *val, int *out, int n) {
     cudaStream_t st = ctx->stream;
     if (n <= 0) return 0;
     const int tiles = nblk(n, prims::SC_TILE);
-    int r = prim_scratch(ctx, P, sizeof(unsigned long long) * tiles); if (r) return r;
-    KL(prims::k_scan_segmax, tiles, prims::SC_THREADS, seg, val, out, n, (unsigned long long *)(P->prim + 256), (unsigned *)P->prim);
+    int r = prim_scratch(ctx, sizeof(unsigned long long) * tiles); if (r) return r;
+    KL(prims::k_scan_segmax, tiles, prims::SC_THREADS, seg, val, out, n, (unsigned long long *)(ctx->prim + 256), (unsigned *)ctx->prim);
     return 0;
 }
 // stable LSD radix sort of (key, value) pairs on key bits [b0, b1); the inputs are left untouched.  The last pass hands
 // every pair to `last` with its output position; *last_start (optional) receives the start of every digit of that pass.
 template <typename Out>
-static int sort_pairs_to(fslrc_ctx *ctx, Pipe *P, const unsigned *kin, const int *vin, int n, int b0, int b1, Out last,
+static int sort_pairs_to(fslrc_ctx *ctx, const unsigned *kin, const int *vin, int n, int b0, int b1, Out last,
                          const unsigned **last_start = nullptr) {
     cudaStream_t st = ctx->stream;
     if (n <= 0) return 0;
@@ -235,25 +283,25 @@ static int sort_pairs_to(fslrc_ctx *ctx, Pipe *P, const unsigned *kin, const int
     const int tiles = nblk(n, prims::RS_TILE);
     const unsigned *ks = kin; const int *vs = vin;
     for (int p = 0; p < npass; p++) {
-        int r = prim_scratch(ctx, P, sizeof(unsigned) * 256 * (size_t)tiles); if (r) return r;
+        int r = prim_scratch(ctx, sizeof(unsigned) * 256 * (size_t)tiles); if (r) return r;
         const int nbits = std::min(8, b1 - b0 - 8 * p);
         const unsigned *gb = hist + 256 * p;
         ctx->launches++;
         if (p == npass - 1) {
             prims::k_rs_onesweep<<<tiles, prims::RS_THREADS, sizeof(prims::RsSmem), st>>>(ks, vs, last, n, b0 + 8 * p, (1 << nbits) - 1, gb,
-                                                                                          (unsigned *)(P->prim + 256), (unsigned *)P->prim);
+                                                                                          (unsigned *)(ctx->prim + 256), (unsigned *)ctx->prim);
         } else {
             const prims::PairOut o = tmp[p & 1];
             prims::k_rs_onesweep<<<tiles, prims::RS_THREADS, sizeof(prims::RsSmem), st>>>(ks, vs, o, n, b0 + 8 * p, (1 << nbits) - 1, gb,
-                                                                                          (unsigned *)(P->prim + 256), (unsigned *)P->prim);
+                                                                                          (unsigned *)(ctx->prim + 256), (unsigned *)ctx->prim);
             ks = o.kout; vs = o.vout;
         }
     }
     if (last_start) *last_start = hist + 256 * (npass - 1);
     return 0;
 }
-static int sort_pairs(fslrc_ctx *ctx, Pipe *P, const unsigned *kin, unsigned *kout, const int *vin, int *vout, int n, int b0, int b1) {
-    return sort_pairs_to(ctx, P, kin, vin, n, b0, b1, prims::PairOut{kout, vout});
+static int sort_pairs(fslrc_ctx *ctx, const unsigned *kin, unsigned *kout, const int *vin, int *vout, int n, int b0, int b1) {
+    return sort_pairs_to(ctx, kin, vin, n, b0, b1, prims::PairOut{kout, vout});
 }
 // wait for the context's stream: spinning (lowest latency) or, for contexts driven from several host threads at once
 // (engine.HostPipeline), sleeping on a blocking-sync event so that a waiting thread leaves its core to the others
@@ -282,15 +330,6 @@ static int bits_for(int64_t n) { int b = 1; while ((1ll << b) < n && b < 32) b++
 static int alloc_records(fslrc_ctx *ctx, Pipe *P, int **s_m, int **s_end);
 static int pipe_bands(fslrc_ctx *ctx, Pipe *P, const int *s_m, const int *s_end);
 
-// exclusive sum of int64 (k_reads_fast's packed (count << 32 | L) flags)
-static int xscan64(fslrc_ctx *ctx, Pipe *P, const long long *in, long long *out, int n, int64_t *total) {
-    cudaStream_t st = ctx->stream;
-    if (n <= 0) { if (total) CK(cudaMemsetAsync(total, 0, sizeof(int64_t), st)); return 0; }
-    const int tiles = nblk(n, prims::SC_TILE);
-    int r = prim_scratch(ctx, P, sizeof(unsigned long long) * tiles); if (r) return r;
-    KL(prims::k_scan_excl<long long>, tiles, prims::SC_THREADS, in, out, n, (unsigned long long *)(P->prim + 256), (unsigned *)P->prim, (long long *)total);
-    return 0;
-}
 // IntervalMap order from data order (stage 4): one stable partition by chromosome + local tie fix, or — long runs of equal
 // (chrom, start) — three stable sorts
 static int pipe_chrom_order(fslrc_ctx *ctx, Pipe *P, const int4 *IT0, unsigned *tkey, unsigned *tval, bool tie_ok, int *s_dp) {
@@ -299,7 +338,7 @@ static int pipe_chrom_order(fslrc_ctx *ctx, Pipe *P, const int4 *IT0, unsigned *
     if (D <= 0) return 0;
     if (tie_ok) {
         unsigned *tkey2, *tval2; DA(tkey2, D); DA(tval2, D);
-        int r = sort_pairs(ctx, P, tkey, tkey2, (const int *)tval, (int *)tval2, D, 0, bits_for(P->pr.n_chrom)); if (r) return r;
+        int r = sort_pairs(ctx, tkey, tkey2, (const int *)tval, (int *)tval2, D, 0, bits_for(P->pr.n_chrom)); if (r) return r;
         KL(k_apply_delta, nblk(D, TB), TB, D, tval2, s_dp);
     } else {
         // (chrom, start, end desc, data order) as three stable sorts from data order: ~end, start, chrom
@@ -307,11 +346,11 @@ static int pipe_chrom_order(fslrc_ctx *ctx, Pipe *P, const int4 *IT0, unsigned *
         DA(ek, D); DA(ek2, D); DA(v1, D); DA(v2, D); DA(iotaD, D);
         KL(k_iota, nblk(D, TB), TB, iotaD, D);
         KL(k_end_keys, nblk(D, TB), TB, D, IT0, ek);
-        int r = sort_pairs(ctx, P, ek, ek2, iotaD, v1, D, 0, 32); if (r) return r;
+        int r = sort_pairs(ctx, ek, ek2, iotaD, v1, D, 0, 32); if (r) return r;
         KL(k_gather_key, nblk(D, TB), TB, D, v1, IT0, 0, ek);
-        r = sort_pairs(ctx, P, ek, ek2, v1, v2, D, 0, 32); if (r) return r;
+        r = sort_pairs(ctx, ek, ek2, v1, v2, D, 0, 32); if (r) return r;
         KL(k_gather_key, nblk(D, TB), TB, D, v2, IT0, 1, ek);
-        r = sort_pairs(ctx, P, ek, ek2, v2, s_dp, D, 0, bits_for(P->pr.n_chrom)); if (r) return r;
+        r = sort_pairs(ctx, ek, ek2, v2, s_dp, D, 0, bits_for(P->pr.n_chrom)); if (r) return r;
     }
     return 0;
 }
@@ -339,7 +378,7 @@ static int pipe_ingest_fast(fslrc_ctx *ctx, Pipe *P, const long long *d_clen, co
     if (A > 0) {
         KL(k_rows_fast, nblk(A, TB), TB, A, R, tb.read_id, tb.chrom, tb.rstart, tb.rend, tb.qstart, tb.qend, pr.n_chrom, d_clen, d_cmask,
            pr.mask_subtelomere, (long long)pr.subtel, flagA, qlen2, (unsigned long long *)(P->cnt + 0), P->err);
-        int r = xscan(ctx, P, flagA, posA, A, P->cnt + 1); if (r) return r;
+        int r = xscan(ctx, flagA, posA, A, P->cnt + 1); if (r) return r;
     }
     { int r = read_counts(ctx, P); if (r) return r; }
     if (ctx->h_pin[NCNT] & EF_NONMONO) {                                    // rows of a read apart, or ids going down: general path
@@ -365,7 +404,7 @@ static int pipe_ingest_fast(fslrc_ctx *ctx, Pipe *P, const long long *d_clen, co
         long long mx = 0; bool known = pr.n_chrom > 0;
         for (int c = 0; c < pr.n_chrom; c++) { if (pr.chrom_len[c] <= 0) known = false; mx = std::max<long long>(mx, pr.chrom_len[c]); }
         kbits = (known && mx < 0x7fffffffLL) ? std::min(32, bits_for(mx + 2)) : 32;
-        int r = sort_pairs(ctx, P, key, key2, val, dfill, D, 0, kbits); if (r) return r;
+        int r = sort_pairs(ctx, key, key2, val, dfill, D, 0, kbits); if (r) return r;
         KL(k_items_fast, nblk(D, TB), TB, D, dfill, REC, IT0, IT1, flag64);
         DA(tkey, D); DA(tval, D);
         KL(k_tie_delta, nblk(D, TB), TB, D, IT0, tkey, tval, (unsigned long long *)(P->cnt + 41), P->err);
@@ -374,7 +413,7 @@ static int pipe_ingest_fast(fslrc_ctx *ctx, Pipe *P, const long long *d_clen, co
     // ---- query rank + read-major offsets from one scan over data order
     DA(P->RI, std::min(R, D));
     if (D > 0) {
-        int r = xscan64(ctx, P, flag64, qo64, D, P->cnt + 2); if (r) return r;
+        int r = xscan64(ctx, flag64, qo64, D, P->cnt + 2); if (r) return r;
         KL(k_firsts_fast, nblk(D, TB), TB, D, flag64, qo64, IT0, IT1, qlen2, pr.qlen_c, pr.naln_c, QO, P->RI, P->err);
     }
     if (R > 0) KL(k_q_of_rid, nblk(R, TB), TB, R, QO, P->q_of_rid);
@@ -395,7 +434,7 @@ static int pipe_ingest_fast(fslrc_ctx *ctx, Pipe *P, const long long *d_clen, co
     if (D > 0 && ctx->h_pin[41] == 0) {                                      // partition by chromosome, moving the records
         const int cbits = bits_for(pr.n_chrom);
         const unsigned *cstart = nullptr;
-        int r = sort_pairs_to(ctx, P, tkey, (const int *)tval, D, 0, cbits, ChromRecOut{rec}, &cstart); if (r) return r;
+        int r = sort_pairs_to(ctx, tkey, (const int *)tval, D, 0, cbits, ChromRecOut{rec}, &cstart); if (r) return r;
         if (cbits <= 8) KL(k_chrom_bounds_digits, 1, 256, pr.n_chrom, D, cstart, P->chrom_lo, P->chrom_hi);
         else KL(k_chrom_bounds, nblk(D, TB), TB, D, P->s_chrom, P->chrom_lo, P->chrom_hi);
     } else if (D > 0) {                                                      // long runs of equal (chrom, start): three full sorts
@@ -429,7 +468,7 @@ static int keep_rows(fslrc_ctx *ctx, Pipe *P, const int *rid, const int *qstart,
     if (A > 0) {
         KL(k_first_last, nblk(A, TB), TB, A, R, rid, first, last, P->err);
         KL(k_keep, nblk(A, TB), TB, A, R, rid, first, last, qstart, qend, flagA, qmin, qmax);
-        return xscan(ctx, P, flagA, posA, A, P->cnt + 0);
+        return xscan(ctx, flagA, posA, A, P->cnt + 0);
     }
     return 0;
 }
@@ -473,7 +512,7 @@ static int pipe_prepare(fslrc_ctx *ctx, Pipe *P) {
     DA(flagF, F); DA(posF, F);
     if (F > 0) {
         KL(k_mask_flags, nblk(F, TB), TB, F, tb.order, FR0, pr.n_chrom, d_clen, d_cmask, pr.mask_subtelomere, (long long)pr.subtel, flagF, P->err);
-        int r = xscan(ctx, P, flagF, posF, F, P->cnt + 1); if (r) return r;
+        int r = xscan(ctx, flagF, posF, F, P->cnt + 1); if (r) return r;
     }
     { int r = read_counts(ctx, P); if (r) return r; r = err_code(ctx); if (r) return r; }
     const int D = P->D = (int)ctx->h_pin[1];
@@ -483,7 +522,7 @@ static int pipe_prepare(fslrc_ctx *ctx, Pipe *P) {
     } else {
         int *key, *key2, *v; DA(key, D); DA(key2, D); DA(v, D);
         if (F > 0) KL(k_compact_fillings, nblk(F, TB), TB, F, (const int *)nullptr, flagF, posF, FR0, key, v);
-        int r = sort_pairs(ctx, P, (const unsigned *)key, (unsigned *)key2, v, dfill, D, 0, 32); if (r) return r;
+        int r = sort_pairs(ctx, (const unsigned *)key, (unsigned *)key2, v, dfill, D, 0, 32); if (r) return r;
     }
     int4 *IT0; int2 *IT1; int *firstdp;
     DA(IT0, D); DA(IT1, D); DA(firstdp, R);
@@ -500,7 +539,7 @@ static int pipe_prepare(fslrc_ctx *ctx, Pipe *P) {
     DA(flagD, D); DA(posD, D); DA(it_q, D);
     if (D > 0) {
         KL(k_is_first, nblk(D, TB), TB, D, IT0, firstdp, flagD);
-        int r = xscan(ctx, P, flagD, posD, D, P->cnt + 2); if (r) return r;
+        int r = xscan(ctx, flagD, posD, D, P->cnt + 2); if (r) return r;
     }
     { int r = read_counts(ctx, P); if (r) return r; r = err_code(ctx); if (r) return r; }
     const int Q = P->Q = (int)ctx->h_pin[2];
@@ -512,7 +551,7 @@ static int pipe_prepare(fslrc_ctx *ctx, Pipe *P) {
     if (D > 0) {
         KL(k_item_q, nblk(D, TB), TB, D, IT0, P->q_of_rid, it_q);
         KL(k_iota, nblk(D, TB), TB, iotaD, D);
-        int r = sort_pairs(ctx, P, (const unsigned *)it_q, (unsigned *)qs, iotaD, rm_dp, D, 0, bits_for(Q)); if (r) return r;
+        int r = sort_pairs(ctx, (const unsigned *)it_q, (unsigned *)qs, iotaD, rm_dp, D, 0, bits_for(Q)); if (r) return r;
         KL(k_read_bounds, nblk(D, TB), TB, D, qs, rm_dp, rmidx, off, len_end);
         KL(k_read_info, nblk(Q, TB), TB, Q, P->rid_of_q, off, len_end, rm_dp, IT1, qmin, qmax, pr.qlen_c, pr.naln_c, P->RI, P->err);
     }
@@ -545,7 +584,7 @@ static int pipe_bands(fslrc_ctx *ctx, Pipe *P, const int *s_m, const int *s_end)
     const int D = P->D, Q = P->Q;
     DA(P->RM, 2 * (int64_t)D); DA(P->pmaxS, D); DA(P->rclass, Q);
     if (D > 0) {
-        int r = segmax_scan(ctx, P, P->s_chrom, s_end, P->pmaxS, D); if (r) return r;
+        int r = segmax_scan(ctx, P->s_chrom, s_end, P->pmaxS, D); if (r) return r;
         CK(cudaMemsetAsync(P->rclass, 0, sizeof(int) * (size_t)std::max(Q, 1), st));
         KL(k_bands, nblk(D, 256), 256, D, P->SR0, s_m, P->s_chrom, P->pmaxS, P->chrom_lo, P->chrom_hi, P->RM, P->rclass,
            (unsigned long long *)(P->cnt + 3), (unsigned long long *)(P->cnt + 14), (unsigned long long *)(P->cnt + 44));
@@ -608,7 +647,7 @@ static int pipe_sat(fslrc_ctx *ctx, Pipe *P) {
     const int Q = P->Q, TB = 256;
     if (Q > 0 && P->pr.overlap > 0.0) {
         KL(k_light_sat, nblk(Q, TB), TB, P->tab, P->rclass, P->cp, P->isP, P->plinfo, P->plcount, (unsigned long long *)(P->cnt + 40));
-        int r = xscan(ctx, P, P->plcount, P->ploff, Q, P->cnt + 45); if (r) return r;
+        int r = xscan(ctx, P->plcount, P->ploff, Q, P->cnt + 45); if (r) return r;
         KL(k_plinfo, nblk(Q, TB), TB, Q, P->plcount, P->ploff, P->plinfo, (unsigned long long *)(P->cnt + 40), P->cnt + 45, P->cap_pl, P->err);
     }
     return 0;
@@ -629,7 +668,7 @@ static int pipe_replay_union(fslrc_ctx *ctx, Pipe *P, int shard, int nshard, con
                 P->cap_entries, P->plinfo, P->isP, P->cp, P->PL, P->err);
     }
     if (Q > 0) {
-        int r = xscan(ctx, P, P->isP, posQ, Q, P->cnt + 6); if (r) return r;
+        int r = xscan(ctx, P->isP, posQ, Q, P->cnt + 6); if (r) return r;
     }
     { int r = read_counts(ctx, P); if (r) return r; r = err_code(ctx); if (r) return r; }
     const int nP = P->nP = (int)ctx->h_pin[6];
@@ -653,10 +692,10 @@ static int pipe_replay_union(fslrc_ctx *ctx, Pipe *P, int shard, int nshard, con
         int4 *RH = nullptr;
         if (!walk) DA(RH, 3 * (int64_t)nP);
         KL(k_run_flags, nblk(nP, TB), TB, nP, P->plist, P->RI, P->RM, sflag, P->stop, P->stopS, P->plinfo, P->tab.chrom_lo, RH);
-        int r = xscan(ctx, P, sflag, spos, nP, P->cnt + 15); if (r) return r;
+        int r = xscan(ctx, sflag, spos, nP, P->cnt + 15); if (r) return r;
         KL(k_compact_flagged, nblk(nP, TB), TB, nP, sflag, spos, sstart);
         KL(k_run_cut, nblk(nP, TB), TB, nP, sflag, spos, sstart, P->cnt + 15, rflag);
-        r = xscan(ctx, P, rflag, rpos, nP, P->cnt + 12); if (r) return r;
+        r = xscan(ctx, rflag, rpos, nP, P->cnt + 12); if (r) return r;
         KL(k_compact_flagged, nblk(nP, TB), TB, nP, rflag, rpos, rstart);
         r = read_counts(ctx, P); if (r) return r;
         const int nRuns = (int)ctx->h_pin[12];
@@ -703,11 +742,11 @@ static int pipe_number(fslrc_ctx *ctx, Pipe *P, int *out_cluster, int *out_n) {
     if (Q > 0) {
         CK(cudaMemsetAsync(csize, 0, sizeof(int) * Q, st));
         KL(k_flatten, nblk(Q, TB), TB, Q, P->parent, P->ing, isroot, csize);
-        int r = xscan(ctx, P, isroot, cidx, Q, P->cnt + 9); if (r) return r;
+        int r = xscan(ctx, isroot, cidx, Q, P->cnt + 9); if (r) return r;
     }
     if (R > 0) {
         KL(k_single_flags, nblk(R, TB), TB, R, P->q_of_rid, P->ing, sflag);
-        int r = xscan(ctx, P, sflag, spos, R, P->cnt + 11); if (r) return r;
+        int r = xscan(ctx, sflag, spos, R, P->cnt + 11); if (r) return r;
         KL(k_number, nblk(R, TB), TB, R, P->q_of_rid, P->ing, P->parent, cidx, csize, spos, P->cnt + 9, out_cluster, out_n);
     }
     return mark(ctx, ST_NUMBER);
@@ -744,9 +783,9 @@ static int export_edges(fslrc_ctx *ctx, Pipe *P, const int32_t *read_id_col) {
     if (n > 0) {
         const int qb = bits_for(Q);
         KL(k_edges_key2, nblk(n, TB), TB, n, dir, key, iota);
-        int r = sort_pairs(ctx, P, key, key2, iota, perm1, n, 0, qb); if (r) return r;
+        int r = sort_pairs(ctx, key, key2, iota, perm1, n, 0, qb); if (r) return r;
         KL(k_edges_key1, nblk(n, TB), TB, n, dir, perm1, key);
-        r = sort_pairs(ctx, P, key, key2, perm1, perm, n, 0, qb); if (r) return r;
+        r = sort_pairs(ctx, key, key2, perm1, perm, n, 0, qb); if (r) return r;
         if (!(P->pr.overlap > 0.0)) KL(k_edges_final<true>, nblk(n, TB), TB, n, P->tab, dir, perm, rid_of_q, L->read1, L->read2, L->jac);
         else KL(k_edges_final<false>, nblk(n, TB), TB, n, P->tab, dir, perm, rid_of_q, L->read1, L->read2, L->jac);
     }
@@ -822,7 +861,7 @@ static int resolve_columns(fslrc_ctx *ctx, Pipe *P, const fslrc_table *in, bool 
         BRING(in->rows_per_read_u8, (size_t)R, d_r8);
         DA(cnt32, R); DA(first, R); DA(rid, A);
         KL(k_widen_u8, nblk(R, 256), 256, R, d_r8, cnt32);
-        int r = xscan(ctx, P, cnt32, first, (int)R); if (r) return r;
+        int r = xscan(ctx, cnt32, first, (int)R); if (r) return r;
         KL(k_rid_from_runs, nblk(R, 256), 256, (int)R, (int)A, first, cnt32, rid);
         out->read_id = rid;
     }
@@ -923,6 +962,7 @@ int fslrc_create(int device, fslrc_ctx **out) {
     ctx->blocking = 0;
     ctx->copy_stream = nullptr; ctx->late_pending = false;
     ctx->edge_capture = 0; ctx->edges = nullptr; ctx->tsv_gen = 0;
+    ctx->prim = nullptr; ctx->prim_bytes = 0;
     if (cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking) != cudaSuccess) { ctx->copy_stream = nullptr; cudaGetLastError(); }
     cudaEventCreateWithFlags(&ctx->ev_c1, cudaEventDisableTiming);
     cudaEventCreateWithFlags(&ctx->ev_c2, cudaEventDisableTiming);
@@ -1166,7 +1206,7 @@ int fslrc_choose_alignment_host(fslrc_ctx *ctx, int64_t n_rows, int64_t n_reads,
 // ---------------------------------------------------------------- mappings.bed ingest / egress on the GPU (tsv.cuh)
 }  // extern "C"
 struct TsvState {
-    std::vector<void *> allocs;
+    Resident mem;            // every device array below (until fslrc_tsv_close or the next fslrc_tsv_open)
     unsigned char *text; long long n; long long *line_start;
     int n_lines, n_rows, n_reads, n_chrom;
     int *read_id, *chrom, *rstart, *rend, *aln, *qstart, *qend, *naln, *score, *first_row;
@@ -1174,24 +1214,10 @@ struct TsvState {
     long long *line_end;     // nullptr: line l ends at line_start[l + 1] - 1; set once fslrc_tsv_delete_false removed rows
     std::vector<std::string> chrom_names;
 };
-template <typename T>
-static int palloc(fslrc_ctx *ctx, T **p, int64_t n) {                  // persistent (until fslrc_tsv_close)
-    void *q = nullptr;
-    CK(cudaMallocAsync(&q, (size_t)(n > 0 ? n : 1) * sizeof(T), ctx->stream));
-    ctx->tsv->allocs.push_back(q);
-    *p = (T *)q;
-    return 0;
-}
-#define PA(ptr, n) do { int r__ = palloc(ctx, &(ptr), (int64_t)(n)); if (r__) return r__; } while (0)
 static const int32_t *tsv_read_id(const fslrc_ctx *ctx) { return ctx->tsv ? ctx->tsv->read_id : nullptr; }
-static void tsv_free(fslrc_ctx *ctx) {
-    if (!ctx->tsv) return;
-    for (void *p : ctx->tsv->allocs) cudaFreeAsync(p, ctx->stream);
-    cudaStreamSynchronize(ctx->stream);
-    delete ctx->tsv; ctx->tsv = nullptr;
-}
+static void tsv_free(fslrc_ctx *ctx) { drop_table(ctx, ctx->tsv); }
 // strings -> dense ids in order of first appearance (pandas.factorize); *n_ids receives the number of distinct strings
-static int tsv_intern(fslrc_ctx *ctx, Pipe *P, const unsigned char *text, int n, const long long *off, const int *len,
+static int tsv_intern(fslrc_ctx *ctx, const unsigned char *text, int n, const long long *off, const int *len,
                       const unsigned long long *hash, int *id_out, int *first_row_of_id /*nullable, capacity n*/, int *err,
                       int64_t *n_ids_dev) {
     cudaStream_t st = ctx->stream;
@@ -1203,13 +1229,11 @@ static int tsv_intern(fslrc_ctx *ctx, Pipe *P, const unsigned char *text, int n,
     KL(k_fill<int>, nblk(cap, TB), TB, first, (int64_t)cap, 0x7fffffff);
     KL(tsv::k_tsv_intern_insert, nblk(n, TB), TB, n, hash, keys, first, cap - 1, slot);
     KL(tsv::k_tsv_intern_verify, nblk(n, TB), TB, n, text, off, len, slot, first, isf, err);
-    int r = xscan(ctx, P, isf, idat, n, n_ids_dev); if (r) return r;
+    int r = xscan(ctx, isf, idat, n, n_ids_dev); if (r) return r;
     KL(tsv::k_tsv_intern_ids, nblk(n, TB), TB, n, slot, first, idat, id_out, first_row_of_id);
     return 0;
 }
-static int tsv_open_impl(fslrc_ctx *ctx, const char *text, int64_t n_bytes, uint64_t hash_seed, fslrc_tsv_info *info, void *stream) {
-    CK(cudaSetDevice(ctx->device));
-    ctx->stream = (cudaStream_t)stream;
+static int tsv_open_impl(fslrc_ctx *ctx, const char *text, int64_t n_bytes, uint64_t hash_seed, fslrc_tsv_info *info) {
     cudaStream_t st = ctx->stream;
     tsv_free(ctx);
     // ---- header (host): which field holds which column (names of collect_mapping_info.py:176-181)
@@ -1228,49 +1252,48 @@ static int tsv_open_impl(fslrc_ctx *ctx, const char *text, int64_t n_bytes, uint
     }
     TsvState *T = ctx->tsv = new TsvState();
     ctx->tsv_gen++;
-    Pipe Pp; memset((void *)&Pp, 0, sizeof(Pp)); Pipe *P = &Pp;       // (scratch of the scan primitive)
     const bool pad = text[n_bytes - 1] != '\n';
     T->n = n_bytes + (pad ? 1 : 0);
-    PA(T->text, T->n + 64);
+    RA(T->mem, T->text, T->n + 64);
     CK(cudaMemcpyAsync(T->text, text, n_bytes, cudaMemcpyHostToDevice, st));
     if (pad) CK(cudaMemsetAsync(T->text + n_bytes, '\n', 1, st));
     CK(cudaEventRecord(ctx->ev[1], st));
     // ---- lines
     const int TB = 256;
     const int64_t nchunks = (T->n + tsv::CHUNK - 1) / tsv::CHUNK;
-    if (nchunks > 0x7ffffff0LL) { tsv_free(ctx); return fail(ctx, FSLRC_ERR_ARG, "tsv: input too large"); }
+    if (nchunks > 0x7ffffff0LL) return fail(ctx, FSLRC_ERR_ARG, "tsv: input too large");
     int *cnt, *pre, *err;
     DA(cnt, nchunks); DA(pre, nchunks); DA(err, 1);
     int64_t *dcount; DA(dcount, 4);
     CK(cudaMemsetAsync(err, 0, sizeof(int), st));
     KL(tsv::k_tsv_count, nblk(nchunks, TB), TB, T->text, (long long)T->n, cnt);
-    { int r = xscan(ctx, P, cnt, pre, (int)nchunks, dcount); if (r) return r; }
+    { int r = xscan(ctx, cnt, pre, (int)nchunks, dcount); if (r) return r; }
     CK(cudaMemcpyAsync(ctx->h_pin, dcount, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
-    if (ctx->h_pin[0] > 0x7ffffff0LL) { free_all(ctx); tsv_free(ctx); return fail(ctx, FSLRC_ERR_ARG, "tsv: too many lines"); }
+    if (ctx->h_pin[0] > 0x7ffffff0LL) return fail(ctx, FSLRC_ERR_ARG, "tsv: too many lines");
     T->n_lines = (int)ctx->h_pin[0];
     T->n_rows = T->n_lines - 1;
-    PA(T->line_start, (int64_t)T->n_lines + 1);
+    RA(T->mem, T->line_start, (int64_t)T->n_lines + 1);
     KL(tsv::k_tsv_lines, nblk(nchunks, TB), TB, T->text, (long long)T->n, pre, T->line_start);
     const int n = T->n_rows;
-    PA(T->read_id, n); PA(T->chrom, n); PA(T->rstart, n); PA(T->rend, n); PA(T->aln, n); PA(T->qstart, n); PA(T->qend, n); PA(T->naln, n);
-    PA(T->q_off, n); PA(T->q_len, n); PA(T->first_row, n);
+    RA(T->mem, T->read_id, n); RA(T->mem, T->chrom, n); RA(T->mem, T->rstart, n); RA(T->mem, T->rend, n);
+    RA(T->mem, T->aln, n); RA(T->mem, T->qstart, n); RA(T->mem, T->qend, n); RA(T->mem, T->naln, n);
+    RA(T->mem, T->q_off, n); RA(T->mem, T->q_len, n); RA(T->mem, T->first_row, n);
     T->score = nullptr;
-    if (w.col[tsv::W_SCORE] >= 0) PA(T->score, n);
+    if (w.col[tsv::W_SCORE] >= 0) RA(T->mem, T->score, n);
     T->n_reads = 0; T->n_chrom = 0;
     if (n > 0) {
         unsigned long long *qh, *ch; long long *coff; int *clen, *cfirst;
         DA(qh, n); DA(ch, n); DA(coff, n); DA(clen, n); DA(cfirst, n);
         KL(tsv::k_tsv_parse, nblk(n, TB), TB, T->text, T->line_start, n, w, (unsigned long long)hash_seed, T->rstart, T->rend, T->naln, T->aln,
            T->qstart, T->qend, T->score, T->q_off, T->q_len, qh, coff, clen, ch, err);
-        int r = tsv_intern(ctx, P, T->text, n, T->q_off, T->q_len, qh, T->read_id, T->first_row, err, dcount + 1); if (r) return r;
-        r = tsv_intern(ctx, P, T->text, n, coff, clen, ch, T->chrom, cfirst, err, dcount + 2); if (r) return r;
+        int r = tsv_intern(ctx, T->text, n, T->q_off, T->q_len, qh, T->read_id, T->first_row, err, dcount + 1); if (r) return r;
+        r = tsv_intern(ctx, T->text, n, coff, clen, ch, T->chrom, cfirst, err, dcount + 2); if (r) return r;
         CK(cudaMemcpyAsync(ctx->h_pin, dcount, 3 * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
         CK(cudaMemcpyAsync(ctx->h_pin + 8, err, sizeof(int), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
         const int e = (int)(ctx->h_pin[8] & 0xffffffff);
         if (e) {
-            free_all(ctx); tsv_free(ctx);
             if (e & tsv::TE_COLLISION) return fail(ctx, FSLRC_ERR_HASH_COLLISION, "tsv: two different names share a 64-bit hash; call again with another hash_seed");
             if (e & tsv::TE_FIELDS) return fail(ctx, FSLRC_ERR_ARG, "tsv: a line has fewer fields than the header");
             if (e & tsv::TE_RANGE) return fail(ctx, FSLRC_ERR_RANGE, "tsv: an integer field does not fit int32");
@@ -1300,29 +1323,21 @@ static int tsv_open_impl(fslrc_ctx *ctx, const char *text, int64_t n_bytes, uint
     if (cudaEventElapsedTime(&ms, ctx->ev[0 + 1], ctx->ev[2]) == cudaSuccess) info->parse_ms = ms; else cudaGetLastError();
     return 0;
 }
-static void pfree(fslrc_ctx *ctx, void *p) {                            // one persistent array, before fslrc_tsv_close
-    std::vector<void *> &a = ctx->tsv->allocs;
-    std::vector<void *>::iterator it = std::find(a.begin(), a.end(), p);
-    if (it != a.end()) { a.erase(it); cudaFreeAsync(p, ctx->stream); }
-}
 // --filter-false on the parsed table: flag the reads (one thread per read), two exclusive scans give the new read ids and
 // the new row positions, one read-back of both totals, and, if any row goes, one compaction into fresh arrays
-static int tsv_delete_false_impl(fslrc_ctx *ctx, fslrc_tsv_info *info, void *stream) {
-    CK(cudaSetDevice(ctx->device));
-    ctx->stream = (cudaStream_t)stream;
+static int tsv_delete_false_impl(fslrc_ctx *ctx, fslrc_tsv_info *info) {
     cudaStream_t st = ctx->stream;
     TsvState *T = ctx->tsv;
     const int n = T->n_rows, R = T->n_reads, TB = 256;
     ctx->tsv_gen++;
     CK(cudaEventRecord(ctx->ev[1], st));
     if (R > 0) {
-        Pipe Pp; memset((void *)&Pp, 0, sizeof(Pp)); Pipe *P = &Pp;
         int *keep_read, *new_id, *keep_row, *new_pos; int64_t *tot;
         DA(keep_read, R); DA(new_id, R); DA(keep_row, n); DA(new_pos, n); DA(tot, 2);
         KL(tsv::k_tsv_false, nblk(R, TB), TB, R, T->text, T->first_row, T->q_off, T->q_len, keep_read);
-        int r = xscan(ctx, P, keep_read, new_id, R, tot); if (r) return r;
+        int r = xscan(ctx, keep_read, new_id, R, tot); if (r) return r;
         KL(tsv::k_tsv_row_keep, nblk(n, TB), TB, n, T->read_id, keep_read, keep_row);
-        r = xscan(ctx, P, keep_row, new_pos, n, tot + 1); if (r) return r;
+        r = xscan(ctx, keep_row, new_pos, n, tot + 1); if (r) return r;
         CK(cudaMemcpyAsync(ctx->h_pin, tot, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
         const int R2 = (int)ctx->h_pin[0], n2 = (int)ctx->h_pin[1];
@@ -1331,14 +1346,15 @@ static int tsv_delete_false_impl(fslrc_ctx *ctx, fslrc_tsv_info *info, void *str
                                  T->q_off, T->q_len, T->line_start, T->line_end};
             tsv::Cols d; memset((void *)&d, 0, sizeof(d));
             int *first_row;
-            PA(d.read_id, n2); PA(d.chrom, n2); PA(d.rstart, n2); PA(d.rend, n2); PA(d.aln, n2); PA(d.qstart, n2); PA(d.qend, n2);
-            PA(d.naln, n2); PA(d.q_off, n2); PA(d.q_len, n2); PA(d.line_start, (int64_t)n2 + 1); PA(d.line_end, (int64_t)n2 + 1);
-            PA(first_row, R2);
-            if (T->score) PA(d.score, n2);
+            RA(T->mem, d.read_id, n2); RA(T->mem, d.chrom, n2); RA(T->mem, d.rstart, n2); RA(T->mem, d.rend, n2);
+            RA(T->mem, d.aln, n2); RA(T->mem, d.qstart, n2); RA(T->mem, d.qend, n2); RA(T->mem, d.naln, n2);
+            RA(T->mem, d.q_off, n2); RA(T->mem, d.q_len, n2); RA(T->mem, d.line_start, (int64_t)n2 + 1); RA(T->mem, d.line_end, (int64_t)n2 + 1);
+            RA(T->mem, first_row, R2);
+            if (T->score) RA(T->mem, d.score, n2);
             KL(tsv::k_tsv_compact, nblk(n, TB), TB, n, keep_row, new_pos, new_id, T->first_row, s, d, first_row);
             void *old[] = {s.read_id, s.chrom, s.rstart, s.rend, s.aln, s.qstart, s.qend, s.naln, s.score, s.q_off, s.q_len,
                            s.line_start, s.line_end, T->first_row};
-            for (void *p : old) if (p) pfree(ctx, p);                  // (stream-ordered: after the compaction has read them)
+            for (void *p : old) if (p) res_free(ctx, T->mem, p);       // (stream-ordered: after the compaction has read them)
             T->read_id = d.read_id; T->chrom = d.chrom; T->rstart = d.rstart; T->rend = d.rend; T->aln = d.aln;
             T->qstart = d.qstart; T->qend = d.qend; T->naln = d.naln; T->score = d.score; T->q_off = d.q_off; T->q_len = d.q_len;
             T->line_start = d.line_start; T->line_end = d.line_end; T->first_row = first_row;
@@ -1355,27 +1371,46 @@ static int tsv_delete_false_impl(fslrc_ctx *ctx, fslrc_tsv_info *info, void *str
     if (cudaEventElapsedTime(&ms, ctx->ev[1], ctx->ev[2]) == cudaSuccess) info->filter_ms = ms; else cudaGetLastError();
     return 0;
 }
+// The second pass of a text render.  len[i] is the byte length of line i (n lines, written by the caller's length kernel); an
+// exclusive scan gives every line's offset, and with the optional header *n_out is the size of the file.  out == NULL only
+// asks for that size; otherwise emit(off, d_out) writes the lines after the header into a device buffer that goes to `out`.
+template <typename Emit>
+static int render_text(fslrc_ctx *ctx, const char *who, int n, const long long *len, const std::string *header, char *out,
+                       int64_t cap, int64_t *n_out, Emit &&emit) {
+    cudaStream_t st = ctx->stream;
+    const int64_t nh = header ? (int64_t)header->size() : 0;
+    long long *off; int64_t *tot;
+    DA(off, n); DA(tot, 1);
+    { int r = xscan64(ctx, len, off, n, tot); if (r) return r; }
+    CK(cudaMemcpyAsync(ctx->h_pin, tot, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    *n_out = ctx->h_pin[0] + nh;
+    if (out) {
+        if (cap < *n_out) return fail(ctx, FSLRC_ERR_ARG, "%s: output buffer too small", who);
+        unsigned char *d_out; DA(d_out, *n_out);
+        if (nh > 0) CK(cudaMemcpyAsync(d_out, header->data(), nh, cudaMemcpyHostToDevice, st));
+        emit((const long long *)off, d_out);
+        CK(cudaMemcpyAsync(out, d_out, *n_out, cudaMemcpyDeviceToHost, st));
+    }
+    free_all(ctx);
+    CK(cudaStreamSynchronize(st));
+    return 0;
+}
 extern "C" {
 
 int fslrc_tsv_open(fslrc_ctx *ctx, const char *text, int64_t n_bytes, uint64_t hash_seed, fslrc_tsv_info *info, void *stream) {
     if (!ctx) return FSLRC_ERR_ARG;
     if (!text || !info || n_bytes <= 0) return fail(ctx, FSLRC_ERR_ARG, "tsv: null or empty input");
-    const int r = tsv_open_impl(ctx, text, n_bytes, hash_seed, info, stream);
-    if (r) {                                                           // every error path: scratch and the half-built table go
-        free_all(ctx); tsv_free(ctx);
-        cudaStreamSynchronize(ctx->stream);
-    }
-    return r;
+    CK(cudaSetDevice(ctx->device));
+    ctx->stream = (cudaStream_t)stream;
+    return table_call(ctx, tsv_free, [&] { return tsv_open_impl(ctx, text, n_bytes, hash_seed, info); });
 }
 int fslrc_tsv_delete_false(fslrc_ctx *ctx, fslrc_tsv_info *info, void *stream) {
     if (!ctx) return FSLRC_ERR_ARG;
     if (!ctx->tsv || !info) return fail(ctx, FSLRC_ERR_ARG, "tsv: no parsed table (fslrc_tsv_open first) or null info");
-    const int r = tsv_delete_false_impl(ctx, info, stream);
-    if (r) {                                                           // the table keeps its old arrays until the compaction ran
-        free_all(ctx);
-        cudaStreamSynchronize(ctx->stream);
-    }
-    return r;
+    CK(cudaSetDevice(ctx->device));
+    ctx->stream = (cudaStream_t)stream;
+    return table_call(ctx, nullptr, [&] { return tsv_delete_false_impl(ctx, info); });   // (the old arrays stay until the compaction ran)
 }
 int fslrc_tsv_chrom_name(fslrc_ctx *ctx, int32_t chrom_id, char *buf, int32_t cap) {
     if (!ctx || !ctx->tsv || !buf || chrom_id < 0 || chrom_id >= ctx->tsv->n_chrom) return FSLRC_ERR_ARG;
@@ -1407,33 +1442,18 @@ int fslrc_tsv_write_cluster_bed(fslrc_ctx *ctx, const int32_t *cluster_dev, cons
     CK(cudaSetDevice(ctx->device));
     ctx->stream = (cudaStream_t)stream;
     cudaStream_t st = ctx->stream;
-    Pipe Pp; memset((void *)&Pp, 0, sizeof(Pp)); Pipe *P = &Pp;
-    const int L = T->n_lines, TB = 256;
-    long long *len, *off; int64_t *tot; int *any_single;
-    DA(len, L); DA(off, L); DA(tot, 1); DA(any_single, 1);
-    CK(cudaMemsetAsync(any_single, 0, sizeof(int), st));
-    if (T->n_reads > 0) KL(tsv::k_tsv_any_single, nblk(T->n_reads, TB), TB, T->n_reads, n_reads_dev, any_single);
-    KL(tsv::k_tsv_outlen, nblk(L, TB), TB, L, T->line_start, T->line_end, T->read_id, cluster_dev, n_reads_dev, any_single, len);
-    {
-        const int tiles = nblk(L, prims::SC_TILE);
-        int r = prim_scratch(ctx, P, sizeof(unsigned long long) * tiles); if (r) return r;
-        KL(prims::k_scan_excl<long long>, tiles, prims::SC_THREADS, len, off, L, (unsigned long long *)(P->prim + 256), (unsigned *)P->prim, (long long *)tot);
-    }
-    CK(cudaMemcpyAsync(ctx->h_pin, tot, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    *n_out = ctx->h_pin[0];
-    int rc = 0;
-    if (out) {
-        if (cap < *n_out) rc = fail(ctx, FSLRC_ERR_ARG, "tsv: output buffer too small");
-        else {
-            unsigned char *d_out; DA(d_out, *n_out);
-            KL(tsv::k_tsv_emit, nblk((int64_t)L * 32, TB), TB, L, T->text, T->line_start, T->line_end, T->read_id, cluster_dev, n_reads_dev, any_single, off, d_out);
-            CK(cudaMemcpyAsync(out, d_out, *n_out, cudaMemcpyDeviceToHost, st));
-        }
-    }
-    free_all(ctx);
-    CK(cudaStreamSynchronize(st));
-    return rc;
+    return table_call(ctx, nullptr, [&]() -> int {
+        const int L = T->n_lines, TB = 256;
+        long long *len; int *any_single;
+        DA(len, L); DA(any_single, 1);
+        CK(cudaMemsetAsync(any_single, 0, sizeof(int), st));
+        if (T->n_reads > 0) KL(tsv::k_tsv_any_single, nblk(T->n_reads, TB), TB, T->n_reads, n_reads_dev, any_single);
+        KL(tsv::k_tsv_outlen, nblk(L, TB), TB, L, T->line_start, T->line_end, T->read_id, cluster_dev, n_reads_dev, any_single, len);
+        return render_text(ctx, "tsv", L, len, nullptr, out, cap, n_out, [&](const long long *off, unsigned char *d_out) {
+            KL(tsv::k_tsv_emit, nblk((int64_t)L * 32, TB), TB, L, T->text, T->line_start, T->line_end, T->read_id, cluster_dev, n_reads_dev,
+               any_single, off, d_out);
+        });
+    });
 }
 int fslrc_tsv_write_representative_bed(fslrc_ctx *ctx, const int32_t *cluster_dev, const int32_t *n_reads_dev, char *out,
                                        int64_t cap, int64_t *n_out, void *stream) {
@@ -1443,44 +1463,27 @@ int fslrc_tsv_write_representative_bed(fslrc_ctx *ctx, const int32_t *cluster_de
     CK(cudaSetDevice(ctx->device));
     ctx->stream = (cudaStream_t)stream;
     cudaStream_t st = ctx->stream;
-    Pipe Pp; memset((void *)&Pp, 0, sizeof(Pp)); Pipe *P = &Pp;
-    const int L = T->n_lines, R = T->n_reads, TB = 256;
-    long long *sum, *len, *off; int *cnt, *err, *any_single, *txt_len; unsigned char *is_rep; char *txt; int64_t *tot;
-    DA(sum, R); DA(cnt, R); DA(is_rep, R); DA(txt_len, R); DA(txt, (int64_t)R * fmtd::FMT_F64_MAX); DA(err, 1); DA(any_single, 1);
-    DA(len, L); DA(off, L); DA(tot, 1);
-    // cluster ids of the clustering are < n_reads, so n_reads bounds them without a read-back; ids from elsewhere are checked
-    { int r = choose_alignment_dev(ctx, T->n_rows, R, R, T->read_id, T->score, cluster_dev, sum, cnt, is_rep, nullptr, err); if (r) return r; }
-    CK(cudaMemsetAsync(any_single, 0, sizeof(int), st));
-    if (R > 0) {
-        KL(tsv::k_tsv_any_single, nblk(R, TB), TB, R, n_reads_dev, any_single);
-        KL(tsv::k_tsv_rep_mean, nblk(R, TB), TB, R, is_rep, sum, cnt, txt, txt_len);
-    }
-    KL(tsv::k_tsv_rep_outlen, nblk(L, TB), TB, L, T->line_start, T->line_end, T->read_id, cluster_dev, n_reads_dev, any_single, is_rep, txt_len, len);
-    {
-        const int tiles = nblk(L, prims::SC_TILE);
-        int r = prim_scratch(ctx, P, sizeof(unsigned long long) * tiles); if (r) return r;
-        KL(prims::k_scan_excl<long long>, tiles, prims::SC_THREADS, len, off, L, (unsigned long long *)(P->prim + 256), (unsigned *)P->prim, (long long *)tot);
-    }
-    CK(cudaMemcpyAsync(ctx->h_pin, tot, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(ctx->h_pin + 1, err, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    int rc = 0;
-    if ((int)(ctx->h_pin[1] & 0xffffffff)) rc = fail(ctx, FSLRC_ERR_RANGE, "tsv: a cluster id is negative or not below n_reads");
-    else {
-        *n_out = ctx->h_pin[0];
-        if (out) {
-            if (cap < *n_out) rc = fail(ctx, FSLRC_ERR_ARG, "tsv: output buffer too small");
-            else {
-                unsigned char *d_out; DA(d_out, *n_out);
-                KL(tsv::k_tsv_rep_emit, nblk((int64_t)L * 32, TB), TB, L, T->text, T->line_start, T->line_end, T->read_id, cluster_dev, n_reads_dev,
-                   any_single, is_rep, txt, txt_len, off, d_out);
-                CK(cudaMemcpyAsync(out, d_out, *n_out, cudaMemcpyDeviceToHost, st));
-            }
+    return table_call(ctx, nullptr, [&]() -> int {
+        const int L = T->n_lines, R = T->n_reads, TB = 256;
+        long long *sum, *len; int *cnt, *err, *any_single, *txt_len; unsigned char *is_rep; char *txt;
+        DA(sum, R); DA(cnt, R); DA(is_rep, R); DA(txt_len, R); DA(txt, (int64_t)R * fmtd::FMT_F64_MAX); DA(err, 1); DA(any_single, 1);
+        DA(len, L);
+        // cluster ids of the clustering are < n_reads, so n_reads bounds them without a read-back; ids from elsewhere are checked
+        { int r = choose_alignment_dev(ctx, T->n_rows, R, R, T->read_id, T->score, cluster_dev, sum, cnt, is_rep, nullptr, err); if (r) return r; }
+        CK(cudaMemsetAsync(any_single, 0, sizeof(int), st));
+        if (R > 0) {
+            KL(tsv::k_tsv_any_single, nblk(R, TB), TB, R, n_reads_dev, any_single);
+            KL(tsv::k_tsv_rep_mean, nblk(R, TB), TB, R, is_rep, sum, cnt, txt, txt_len);
         }
-    }
-    free_all(ctx);
-    CK(cudaStreamSynchronize(st));
-    return rc;
+        KL(tsv::k_tsv_rep_outlen, nblk(L, TB), TB, L, T->line_start, T->line_end, T->read_id, cluster_dev, n_reads_dev, any_single, is_rep, txt_len, len);
+        CK(cudaMemcpyAsync(ctx->h_pin + 1, err, sizeof(int), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if ((int)(ctx->h_pin[1] & 0xffffffff)) return fail(ctx, FSLRC_ERR_RANGE, "tsv: a cluster id is negative or not below n_reads");
+        return render_text(ctx, "tsv", L, len, nullptr, out, cap, n_out, [&](const long long *off, unsigned char *d_out) {
+            KL(tsv::k_tsv_rep_emit, nblk((int64_t)L * 32, TB), TB, L, T->text, T->line_start, T->line_end, T->read_id, cluster_dev, n_reads_dev,
+               any_single, is_rep, txt, txt_len, off, d_out);
+        });
+    });
 }
 int fslrc_tsv_write_edges(fslrc_ctx *ctx, char *out, int64_t cap, int64_t *n_out, void *stream) {
     if (!ctx) return FSLRC_ERR_ARG;
@@ -1493,31 +1496,16 @@ int fslrc_tsv_write_edges(fslrc_ctx *ctx, char *out, int64_t cap, int64_t *n_out
     CK(cudaSetDevice(ctx->device));
     ctx->stream = (cudaStream_t)stream;
     cudaStream_t st = ctx->stream;
-    Pipe Pp; memset((void *)&Pp, 0, sizeof(Pp)); Pipe *P = &Pp;
-    const int n = (int)E->n, L = n + 1, TB = 256;
-    long long *len, *off; int64_t *tot;
-    DA(len, L); DA(off, L); DA(tot, 1);
-    KL(tsv::k_tsv_edge_outlen, nblk(L, TB), TB, n, E->read1, E->read2, E->jac, T->first_row, T->q_len, len);
-    {
-        const int tiles = nblk(L, prims::SC_TILE);
-        int r = prim_scratch(ctx, P, sizeof(unsigned long long) * tiles); if (r) return r;
-        KL(prims::k_scan_excl<long long>, tiles, prims::SC_THREADS, len, off, L, (unsigned long long *)(P->prim + 256), (unsigned *)P->prim, (long long *)tot);
-    }
-    CK(cudaMemcpyAsync(ctx->h_pin, tot, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    *n_out = ctx->h_pin[0];
-    int rc = 0;
-    if (out) {
-        if (cap < *n_out) rc = fail(ctx, FSLRC_ERR_ARG, "tsv: output buffer too small");
-        else {
-            unsigned char *d_out; DA(d_out, *n_out);
-            KL(tsv::k_tsv_edge_emit, nblk((int64_t)L * 32, TB), TB, n, T->text, E->read1, E->read2, E->jac, T->first_row, T->q_off, T->q_len, off, d_out);
-            CK(cudaMemcpyAsync(out, d_out, *n_out, cudaMemcpyDeviceToHost, st));
-        }
-    }
-    free_all(ctx);
-    CK(cudaStreamSynchronize(st));
-    return rc;
+    return table_call(ctx, nullptr, [&]() -> int {
+        const int n = (int)E->n, L = n + 1, TB = 256;
+        long long *len;
+        DA(len, L);
+        KL(tsv::k_tsv_edge_outlen, nblk(L, TB), TB, n, E->read1, E->read2, E->jac, T->first_row, T->q_len, len);
+        return render_text(ctx, "tsv", L, len, nullptr, out, cap, n_out, [&](const long long *off, unsigned char *d_out) {
+            KL(tsv::k_tsv_edge_emit, nblk((int64_t)L * 32, TB), TB, n, T->text, E->read1, E->read2, E->jac, T->first_row, T->q_off, T->q_len,
+               off, d_out);
+        });
+    });
 }
 void fslrc_tsv_close(fslrc_ctx *ctx) {
     if (!ctx) return;

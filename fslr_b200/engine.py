@@ -170,6 +170,75 @@ class _DevView:
         self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": "<i4", "data": (int(ptr), False), "version": 2}
 
 
+class ResidentTable:
+    """A mappings table built on the device and kept there by the library context (tsv.ParsedBed, mapping_info.BamTable).
+    Quacks like ColumnarTable where the engine needs it.  The context holds ONE table of each kind: the next open on the
+    same engine frees this one's device columns, after which every method raises RuntimeError ("stale")."""
+
+    _replaced = ""          # subclasses: what replaced a stale table, for the error message
+    _names_fn = ""          # subclasses: the library's qname entry point, fn(ctx, offsets, lengths)
+    _close_fn = ""          # subclasses: the library's close
+
+    def __init__(self, engine, data, info):
+        self.engine, self._data, self.info = engine, data, info
+        self.n_rows, self.n_reads = int(info.n_rows), int(info.n_reads)
+        self.order = None
+        self.out_cluster = torch.empty(max(self.n_reads, 1), dtype=torch.int32, device=engine.device)
+        self.out_n_reads = torch.empty(max(self.n_reads, 1), dtype=torch.int32, device=engine.device)
+        self._names = None
+        gen = engine._table_gen
+        gen[type(self)] = self._gen = gen.get(type(self), 0) + 1
+
+    def _live(self):
+        if self.engine is None:
+            raise RuntimeError("%s is closed" % type(self).__name__)
+        if self._gen != self.engine._table_gen[type(self)]:
+            raise RuntimeError("stale %s: %s (the library context holds one at a time)" % (type(self).__name__, self._replaced))
+
+    @property
+    def n_chrom(self):
+        return len(self.chrom_names)
+
+    def _name_bytes(self):
+        """The bytes the offsets of the names entry point index."""
+        raise NotImplementedError
+
+    def qnames(self):
+        """qname of every read id (ParsedBed: ids in order of first appearance; BamTable: in output order), sliced out of
+        the input bytes on the host."""
+        if self._names is None:
+            self._live()
+            off = np.zeros(max(self.n_reads, 1), dtype=np.int64)
+            ln = np.zeros(max(self.n_reads, 1), dtype=np.int32)
+            self.engine._check(getattr(self.engine.lib, self._names_fn)(self.engine.ctx, off.ctypes.data, ln.ctypes.data))
+            buf = self._name_bytes()
+            self._names = np.array([buf[o:o + l].decode() for o, l in zip(off[:self.n_reads], ln[:self.n_reads])], dtype=object)
+        return self._names
+
+    def cluster(self, cluster_mask="subtelomere", tie_order=None, edges=False, **options):
+        """The clustering step (main.py:209-257,334-342) on the device-resident table.  Returns ClusterResult; the per-read
+        result also stays on the device (out_cluster / out_n_reads) for the renderers.
+        tie_order: how fillings with equal starts are ordered (cluster.py:114), which decides the cluster numbering.
+        None: `self.order` when the caller set one, else the GPU's stable sort (ties keep bed order).  "stable": the GPU's
+        stable sort.  "reference": the permutation fslr's own `sort_values('start')` gives on this host, so the ids equal
+        fslr's: the start column is built on the device (fslrc_filling_starts), sorted on the host with the reference's
+        pandas call and sent back, once per table (kept for later calls); it applies to that call only.
+        edges=True: ClusterResult.edges holds the similarity graph (cluster.py:187-227's match_df rows, as read ids); for a
+        ParsedBed, edges_bytes() / write_edges() can render it until the next clustering call on this engine."""
+        self._live()
+        params = ClusterParams.from_options(self, cluster_mask=cluster_mask, **options)
+        out = self.engine.run_resident(self, self, params, order=self.engine.tie_order(self, tie_order), edges=edges)
+        stats, el = out if edges else (out, None)
+        n = self.n_reads
+        return ClusterResult(self.out_cluster[:n].cpu().numpy(), self.out_n_reads[:n].cpu().numpy(), bool(stats["no_clusters"]), stats, el)
+
+    def close(self):
+        if self.engine is not None:
+            if self._gen == self.engine._table_gen[type(self)]:    # (a stale object owns nothing any more)
+                getattr(self.engine.lib, self._close_fn)(self.engine.ctx)
+            self.engine = None
+
+
 class Engine:
     def __init__(self, device=0):
         if not torch.cuda.is_available():
@@ -183,6 +252,7 @@ class Engine:
         if rc != 0:
             raise _native.FslrError(rc, "fslrc_create failed")
         self._capture = False
+        self._table_gen = {}                          # ResidentTable subclass -> generation of the table the context holds
 
     def pinned_bytes(self, n):
         """A pinned uint8 staging buffer of at least n bytes, kept and reused (pinning hundreds of MB costs more than the
@@ -191,6 +261,27 @@ class Engine:
         if buf is None or buf.numel() < n:
             self._pinned = buf = torch.empty(max(int(n * 1.25), 1 << 20), dtype=torch.uint8).pin_memory()
         return buf[:max(n, 1)]
+
+    def _cuda_stream(self):
+        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def open_table(self, fn, args, hash_seed, info):
+        """fn(ctx, *args, seed, &info, stream): an open of a device-resident table, called again with the next seed (up to
+        four seeds) when two names share a 64-bit hash."""
+        for attempt in range(4):
+            rc = fn(self.ctx, *args, hash_seed + attempt, C.byref(info), self._cuda_stream())
+            if rc != _native.ERR_HASH_COLLISION:
+                break
+        self._check(rc)
+
+    def render_bytes(self, fn, *args):
+        """fn(ctx, *args, out, cap, &n_out, stream): a renderer of a device-resident table, called once for the size and once
+        into the reused pinned staging buffer.  Returns a VIEW of that buffer: valid until the next rendering call."""
+        n = C.c_int64()
+        self._check(fn(self.ctx, *args, None, 0, C.byref(n), self._cuda_stream()))
+        out = self.pinned_bytes(n.value)
+        self._check(fn(self.ctx, *args, out.data_ptr(), n.value, C.byref(n), self._cuda_stream()))
+        return out[:n.value].numpy()
 
     def close(self):
         if getattr(self, "ctx", None):

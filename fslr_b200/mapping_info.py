@@ -18,10 +18,8 @@ import numpy as np
 import torch
 
 from . import _native
-from .engine import ClusterResult, _DevView, get_engine
-from .table import ClusterParams
+from .engine import _COLS, ResidentTable, _DevView, get_engine
 
-_COLS = ("read_id", "chrom", "rstart", "rend", "aln_size", "qstart", "qend", "n_alignments")
 OUT_COLUMNS = ["chrom", "rstart", "rend", "qname", "n_alignments", "aln_size", "qstart", "qend", "strand", "mapq", "qlen",
                "alignment_score", "short_anchor<50bp", "fslr_version", "inferred_by_primer", "seq"]   # collect_mapping_info.py:176-177
 
@@ -151,13 +149,16 @@ def _default_version():
         return __version__
 
 
-class BamTable:
+class BamTable(ResidentTable):
     """The mappings table built on the device from a BAM file, rows in the order of collect_mapping_info.py:174.  Quacks
     like ColumnarTable where the clustering engine needs it (chrom_names, chrom_len, n_chrom, n_rows, n_reads, cols)."""
 
+    _replaced = "a later read_bam_table() on this device replaced the table"
+    _names_fn = "fslrc_bam_read_names"
+    _close_fn = "fslrc_bam_close"
+
     def __init__(self, engine, data, info, refs, primers, with_regions):
-        self.engine, self._data, self.info = engine, data, info
-        self.n_rows, self.n_reads = int(info.n_rows), int(info.n_reads)
+        super().__init__(engine, data, info)
         self.n_records, self.n_mapped = int(info.n_records), int(info.n_mapped)
         self.primer_names = list(primers)
         self.chrom_names = [n for n, _ in refs] + self.primer_names       # inferred rows carry the primer name as chrom (:124,143)
@@ -168,24 +169,6 @@ class BamTable:
         view = lambda p: torch.as_tensor(_DevView(p, (self.n_rows,)), device=dev)
         self.columns = {k: view(getattr(info, k)) for k in _native.BAM_COLUMNS}
         self.cols = {k: self.columns[k] for k in _COLS}
-        self.order = None
-        self.out_cluster = torch.empty(max(self.n_reads, 1), dtype=torch.int32, device=dev)
-        self.out_n_reads = torch.empty(max(self.n_reads, 1), dtype=torch.int32, device=dev)
-        self._names = None
-        # one table per library context (fslrc_bam_open frees the previous one): see ParsedBed
-        engine._bam_gen = getattr(engine, "_bam_gen", 0) + 1
-        self._gen = engine._bam_gen
-
-    def _live(self):
-        if self.engine is None:
-            raise RuntimeError("BamTable is closed")
-        if self._gen != self.engine._bam_gen:
-            raise RuntimeError("stale BamTable: a later read_bam_table() on this device replaced the table "
-                               "(the library context holds one at a time)")
-
-    @property
-    def n_chrom(self):
-        return len(self.chrom_names)
 
     def column(self, name):
         """Host copy of one column (int32)."""
@@ -202,15 +185,8 @@ class BamTable:
             self.engine._check(self.engine.lib.fslrc_bam_read_stream(self.engine.ctx, self._data.ctypes.data, n.value, C.byref(n)))
         return self._data
 
-    def qnames(self):
-        """qname of every read id (reads numbered in output order)."""
-        if self._names is None:
-            off = np.zeros(max(self.n_reads, 1), dtype=np.int64)
-            ln = np.zeros(max(self.n_reads, 1), dtype=np.int32)
-            self.engine._check(self.engine.lib.fslrc_bam_read_names(self.engine.ctx, off.ctypes.data, ln.ctypes.data))
-            buf = self._stream().tobytes()
-            self._names = np.array([buf[o:o + l].decode() for o, l in zip(off[:self.n_reads], ln[:self.n_reads])], dtype=object)
-        return self._names
+    def _name_bytes(self):
+        return self._stream().tobytes()
 
     def to_dataframe(self):
         """The table as pandas would read the written file back (without `seq` and `fslr_version`)."""
@@ -231,35 +207,12 @@ class BamTable:
     def mappings_bed_bytes(self, fslr_version=None):
         """`<base>.mappings.bed` (collect_mapping_info.py:176-181) as bytes, rendered on the device."""
         self._live()
-        lib, ctx = self.engine.lib, self.engine.ctx
         ver = (fslr_version if fslr_version is not None else _default_version()).encode()
         names = b"".join(n.encode() + b"\x00" for n in self.chrom_names)
-        stream = C.c_void_p(torch.cuda.current_stream(self.engine.device).cuda_stream)
-        n = C.c_int64()
-        self.engine._check(lib.fslrc_bam_write_mappings_bed(ctx, names, ver, None, 0, C.byref(n), stream))
-        out = self.engine.pinned_bytes(n.value)       # reused staging buffer: the result is valid until the next rendering call
-        self.engine._check(lib.fslrc_bam_write_mappings_bed(ctx, names, ver, out.data_ptr(), n.value, C.byref(n), stream))
-        return out[:n.value].numpy()
+        return self.engine.render_bytes(self.engine.lib.fslrc_bam_write_mappings_bed, names, ver)
 
     def write_mappings_bed(self, path, fslr_version=None):
         self.mappings_bed_bytes(fslr_version).tofile(path)
-
-    def cluster(self, cluster_mask="subtelomere", tie_order=None, edges=False, **options):
-        """The clustering step (main.py:209-257,334-342) on the device-resident table.  tie_order as ParsedBed.cluster:
-        None (`self.order` if set, else the GPU's stable sort), "stable", or "reference" (fslr's own tie order on this
-        host, computed once per table).  edges=True: ClusterResult.edges holds the similarity graph."""
-        params = ClusterParams.from_options(self, cluster_mask=cluster_mask, **options)
-        self._live()
-        out = self.engine.run_resident(self, self, params, order=self.engine.tie_order(self, tie_order), edges=edges)
-        stats, el = out if edges else (out, None)
-        n = self.n_reads
-        return ClusterResult(self.out_cluster[:n].cpu().numpy(), self.out_n_reads[:n].cpu().numpy(), bool(stats["no_clusters"]), stats, el)
-
-    def close(self):
-        if self.engine is not None:
-            if self._gen == self.engine._bam_gen:
-                self.engine.lib.fslrc_bam_close(self.engine.ctx)
-            self.engine = None
 
 
 def read_bam_table(bam, regions_path=None, primers=None, device=0, hash_seed=0, threads=8, device_inflate=True):
@@ -306,15 +259,10 @@ def read_bam_table(bam, regions_path=None, primers=None, device=0, hash_seed=0, 
     n_regions = len(rc) if regions else -1                               # `if regions:` (:72,96): an empty file means no column
     rc, rs, re_ = (np.asarray(a, dtype=np.int32) for a in (rc, rs, re_))
     info = _native.BamInfo()
-    stream = C.c_void_p(torch.cuda.current_stream(eng.device).cuda_stream)
     names = b"".join(n.encode() + b"\x00" for n in pnames)
     fn = eng.lib.fslrc_bam_open if inflated else eng.lib.fslrc_bam_open_bgzf
-    for attempt in range(4):                                             # a 64-bit hash collision between two names: reseed
-        code = fn(eng.ctx, data.ctypes.data, data.shape[0], first, len(refs), names, plen.ctypes.data, len(pnames),
-                  rc.ctypes.data, rs.ctypes.data, re_.ctypes.data, n_regions, hash_seed + attempt, C.byref(info), stream)
-        if code != _native.ERR_HASH_COLLISION:
-            break
-    eng._check(code)
+    eng.open_table(fn, (data.ctypes.data, data.shape[0], first, len(refs), names, plen.ctypes.data, len(pnames),
+                        rc.ctypes.data, rs.ctypes.data, re_.ctypes.data, n_regions), hash_seed, info)
     return BamTable(eng, data if inflated else None, info, refs, pnames, n_regions >= 0)
 
 
